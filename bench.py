@@ -2,6 +2,7 @@
 """bench.py -- FEM loss+grad throughput of the fused sm_100a kernels (and the reference arm).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (fused Poisson energy loss + gradient w.r.t. u) over one
 batch of synthetic input.  Default workload = BASELINE.json configs[1]: Poisson 2-D parametric,
@@ -180,9 +181,10 @@ def shared_config(name, world):
 FLOPS_PER_DOF = {2: 90.0, 3: 280.0}     # closed-form fp32 operations per DOF, fwd + adjoint (SURVEY.md 8d)
 
 
-def time_workload(name, dev, seed, K, W, reps, world=1, barrier=None, use_graph=True):
+def time_workload(name, dev, seed, K, W, reps, world=1, barrier=None, use_graph=True, keep_last=False):
     """Device-timed fused loss+gradient launches of one workload on this rank: K launches replayed
-    from one CUDA graph, CUDA events, median of `reps`.  Returns ms per step (this rank) and the mode."""
+    from one CUDA graph, CUDA events, median of `reps`.  Returns ms per step (this rank) and the mode;
+    with `keep_last`, also `last`: host copies of (loss, grad) of the last timed step."""
     import torch
     fem = make_fem(name)
     nsets = nsets_for(name)
@@ -209,7 +211,7 @@ def time_workload(name, dev, seed, K, W, reps, world=1, barrier=None, use_graph=
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph, stream=side):
                 for i in range(K):
-                    launch(i)                      # outputs are recycled by the graph's pool
+                    out = launch(i)                # outputs are recycled by the graph's pool; the last stays live
             graph.replay()                         # one untimed replay
             torch.cuda.synchronize()
         except Exception as e:   # noqa: BLE001
@@ -229,7 +231,7 @@ def time_workload(name, dev, seed, K, W, reps, world=1, barrier=None, use_graph=
             graph.replay()
         else:
             for i in range(K):
-                launch(i)
+                out = launch(i)
         e1.record()
         if barrier is not None:
             barrier()
@@ -237,7 +239,40 @@ def time_workload(name, dev, seed, K, W, reps, world=1, barrier=None, use_graph=
             torch.cuda.synchronize()
         times.append(e0.elapsed_time(e1))
     ms_step = sorted(times)[len(times) // 2] / K
-    return {"ms_step": ms_step, "mode": mode, "sets": sets, "fem": fem, "nsets": nsets}
+    res = {"ms_step": ms_step, "mode": mode, "sets": sets, "fem": fem, "nsets": nsets}
+    if keep_last:
+        res["last"] = {"loss": out[0].detach().cpu(), "grad": out[1].detach().cpu()}
+    return res
+
+
+DUMP_BYTES = 60_000_000     # --dump-outputs writes at most this much array data (64 MB with headroom)
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of `arrays` as out_dir/<name>.npy (float32 / float64).  When the total exceeds
+    DUMP_BYTES, every array is cut to about the same fraction of its elements: every `stride`-th flat
+    element from an offset drawn by a generator seeded with 0, so the same shapes always give the same
+    sample, and no index array is built."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    frac = min(1.0, DUMP_BYTES / max(total, 1))
+    written = {}
+    for name, t in arrays.items():
+        flat = t.detach().cpu().reshape(-1)
+        if flat.dtype not in (torch.float32, torch.float64):
+            flat = flat.float()
+        stride = -(-flat.numel() // max(1, int(flat.numel() * frac)))      # ceil: never above the budget
+        if stride > 1:
+            g = torch.Generator(device="cpu").manual_seed(0)
+            offset = int(torch.randint(stride, (1,), generator=g))
+            arr = flat[offset::stride].numpy()
+        else:
+            arr = flat.numpy().reshape(tuple(t.shape))
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+        written[name] = {"shape": list(t.shape), "stored": int(arr.size), "dtype": str(arr.dtype)}
+    return written
 
 
 def copy_reference(dev, nbytes, K=50, reps=3):
@@ -479,7 +514,8 @@ def run_reference(args):
     def step():
         u = d["u"].clone().requires_grad_(True)
         OL.energy_loss(o, u, **kw).backward()
-    # bounded sample: shrink it until (K + W) steps fit in ~2 minutes of CPU time
+    # bounded sample: shrink the batch until (K + W) steps fit in ~2 minutes of CPU time; K and W
+    # stay what --steps and --warmup say, so at a batch of 1 the run may take longer than that
     step()
     t0 = time.perf_counter(); step(); t1 = time.perf_counter() - t0
     budget, K, W = 120.0, args.steps, args.warmup
@@ -487,11 +523,6 @@ def run_reference(args):
         sB = max(1, int(sB * budget / (t1 * (K + W))))
         d = make_inputs_cpu(name, sB)
         kw = call_kwargs(d)
-        step()
-        t0 = time.perf_counter(); step(); t1 = time.perf_counter() - t0
-    if t1 * (K + W) > budget:
-        K = max(1, int(budget / t1) - W)
-    args.steps = K
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
@@ -599,8 +630,10 @@ def run_ours(args):
         sampler.start()
         time.sleep(0.25)
     reps = args.reps
-    res = time_workload(name, dev, 1234 + 17 * rank, K, W, reps, world, barrier, not args.no_graph)
+    res = time_workload(name, dev, 1234 + 17 * rank, K, W, reps, world, barrier, not args.no_graph,
+                        keep_last=bool(args.dump_outputs))
     sets, fem, nsets, mode = res["sets"], res["fem"], res["nsets"], res["mode"]
+    dumped = dump_outputs(args.dump_outputs, res.pop("last")) if args.dump_outputs and rank == 0 else None
     t = torch.tensor([res["ms_step"]], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -867,6 +900,8 @@ def run_ours(args):
             "points": points,
             "slab": slab,
         }
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -1101,7 +1136,12 @@ def main():
                     help="skip the 256^3 z-slab arm reported under `slab` (N > 1)")
     ap.add_argument("--train-steps", type=int, default=20,
                     help="also time this many full training steps (UNet + loss + DDP + Adam); 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write (loss, grad) of the last timed step of rank 0 as DIR/loss.npy and DIR/grad.npy "
+                         "(a seeded sample of grad when both exceed 60 MB); the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "poisson3d_256_slab"):
+        ap.error("--dump-outputs covers the fused-kernel arm (--impl ours) of the batched workloads")
     if args.impl == "reference":
         if args.workload == "poisson3d_256_slab":
             args.workload = "poisson3d_256_b1"
