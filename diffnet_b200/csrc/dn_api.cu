@@ -314,8 +314,11 @@ static int run2t(const Common& c, const dn_geom* g, float* grad, int mode, int m
   const float kx = c.k.kx, ky = c.k.ky, kf = c.k.kf, t = c.k.t;
   p.k2.kx = make_float2(kx, kx); p.k2.ky = make_float2(ky, ky); p.k2.t = make_float2(t, t);
   p.k2.kxt = make_float2(kx * t, kx * t); p.k2.kyt = make_float2(ky * t, ky * t);
-  p.k2.nkf = make_float2(-kf, -kf); p.k2.nkft = make_float2(-kf * t, -kf * t);
-  p.k2.nkftt = make_float2(-kf * t * t, -kf * t * t);
+  // nodal source stencil (FK == 1): 1-D element mass [[1+t, 1-t], [1-t, 1+t]] in x (times -kf) and in y
+  const float fc = 1.f - t, fw = 2.f * (1.f + t);
+  p.k2.nfc = make_float2(-kf * fc, -kf * fc); p.k2.nfw = make_float2(-kf * fw, -kf * fw);
+  p.k2.yc = make_float2(fc, fc); p.k2.yw = make_float2(fw, fw);
+  p.k2.fmir = make_float2(-(1.f + t) / fc, -(1.f + t) / fc);
   p.k2.c0x_const = make_float2(4.f * kx, 4.f * kx); p.k2.c0y_const = make_float2(4.f * ky, 4.f * ky);
   p.k2.nkb = make_float2(-c.k.kb, -c.k.kb);
   p.grad = grad;

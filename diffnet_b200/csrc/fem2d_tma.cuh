@@ -13,6 +13,7 @@
 //     right neighbour), masked, and reduced to its x-sums / x-differences, which serve both the
 //     element row above and the one below.  The element math is the closed form of DESIGN.md 4
 //     evaluated on float2 PAIRS of elements with FFMA2/FADD2/FMUL2 (two elements per issue slot).
+//     The source term is linear in u: it enters per node, as a separable stencil, when a row closes.
 //   * Gradient gather without atomics: contributions to the top nodes are completed by one
 //     shuffle from the left lane (one shared-memory word across warp seams), contributions to
 //     the bottom nodes are carried in registers to the next row.  One __syncthreads per row
@@ -33,8 +34,12 @@ namespace dn {
 
 // Packed constants of one launch (see prepare(): kx, ky carry S c_k W (2/h)^2 / 64, kf = S c_f W / 16)
 struct K2 {
-  float2 kx, ky, kxt, kyt, t, nkf, nkft, nkftt, c0x_const, c0y_const;
-  float2 nkb;   // -(S c_f): weight of an assembled load vector (FK == 2)
+  float2 kx, ky, kxt, kyt, t, c0x_const, c0y_const;
+  // FK == 1, the nodal source stencil (Fem2T::load_row / src_share): 1-D element mass [[1+t, 1-t], [1-t, 1+t]]
+  float2 nfc, nfw;   // x-stencil: -kf (1-t) per row neighbour, -kf 2(1+t) own weight
+  float2 fmir;       // -(1+t)/(1-t): the missing neighbour of an image edge node, in units of the node's own f
+  float2 yc, yw;     // y-stencil: (1-t) per neighbour row, 2(1+t) own weight (half of it in the image's top/bottom row)
+  float2 nkb;        // -(S c_f): weight of an assembled load vector (FK == 2)
 };
 
 struct P2T {
@@ -121,14 +126,14 @@ __device__ __forceinline__ RowSD row_sd(const float (&v)[5]) {
 }
 
 
-// Two Q1 elements at once.  Inputs: x-sums/differences of u (top st,dt / bottom sb,db), of nu and
-// of f.  Outputs: energy pair E and the nodal gradient pairs ga (top-left), gb (top-right),
+// Two Q1 elements at once.  Inputs: x-sums/differences of u (top st,dt / bottom sb,db) and of nu.
+// Outputs: energy pair E and the nodal gradient pairs ga (top-left), gb (top-right),
 // gc (bottom-left), gd (bottom-right).  Quadratic part in the half-gradient convention
-// q = (1/2) dEq/dA, so E = sum A (q - b) and g = q + (q - b).
-template <bool HAS_NU, bool HAS_F>
+// q = (1/2) dE/dA, so E = sum A q and g = 2 q.  The source term is not part of the element pair: it
+// is linear in u and enters per node (Fem2T::src_share).
+template <bool HAS_NU>
 __device__ __forceinline__ float2 elem_pair(const K2& k, float2 st, float2 dt, float2 sb, float2 db,
                                             float2 nst, float2 ndt, float2 nsb, float2 ndb,
-                                            float2 fst, float2 fdt, float2 fsb, float2 fdb,
                                             float2 vw, float2& ga, float2& gb, float2& gc,
                                             float2& gd) {
   const float2 Ae = sub2(sb, st), Ax = add2(dt, db), Axe = sub2(db, dt);
@@ -150,34 +155,22 @@ __device__ __forceinline__ float2 elem_pair(const K2& k, float2 st, float2 dt, f
     qe = mul2(c0y, Ae);
     qxe = mul2(add2(c0x, c0y), tAxe);
   }
-  float2 E, g0, gx, ge, gxe;
-  if constexpr (HAS_F) {
-    const float2 A0 = add2(st, sb);
-    const float2 nb0 = mul2(k.nkf, add2(fst, fsb));                    // -kf B0
-    const float2 tx = fma2(k.nkft, add2(fdt, fdb), qx);                // q - kf t Bxi
-    const float2 te = fma2(k.nkft, sub2(fsb, fst), qe);                // q - kf t Beta
-    const float2 txe = fma2(k.nkftt, sub2(fdb, fdt), qxe);             // q - kf t^2 Bxieta
-    E = fma2(A0, nb0, fma2(Ax, tx, fma2(Ae, te, mul2(Axe, txe))));
-    g0 = nb0; gx = add2(qx, tx); ge = add2(qe, te); gxe = add2(qxe, txe);
-    const float2 m0 = sub2(g0, ge), m1 = add2(g0, ge), n0 = sub2(gx, gxe), n1 = add2(gx, gxe);
-    ga = sub2(m0, n0); gb = add2(m0, n0); gc = sub2(m1, n1); gd = add2(m1, n1);
-  } else {
-    E = fma2(Ax, qx, fma2(Ae, qe, mul2(Axe, qxe)));
-    gx = add2(qx, qx); ge = add2(qe, qe); gxe = add2(qxe, qxe);
-    const float2 n0 = sub2(gx, gxe), n1 = add2(gx, gxe);
-    // m0 = -ge, m1 = +ge
-    ga = sub2(f2(-ge.x, -ge.y), n0); gb = sub2(n0, ge); gc = sub2(ge, n1); gd = add2(ge, n1);
-  }
+  const float2 E = fma2(Ax, qx, fma2(Ae, qe, mul2(Axe, qxe)));
+  const float2 gx = add2(qx, qx), ge = add2(qe, qe), gxe = add2(qxe, qxe);
+  const float2 n0 = sub2(gx, gxe), n1 = add2(gx, gxe);
+  // m0 = -ge, m1 = +ge
+  ga = sub2(f2(-ge.x, -ge.y), n0); gb = sub2(n0, ge); gc = sub2(ge, n1); gd = add2(ge, n1);
   return E;
 }
 
-// Per-thread state of one masked node row: x-sums / x-differences of u, nu, f and the 0/1
-// "free node" multipliers (0 where a Dirichlet mask fired).
+// Per-thread state of one masked node row: x-sums / x-differences of u and nu, the 0/1
+// "free node" multipliers (0 where a Dirichlet mask fired) and what the source term needs.
 struct Row2T {
-  RowSD u, n, f;
+  RowSD u, n;
   float2 keep01, keep23;
   float2 lb01, lb23;   // FK == 2: -(S c_f) b of the 4 own nodes (their gradient share), and
   float lE;            //          their energy share sum(-(S c_f) b u)
+  float2 fx01, fx23;   // FK == 1: -kf (M_x f) of the 4 own nodes (x-stencil of f)
 };
 // Gradient accumulators of one node row: own nodes 0..3 and the right neighbour's node 0.
 struct Acc2T {
@@ -188,17 +181,26 @@ struct Acc2T {
 // FK: 0 no source term, 1 nodal source f (interpolated to the Gauss points), 2 `f` is an ASSEMBLED load vector
 // b_a = sum_e sum_g w_g N_a(g) f_g (dn_fem_load_vector_f32): the term -c_f sum_a b_a u_a is added per node when its
 // row closes -- what the reference's f-at-Gauss-points form (e8_2d_poisson_mms.py:154-175) costs once b exists.
+//
+// FK == 1 takes the same per-node route.  The element source energy -kf (A0 B0 + t (Ax Bxi + Ae Beta) + t^2 Axe Bxieta)
+// is the tensor product of the 1-D element mass M = [[1+t, 1-t], [1-t, 1+t]] in x and in y (A0 = s_x s_y u,
+// Ax = d_x s_y u, ...; s s' + t d d' = a^T M b), so the assembled term is -kf u^T (M_y (x) M_x) f: node a's gradient
+// share is the separable stencil g_a = -kf (M_y (M_x f))_a and the energy is sum_a u_a g_a.  M_x f is taken when a row
+// is loaded (Row2T::fx), the y-combination when the row closes (src_share).  A node on the image's edge has one
+// element in that direction, i.e. own weight (1+t): in x a mirrored neighbour (K2::fmir) gives it, in y the weight wy.
 template <int NM, bool VF, bool HAS_NU, int FK, bool NUMASK, bool MI = true>
 struct Fem2T {
   static constexpr bool HAS_F = (FK == 1), LV = (FK == 2);
+  static constexpr bool NODAL = HAS_F || LV;      // a per-node source share (Row2T::lb, lE) enters when a row closes
   static constexpr int NF = 1 + (HAS_NU ? 1 : 0) + (FK ? 1 : 0) + (NUMASK ? 1 : 0) + NM + (VF ? 1 : 0);
   static constexpr int F_U = 0, F_NU = 1, F_F = F_NU + (HAS_NU ? 1 : 0), F_NM = F_F + (FK ? 1 : 0),
                        F_M = F_NM + (NUMASK ? 1 : 0), F_VF = F_M + NM;
 
   // Read one node row from its ring stage (own 4 nodes + right neighbour of every field), apply
   // the Dirichlet conditions (array order: later masks win) and the nu mask, reduce to x-sums.
+  // FK == 1: also the left neighbour of f and the x-stencil of f.
   static __device__ __forceinline__ void load_row(const P2T& p, const float* __restrict__ sp, int fstride,
-                                                  bool has_right, Row2T& o) {
+                                                  bool has_left, bool has_right, Row2T& o) {
     float v[NF][5];
 #pragma unroll
     for (int f = 0; f < NF; ++f) {
@@ -207,6 +209,8 @@ struct Fem2T {
       const float h = q[4];            // in-bounds of the ring for every thread (padded), masked below
       v[f][0] = t.x; v[f][1] = t.y; v[f][2] = t.z; v[f][3] = t.w; v[f][4] = has_right ? h : 0.f;
     }
+    float fl = 0.f;                    // f left of node 0: the ring holds the whole row (x0 = 0: the u field's last word)
+    if constexpr (HAS_F) fl = sp[F_F * fstride - 1];
     float ub[5], nb[5], fb[5], kp[4];
 #pragma unroll
     for (int e = 0; e < 5; ++e) {
@@ -235,17 +239,35 @@ struct Fem2T {
       const float2 le = fma2(o.lb01, f2(ub[0], ub[1]), mul2(o.lb23, f2(ub[2], ub[3])));
       o.lE = le.x + le.y;
     }
+    if constexpr (HAS_F) {
+      // -kf (M_x f): (1-t) per neighbour node, 2(1+t) own.  A row end has one element: (1+t) own, which the
+      // mirrored neighbour fmir f gives ((1-t) fmir + 2(1+t) = 1+t) with the interior weights unchanged.
+      fl = has_left ? fl : p.k2.fmir.x * fb[0];
+      const float fr = has_right ? fb[4] : p.k2.fmir.x * fb[3];
+      o.fx01 = fma2(p.k2.nfc, f2(fl + fb[1], fb[0] + fb[2]), mul2(p.k2.nfw, f2(fb[0], fb[1])));
+      o.fx23 = fma2(p.k2.nfc, f2(fb[1] + fb[3], fb[2] + fr), mul2(p.k2.nfw, f2(fb[2], fb[3])));
+    }
     o.u = row_sd(ub);
-    // the last element of a row does not exist: E and g are linear in (nu, f), so zeroing their
+    // the last element of a row does not exist: E and g are linear in nu, so zeroing its
     // x-sums/differences for that element removes it (nu == 1 uses the weight vw instead)
     if constexpr (HAS_NU) {
       o.n = row_sd(nb);
       if (!has_right) { o.n.s23.y = 0.f; o.n.d23.y = 0.f; }
     }
-    if constexpr (HAS_F) {
-      o.f = row_sd(fb);
-      if (!has_right) { o.f.s23.y = 0.f; o.f.d23.y = 0.f; }
-    }
+  }
+
+  // FK == 1: node row `row` closes between the rows above (x-stencil xa) and below (xb) -- zero where the image
+  // ends, and then wy = (1+t) instead of 2(1+t).  Fills row.lb (gradient share) and row.lE (energy share).  The
+  // energy share sum_a u_a lb_a is taken from the row's u x-sums / x-differences (u0 = (s0 - d0) / 2, u1 = (s0 + d0) / 2,
+  // the same for u2, u3): no register holds the row's u itself until it closes.
+  static __device__ __forceinline__ void src_share(const K2& k, float2 xa01, float2 xa23, float2 xb01,
+                                                   float2 xb23, float2 wy, Row2T& row) {
+    row.lb01 = fma2(k.yc, add2(xa01, xb01), mul2(wy, row.fx01));
+    row.lb23 = fma2(k.yc, add2(xa23, xb23), mul2(wy, row.fx23));
+    const float2 ls = f2(row.lb01.x + row.lb01.y, row.lb23.x + row.lb23.y);
+    const float2 ld = f2(row.lb01.y - row.lb01.x, row.lb23.y - row.lb23.x);
+    const float2 le = fma2(f2(row.u.s01.x, row.u.s23.x), ls, mul2(f2(row.u.d01.x, row.u.d23.x), ld));
+    row.lE = 0.5f * (le.x + le.y);
   }
 
   // Element row between `top` and `bot`: adds its gradient to At (top nodes) and WRITES Ab
@@ -253,18 +275,16 @@ struct Fem2T {
   static __device__ __forceinline__ float elem_row(const K2& k, const Row2T& top, const Row2T& bot,
                                                    float2 vw01, float2 vw23, Acc2T& At, Acc2T& Ab) {
     float2 ga, gb, gc, gd;
-    const float2 E0 = elem_pair<HAS_NU, HAS_F>(k, top.u.s01, top.u.d01, bot.u.s01, bot.u.d01,
-                                              top.n.s01, top.n.d01, bot.n.s01, bot.n.d01,
-                                              top.f.s01, top.f.d01, bot.f.s01, bot.f.d01, vw01,
-                                              ga, gb, gc, gd);
+    const float2 E0 = elem_pair<HAS_NU>(k, top.u.s01, top.u.d01, bot.u.s01, bot.u.d01,
+                                        top.n.s01, top.n.d01, bot.n.s01, bot.n.d01, vw01,
+                                        ga, gb, gc, gd);
     At.a01 = add2(At.a01, ga);
     At.a01.y += gb.x; At.a23.x += gb.y;
     Ab.a01 = gc; Ab.a01.y += gd.x;
     const float carry = gd.y;
-    const float2 E1 = elem_pair<HAS_NU, HAS_F>(k, top.u.s23, top.u.d23, bot.u.s23, bot.u.d23,
-                                              top.n.s23, top.n.d23, bot.n.s23, bot.n.d23,
-                                              top.f.s23, top.f.d23, bot.f.s23, bot.f.d23, vw23,
-                                              ga, gb, gc, gd);
+    const float2 E1 = elem_pair<HAS_NU>(k, top.u.s23, top.u.d23, bot.u.s23, bot.u.d23,
+                                        top.n.s23, top.n.d23, bot.n.s23, bot.n.d23, vw23,
+                                        ga, gb, gc, gd);
     At.a23 = add2(At.a23, ga);
     At.a23.y += gb.x; At.a4 += gb.y;
     Ab.a23 = gc; Ab.a23.x += carry; Ab.a23.y += gd.x;
@@ -388,23 +408,25 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
   const int nrows = j_last - j_first + 1;          // node rows streamed: >= 2
   const int nst = (nrows + 1) >> 1;                // stages streamed (the last may hold one row)
 
-  // ---- producer: thread 0 copies, per stage, two rows of every field (one bulk copy per field)
+  // ---- producer: thread 0 copies, per stage, two rows of every field (one bulk copy per field).  The source rows
+  // of the next stage start where the last stage's ended (stride_y == nx is an eligibility condition of this path):
+  // the field addresses are set up once and advance by two rows per stage.
+  const uint32_t row_bytes = (uint32_t)(nx * 4);
+  const float* src[NF];
+#pragma unroll
+  for (int f = 0; f < NF; ++f) src[f] = p.fld[f].p + (long long)b * p.fld[f].sb + (long long)j_first * nx;
   int issued = 0, ist = 0;
   auto issue_stage = [&]() {
     if (tid == 0) {
-      const int r0 = 2 * issued;
-      const int nr = min(2, nrows - r0);
-      const uint32_t row_bytes = (uint32_t)(nx * 4);
+      const uint32_t nr_bytes = (issued + 1 < nst || !(nrows & 1)) ? 2 * row_bytes : row_bytes;
       uint64_t* bar = full + ist;
       float* dst = ring + ist * stage_floats;
-      mbar_arrive_expect_tx(bar, (uint32_t)(NF * nr) * row_bytes);
+      mbar_arrive_expect_tx(bar, (uint32_t)NF * nr_bytes);
 #pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        // rows are contiguous in memory (stride_y == nx is an eligibility condition of this path)
-        const float* src = p.fld[f].p + (long long)b * p.fld[f].sb + (long long)(j_first + r0) * nx;
-        bulk_g2s(dst + f * 2 * nx, src, (uint32_t)nr * row_bytes, bar);
-      }
+      for (int f = 0; f < NF; ++f) bulk_g2s(dst + f * 2 * nx, src[f], nr_bytes, bar);
     }
+#pragma unroll
+    for (int f = 0; f < NF; ++f) src[f] += 2 * nx;
     ++issued;
     ist = (ist + 1 == S) ? 0 : ist + 1;
   };
@@ -422,10 +444,14 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
 
   const bool act = tid * 4 < nx;
   const int x0 = act ? tid * 4 : 0;          // idle lanes of the last warp shadow lane 0 (results dropped)
-  const bool has_right = (x0 + 4) < nx;
+  const bool has_right = (x0 + 4) < nx, has_left = x0 > 0;
   const float2 vw01 = f2(1.f, 1.f);
   const float2 vw23 = f2(1.f, has_right ? 1.f : 0.f);
   const K2& k = p.k2;
+  // FK == 1: the y-stencil's own weight in the image's top and bottom row, and the x-stencil of the row above the
+  // next row to close (zero above row 0)
+  const float2 wy_edge = mul2(f2(0.5f), k.yw);
+  float2 xc01 = f2(0.f), xc23 = f2(0.f);
   const bool seam_in = (lane == 0) && (warp > 0);
 
   double acc = 0.0;
@@ -440,22 +466,25 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
     const float fromL = __shfl_up_sync(0xffffffffu, A.a4, 1);
     float2 g01 = A.a01, g23 = A.a23;
     if (lane > 0) g01.x += fromL;
-    if constexpr (F::LV) { g01 = add2(g01, row.lb01); g23 = add2(g23, row.lb23); }
+    if constexpr (F::NODAL) { g01 = add2(g01, row.lb01); g23 = add2(g23, row.lb23); }
     g01 = mul2(g01, row.keep01);
     g23 = mul2(g23, row.keep23);
     G = make_float4(g01.x, g01.y, g23.x, g23.y);
   };
-  // branch-free: a predicated 16-byte store, the residual-form square sum selected into `pend` (added to the
-  // fp64 accumulator together with the next stage's energy).  `inr`: the row is owned by this chunk -- a
-  // compile-time true everywhere but in the first stage.
-  const bool wr = act && (gout != nullptr), rs = act && (p.mode != 0), en = act && (p.mode == 0);
+  // branch-free: a predicated 16-byte store; the residual form's square sum (RES) or the row's source energy
+  // selected into `pend` (added to the fp64 accumulator together with the next stage's energy).  `inr`: the row
+  // is owned by this chunk -- a compile-time true everywhere but in the first stage.
+  const bool wr = act && (gout != nullptr);
   float pend = 0.f;
-  auto store_row = [&](float4 G, float keep0, float seam_v, const int jr, const bool inr, const float le) {
+  auto store_row = [&](auto res_c, float4 G, float keep0, float seam_v, const int jr, const bool inr, const float le) {
     G.x += seam_in ? seam_v * keep0 : 0.f;
     if (inr && wr) *reinterpret_cast<float4*>(gout + (long long)(jr - j_first) * nx) = G;
-    const float sq = G.x * G.x + G.y * G.y + G.z * G.z + G.w * G.w;
-    pend += (inr && rs) ? sq : 0.f;
-    if constexpr (F::LV) pend += (inr && en) ? le : 0.f;      // the row's load-vector energy, once, by its owner
+    if constexpr (decltype(res_c)::value) {
+      const float sq = G.x * G.x + G.y * G.y + G.z * G.z + G.w * G.w;
+      pend += (inr && act) ? sq : 0.f;
+    } else if constexpr (F::NODAL) {
+      pend += (inr && act) ? le : 0.f;     // the row's source energy, once, by its owner
+    }
   };
 
   Row2T rowA, rowB;          // even node rows of the chunk live in A, odd ones in B
@@ -467,9 +496,9 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
   // row, the only place a halo row must not be stored), the steady loop (every check of the general body is a
   // compile-time constant there: one straight-line block per stage between the data wait and the CTA barrier,
   // so the two rows' shared loads, masks and element pairs can be scheduled across each other), and the trailing
-  // half stage of a chunk that streams an odd number of rows.
-  auto stage = [&](auto first_c, auto odd_c, const int q) {
-    constexpr bool FIRST = decltype(first_c)::value, HAS_ODD = decltype(odd_c)::value;
+  // half stage of a chunk that streams an odd number of rows.  RES (res_c): the loss is the residual form.
+  auto stage = [&](auto first_c, auto odd_c, auto res_c, const int q) {
+    constexpr bool FIRST = decltype(first_c)::value, HAS_ODD = decltype(odd_c)::value, RES = decltype(res_c)::value;
     mbar_wait(full + st, phase);
     const float* sp = sbase + st * stage_floats;
     const int r0 = 2 * q;                              // even row of this stage (chunk-relative)
@@ -478,26 +507,35 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
     float kp0 = 0.f, kp1 = 0.f, e = 0.f, le0 = 0.f, le1 = 0.f;
 
     // ---- even row -> A; element row (B above, A below); node row r0-1 (B) closes
-    F::load_row(p, sp, 2 * nx, has_right, rowA);
+    F::load_row(p, sp, 2 * nx, has_left, has_right, rowA);
     if constexpr (!FIRST) {
       const float e0 = F::elem_row(k, rowB, rowA, vw01, vw23, accB, accA);
       e += (j_first + r0 - 1 >= r_begin) ? e0 : 0.f;
       sts_if(lane == 31, seam + (par * 2 + 0) * nw + warp, accB.a4);
+      if constexpr (F::HAS_F) {
+        F::src_share(k, xc01, xc23, rowA.fx01, rowA.fx23, k.yw, rowB);
+        xc01 = rowB.fx01; xc23 = rowB.fx23;
+      }
       close_row(accB, rowB, G0);
       kp0 = rowB.keep01.x;
-      if constexpr (F::LV) le0 = rowB.lE;
+      if constexpr (F::NODAL) le0 = rowB.lE;
     }
     // ---- odd row -> B; element row (A above, B below); node row r0 (A) closes
     if constexpr (HAS_ODD) {
-      F::load_row(p, sp + nx, 2 * nx, has_right, rowB);
+      F::load_row(p, sp + nx, 2 * nx, has_left, has_right, rowB);
       const float e1 = F::elem_row(k, rowA, rowB, vw01, vw23, accA, accB);
       e += (j_first + r0 >= r_begin) ? e1 : 0.f;
       sts_if(lane == 31, seam + (par * 2 + 1) * nw + warp, accA.a4);
+      if constexpr (F::HAS_F) {
+        // FIRST: row j_first is the image's top row, or a halo row this chunk does not store
+        F::src_share(k, xc01, xc23, rowB.fx01, rowB.fx23, FIRST ? wy_edge : k.yw, rowA);
+        xc01 = rowA.fx01; xc23 = rowA.fx23;
+      }
       close_row(accA, rowA, G1);
       kp1 = rowA.keep01.x;
-      if constexpr (F::LV) le1 = rowA.lE;
+      if constexpr (F::NODAL) le1 = rowA.lE;
     }
-    acc += (double)(((p.mode == 0 && act) ? e : 0.f) + pend);
+    acc += (double)(((!RES && act) ? e : 0.f) + pend);
     pend = 0.f;
     __syncthreads();      // stage consumed by every thread; seam words of both rows visible
     if (issued < nst) issue_stage();
@@ -507,29 +545,36 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
     const int wl = warp > 0 ? warp - 1 : 0;
     const float s0 = seam[(par * 2 + 0) * nw + wl];
     const float s1 = seam[(par * 2 + 1) * nw + wl];
-    if constexpr (!FIRST) store_row(G0, kp0, s0, j_first + r0 - 1, true, le0);
-    if constexpr (HAS_ODD) store_row(G1, kp1, s1, j_first + r0, FIRST ? (j_first >= r_begin) : true, le1);
+    if constexpr (!FIRST) store_row(res_c, G0, kp0, s0, j_first + r0 - 1, true, le0);
+    if constexpr (HAS_ODD) store_row(res_c, G1, kp1, s1, j_first + r0, FIRST ? (j_first >= r_begin) : true, le1);
   };
-  const int nfull = nrows >> 1;                        // >= 1: a chunk streams at least two rows
-  stage(std::true_type{}, std::true_type{}, 0);
-  for (int q = 1; q < nfull; ++q) stage(std::false_type{}, std::true_type{}, q);
-  if (nrows & 1) stage(std::false_type{}, std::false_type{}, nfull);
+  // The whole march exists once per loss form (one uniform branch on p.mode): the energy march carries no square
+  // sums, the residual march no element energies.
+  auto march = [&](auto res_c) {
+    const int nfull = nrows >> 1;                        // >= 1: a chunk streams at least two rows
+    stage(std::true_type{}, std::true_type{}, res_c, 0);
+    for (int q = 1; q < nfull; ++q) stage(std::false_type{}, std::true_type{}, res_c, q);
+    if (nrows & 1) stage(std::false_type{}, std::false_type{}, res_c, nfull);
 
-  // ---- last node row of the image: no element row below it; its sum is already complete
-  if (r_end == p.ny) {
-    const bool lastB = (nrows & 1) == 0;             // the last streamed row is odd -> lives in B
-    const Acc2T& A = lastB ? accB : accA;
-    const Row2T& row = lastB ? rowB : rowA;
-    const int par = nst & 1;
-    if (lane == 31) seam[(par * 2) * nw + warp] = A.a4;
-    float4 G;
-    close_row(A, row, G);
-    __syncthreads();
-    const float sv = seam_in ? seam[(par * 2) * nw + warp - 1] : 0.f;
-    float le = 0.f;
-    if constexpr (F::LV) le = row.lE;
-    store_row(G, row.keep01.x, sv, p.ny - 1, true, le);
-  }
+    // ---- last node row of the image: no element row below it; its sum is already complete
+    if (r_end == p.ny) {
+      const bool lastB = (nrows & 1) == 0;             // the last streamed row is odd -> lives in B
+      const Acc2T& A = lastB ? accB : accA;
+      Row2T row = lastB ? rowB : rowA;
+      const int par = nst & 1;
+      if (lane == 31) seam[(par * 2) * nw + warp] = A.a4;
+      if constexpr (F::HAS_F) F::src_share(k, xc01, xc23, f2(0.f), f2(0.f), wy_edge, row);
+      float4 G;
+      close_row(A, row, G);
+      __syncthreads();
+      const float sv = seam_in ? seam[(par * 2) * nw + warp - 1] : 0.f;
+      float le = 0.f;
+      if constexpr (F::NODAL) le = row.lE;
+      store_row(res_c, G, row.keep01.x, sv, p.ny - 1, true, le);
+    }
+  };
+  if (p.mode != 0) march(std::true_type{});
+  else march(std::false_type{});
   acc += (double)pend;
 
   // all streaming done: the next grid in the stream may start launching behind our epilogue

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""tools/sass_cost.py <lib.so|cubin> <function-regex> [--loops N] -- static dispatch-cost estimate of a kernel's
+"""tools/sass_cost.py <lib.so|cubin|.o> <function-regex> [--loops N] [--stage] -- static dispatch-cost estimate of a kernel's
 innermost loops from its SASS (no GPU needed).
 
 Cost model measured on B200 with tools/micro/fp32_mix.cu and pipe_mix.cu: one sub-partition dispatches
@@ -10,6 +10,13 @@ do NOT overlap (FADD2 + LOP3 + IADD3 = 4.8 cycles, not 2.4).  So the estimate is
 
 Prints, for each of the N largest loops (backward branches): instructions, estimated cycles per
 iteration, and the opcode histogram.
+
+--stage picks instead the loops that enclose exactly ONE BAR.SYNC: the steady row-stage loops of the
+streaming kernels (their data-wait retry loops branch back from the end of the function and enclose
+several barriers).  k_fem2d_tma has two, one per loss form: the energy march is the one with FFMA2-heavy
+element energies, the residual march the one with the scalar square sums.  It also prints how many of
+each loop's instructions follow the barrier (warp 0 runs the ring refill there, before its next wait).
+    python tools/sass_cost.py diffnet_b200/build/fem2dt_mk2.o 'ILi2ELb0ELb1ELi1ELb0ELb1ELi512' --stage
 """
 import collections
 import re
@@ -55,6 +62,7 @@ def main():
         a, b = sys.argv[sys.argv.index("--range") + 1].split(":")
         rng = (int(a, 16), int(b, 16))
     show_back = "--branches" in sys.argv
+    stage = "--stage" in sys.argv
     txt = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True).stdout
     funcs = re.split(r"\n\s*Function : ", txt)
     for f in funcs[1:]:
@@ -77,8 +85,14 @@ def main():
         loops.sort(key=lambda ab: ab[0] - ab[1])
         if show_back:
             print("   backward branches:", ", ".join(f"{lo:#x}..{hi:#x}" for lo, hi in sorted(loops)))
+        bars = [a for a, o, _ in ins if o.startswith("BAR.SYNC")]
+        if stage:
+            loops = [(lo, hi) for lo, hi in loops if sum(lo <= b <= hi for b in bars) == 1]
         for lo, hi in ([rng] if rng else loops[:nloops]):
             body = [(a, o, g) for a, o, g in ins if lo <= a <= hi]
+            if stage:
+                bar = next(b for b in bars if lo <= b <= hi)
+                print(f"   stage loop: {sum(a > bar for a, _, _ in body)} of its instructions follow the BAR.SYNC")
             hist = collections.Counter()
             cyc = 0.0
             for a, o, g in body:
