@@ -55,6 +55,10 @@ _RESID_ARGS = [_P(dn_field), _P(dn_field), _P(dn_field), _P(dn_mask), C.c_int, C
 _GP_ARGS = [_P(dn_field), _P(dn_geom), C.c_int, C.c_void_p, C.c_void_p]
 _GPADJ_ARGS = [C.c_void_p, _P(dn_geom), C.c_int, C.c_void_p, C.c_void_p]
 _GPM_ARGS = [_P(dn_field), _P(dn_geom), C.c_int, _P(C.c_int), _P(C.c_void_p), C.c_void_p]
+_EIG_ARGS = [_P(dn_field), _P(dn_field), _P(dn_field), _P(dn_field), _P(dn_mask), C.c_int, _P(dn_field),
+             _P(dn_geom), _P(dn_consts), C.c_void_p, C.c_void_p, _P(C.c_void_p), C.c_void_p]
+_RIG_ARGS = [_P(dn_field), _P(dn_field), _P(dn_field), _P(dn_field), _P(dn_mask), C.c_int, _P(dn_geom), C.c_double,
+             C.c_void_p, C.c_void_p, _P(C.c_void_p), C.c_void_p]
 _GPMADJ_ARGS = [_P(C.c_void_p), _P(dn_geom), C.c_int, _P(C.c_int), C.c_void_p, C.c_void_p]
 
 # symbol -> (restype, argtypes); tests/test_abi.py checks this table against include/diffnet_fem.h
@@ -74,6 +78,10 @@ PROTOTYPES = {
                                        C.c_void_p]),
     "dn_fem_residual_2d_f32": (C.c_int, _RESID_ARGS),
     "dn_fem_residual_3d_f32": (C.c_int, _RESID_ARGS),
+    "dn_fem_energy_input_grads_2d_f32": (C.c_int, _EIG_ARGS),
+    "dn_fem_energy_input_grads_3d_f32": (C.c_int, _EIG_ARGS),
+    "dn_fem_residual_input_grads_2d_f32": (C.c_int, _RIG_ARGS),
+    "dn_fem_residual_input_grads_3d_f32": (C.c_int, _RIG_ARGS),
     "dn_fem_gp_eval_2d_f32": (C.c_int, _GP_ARGS),
     "dn_fem_gp_eval_3d_f32": (C.c_int, _GP_ARGS),
     "dn_fem_gp_eval_adj_2d_f32": (C.c_int, _GPADJ_ARGS),

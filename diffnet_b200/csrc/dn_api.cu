@@ -10,6 +10,7 @@
 #include "fem2d_tma.cuh"
 #include "fem3d.cuh"
 #include "gp_eval.cuh"
+#include "input_grads.cuh"
 
 namespace dn {
 int debug_plan3t(const dn_geom* g, int nfields, int has_nu, int64_t* out);
@@ -551,6 +552,145 @@ int dn_fem_residual_3d_f32(const dn_field* u, const dn_field* nu, const dn_field
   return run3d(cm.u, cm.nu, cm.f, cm.fgp, cm.numask, cm.mk, cm.MK, cm.k, cm.rule, cm.vec4, g,
                residual, 1, apply_masks_to_input ? 1 : 0, workspace, workspace_bytes, loss_out,
                loss_out_f32, stream, sms);
+}
+
+// ------------------------------------------------------------------------------------ input gradients
+static double mean_count(const dn_geom* g, int nsd, int reduction) {
+  if (reduction != 0) return 1.0;
+  if (g->mean_count > 0) return g->mean_count;
+  return (double)g->batch * (g->nx - 1) * (double)(g->ny - 1) * (nsd == 3 ? (double)(g->nz - 1) : 1.0);
+}
+
+static int ingrad_common(int nsd, const dn_field* u, const dn_field* nu, const dn_field* f, const dn_field* fgp,
+                         const dn_mask* masks, int nmasks, const dn_geom* g, float* const* grad_values, InGrad* q) {
+  if (!g) return fail(DN_EINVAL, "geom is NULL");
+  if (g->nsd != nsd) return fail(DN_EINVAL, "geom.nsd=%d but the %d-D entry point was called", g->nsd, nsd);
+  if (g->batch < 1 || g->nx < 2 || g->ny < 2 || (nsd == 3 && g->nz < 2))
+    return fail(DN_EINVAL, "need batch >= 1 and >= 2 nodes per direction (B=%d nx=%d ny=%d nz=%d)",
+                g->batch, g->nx, g->ny, g->nz);
+  if (!(g->hx > 0) || !(g->hy > 0) || (nsd == 3 && !(g->hz > 0)))
+    return fail(DN_EINVAL, "element sizes must be positive");
+  if (g->z_own_hi > g->z_own_lo)
+    return fail(DN_EINVAL, "input gradients are not available under z-slab ownership (z_own_lo/hi set): a slab "
+                           "would only hold a partial gradient");
+  if (!u || !u->ptr) return fail(DN_EINVAL, "u is NULL");
+  if (nmasks < 0 || nmasks > DN_MAX_MASKS) return fail(DN_EINVAL, "nmasks=%d (max %d)", nmasks, DN_MAX_MASKS);
+  if (nmasks > 0 && !masks) return fail(DN_EINVAL, "masks is NULL");
+  double gx[4], gw[4];
+  if (gauss_rule(g->ngp_1d, gx, gw)) return fail(DN_EINVAL, "ngp_1d=%d (2..4)", g->ngp_1d);
+  memset(q, 0, sizeof(*q));
+  const bool bat = g->batch > 1;
+  q->B = g->batch; q->nx = g->nx; q->ny = g->ny; q->nz = (nsd == 3) ? g->nz : 1;
+  q->u = to_field(u); q->nu = to_field(nu); q->f = to_field(f);
+  if (fgp && fgp->ptr) {
+    const long long nel = (long long)(g->nx - 1) * (g->ny - 1) * (nsd == 3 ? g->nz - 1 : 1);
+    long long ngp = 1;
+    for (int d = 0; d < nsd; ++d) ngp *= g->ngp_1d;
+    if (bat && fgp->stride_b != 0 && fgp->stride_b != ngp * nel)
+      return fail(DN_EINVAL, "fgp must be dense (stride_b = ngp * elems, or 0)");
+    q->fgp = fgp->ptr;
+    q->fgp_sb = bat ? fgp->stride_b : 0;
+  }
+  q->nmasks = nmasks;
+  for (int i = 0; i < nmasks; ++i) {
+    if (!masks[i].mask.ptr) return fail(DN_EINVAL, "masks[%d].mask is NULL", i);
+    q->mk[i] = Mask{to_field(&masks[i].mask), to_field(&masks[i].value_field), masks[i].value};
+    q->g_v[i] = grad_values ? grad_values[i] : nullptr;
+    if (q->g_v[i] && !q->mk[i].vf.p) return fail(DN_EINVAL, "grad_values[%d] needs masks[%d].value_field", i, i);
+    if (q->g_v[i] && bat && q->mk[i].vf.sb == 0) q->bc |= 8u << i;
+  }
+  q->ng = g->ngp_1d;
+  double W1 = 0, m2 = 0;
+  for (int i = 0; i < 4; ++i) {
+    q->x[i] = i < g->ngp_1d ? (float)gx[i] : 0.f;
+    q->w[i] = i < g->ngp_1d ? (float)gw[i] : 0.f;
+    if (i < g->ngp_1d) { W1 += gw[i]; m2 += gw[i] * gx[i] * gx[i]; }
+  }
+  const double t = m2 / W1;
+  q->ma = (float)(0.25 * W1 * (1.0 + t));
+  q->mc = (float)(0.25 * W1 * (1.0 - t));
+  q->d[0] = (float)(1.0 / g->hx); q->d[1] = (float)(1.0 / g->hy); q->d[2] = nsd == 3 ? (float)(1.0 / g->hz) : 0.f;
+  return DN_OK;
+}
+
+static int energy_input_grads(int nsd, const dn_field* u, const dn_field* nu, const dn_field* f, const dn_field* fgp,
+                              const dn_mask* masks, int nmasks, const dn_field* nu_zero_mask, const dn_geom* g,
+                              const dn_consts* c, float* grad_f, float* grad_fgp, float* const* grad_values,
+                              void* stream) {
+  int sms = 0;
+  if (int rc = device_ok(&sms)) return rc;
+  if (!c) return fail(DN_EINVAL, "consts is NULL");
+  if (c->flags & DN_F_LOAD_VECTOR) return fail(DN_EINVAL, "input gradients take f_gp itself, not DN_F_LOAD_VECTOR");
+  if (f && f->ptr && fgp && fgp->ptr) return fail(DN_EINVAL, "give f or fgp, not both");
+  InGrad q;
+  if (int rc = ingrad_common(nsd, u, nu, f, fgp, masks, nmasks, g, grad_values, &q)) return rc;
+  q.numask = to_field(nu_zero_mask);
+  if (q.numask.p && !q.nu.p) return fail(DN_EINVAL, "nu_zero_mask needs nu");
+  if (grad_f && !q.f.p) return fail(DN_EINVAL, "grad_f requested without f");
+  if (grad_fgp && !q.fgp) return fail(DN_EINVAL, "grad_fgp requested without fgp");
+  const double S = c->scale / mean_count(g, nsd, c->reduction);
+  q.mode = 0;
+  q.cM = q.cS = q.cG = (float)(-S * c->c_f);
+  q.cK = (float)(2.0 * S * c->c_k);
+  q.g_f = grad_f;
+  q.g_fgp = grad_fgp;
+  if (grad_f && g->batch > 1 && q.f.sb == 0) q.bc |= 1u;
+  if (grad_fgp && g->batch > 1 && q.fgp_sb == 0) q.bc |= 2u;
+  bool any = grad_f || grad_fgp;
+  for (int k = 0; k < nmasks; ++k) any = any || q.g_v[k];
+  if (!any) return DN_OK;
+  return check_cuda(launch_input_grads(q, nsd, sms, (cudaStream_t)stream), "energy input-gradient launch");
+}
+
+static int residual_input_grads(int nsd, const dn_field* u, const dn_field* nu, const dn_field* f,
+                                const dn_field* residual, const dn_mask* masks, int nmasks, const dn_geom* g,
+                                double jac, float* grad_nu, float* grad_f, float* const* grad_values, void* stream) {
+  int sms = 0;
+  if (int rc = device_ok(&sms)) return rc;
+  InGrad q;
+  if (int rc = ingrad_common(nsd, u, nu, f, nullptr, masks, nmasks, g, grad_values, &q)) return rc;
+  if (!residual || !residual->ptr) return fail(DN_EINVAL, "residual is NULL");
+  q.R = to_field(residual);
+  if (grad_nu && !q.nu.p) return fail(DN_EINVAL, "grad_nu requested without nu");
+  if (grad_f && !q.f.p) return fail(DN_EINVAL, "grad_f requested without f");
+  q.mode = 1;
+  q.cM = (float)(-2.0 * jac);
+  q.cK = q.cN = (float)(2.0 * jac);
+  q.g_f = grad_f;
+  q.g_nu = grad_nu;
+  if (grad_f && g->batch > 1 && q.f.sb == 0) q.bc |= 1u;
+  if (grad_nu && g->batch > 1 && q.nu.sb == 0) q.bc |= 4u;
+  bool any = grad_f || grad_nu;
+  for (int k = 0; k < nmasks; ++k) any = any || q.g_v[k];
+  if (!any) return DN_OK;
+  return check_cuda(launch_input_grads(q, nsd, sms, (cudaStream_t)stream), "residual input-gradient launch");
+}
+
+int dn_fem_energy_input_grads_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f, const dn_field* fgp,
+                                     const dn_mask* masks, int nmasks, const dn_field* nu_zero_mask, const dn_geom* g,
+                                     const dn_consts* c, float* grad_f, float* grad_fgp, float* const* grad_values,
+                                     void* stream) {
+  return energy_input_grads(2, u, nu, f, fgp, masks, nmasks, nu_zero_mask, g, c, grad_f, grad_fgp, grad_values,
+                            stream);
+}
+int dn_fem_energy_input_grads_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f, const dn_field* fgp,
+                                     const dn_mask* masks, int nmasks, const dn_field* nu_zero_mask, const dn_geom* g,
+                                     const dn_consts* c, float* grad_f, float* grad_fgp, float* const* grad_values,
+                                     void* stream) {
+  return energy_input_grads(3, u, nu, f, fgp, masks, nmasks, nu_zero_mask, g, c, grad_f, grad_fgp, grad_values,
+                            stream);
+}
+int dn_fem_residual_input_grads_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                       const dn_field* residual, const dn_mask* masks, int nmasks, const dn_geom* g,
+                                       double jac, float* grad_nu, float* grad_f, float* const* grad_values,
+                                       void* stream) {
+  return residual_input_grads(2, u, nu, f, residual, masks, nmasks, g, jac, grad_nu, grad_f, grad_values, stream);
+}
+int dn_fem_residual_input_grads_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                       const dn_field* residual, const dn_mask* masks, int nmasks, const dn_geom* g,
+                                       double jac, float* grad_nu, float* grad_f, float* const* grad_values,
+                                       void* stream) {
+  return residual_input_grads(3, u, nu, f, residual, masks, nmasks, g, jac, grad_nu, grad_f, grad_values, stream);
 }
 
 static int gp_common(const dn_geom* g, int which, int nsd, GpTables* tb) {

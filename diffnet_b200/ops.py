@@ -1,7 +1,7 @@
 """torch.autograd.Function wrappers over the C ABI (the drop-in seam for DiffNet's loss()).
 
-  fem_energy(...)    fused Poisson energy loss, differentiable w.r.t. u (and nu in 2-D)
-  fem_residual(...)  assembled-residual loss  sum(R^2), differentiable w.r.t. u
+  fem_energy(...)    fused Poisson energy loss, differentiable w.r.t. u, nu, f, f_gp and Dirichlet value fields
+  fem_residual(...)  assembled-residual loss  sum(R^2), differentiable w.r.t. u, nu, f and Dirichlet value fields
   gp_eval(...)       gauss_pt_evaluation{,_der_x,_der_y,_der_z}, differentiable w.r.t. its input
 
 Everything runs on the CUDA stream torch considers current; there is no host sync inside and no
@@ -424,6 +424,129 @@ def residual_raw(geom: Geometry, u, nu=None, f=None, dirichlet=(), jac=1.0, appl
     return loss, R
 
 
+def _value_fields(dirichlet):
+    """The tensor Dirichlet values, in list order (the ones autograd can differentiate)."""
+    return tuple(v for _, v in dirichlet if torch.is_tensor(v))
+
+
+def _per_sample(t: Optional[torch.Tensor], B: int) -> Optional[torch.Tensor]:
+    """The canonical view of a field whose gradient is wanted.  The launch writes ONE (1, ...) gradient summed over
+    the batch for a field it reads with stride_b = 0.  A field that spans the batch with stride_b = 0 (``expand``)
+    needs a gradient per sample (autograd's expand backward sums it), so its values are materialised here."""
+    if t is not None and B > 1 and t.shape[0] == B and t.stride(0) == 0:
+        return t.contiguous()
+    return t
+
+
+def _grad_batch(t: torch.Tensor, B: int) -> int:
+    """Batch of the gradient the launch writes for the canonical field ``t`` (after ``_per_sample``)."""
+    return B if (B > 1 and t.shape[0] == B) else 1
+
+
+def _grad_values_dirichlet(dirichlet, want_values, geom: Geometry, B: int):
+    """``dirichlet`` with every differentiated value field in the form ``_per_sample`` gives."""
+    out, it = [], iter(want_values)
+    for i, (m, v) in enumerate(dirichlet):
+        if torch.is_tensor(v) and next(it):
+            v = _per_sample(_canon(v, geom, f"dirichlet[{i}].value"), B)
+        out.append((m, v))
+    return out
+
+
+def _grad_values_arg(dirichlet, want_values, geom: Geometry, B: int, dev):
+    """Output buffers for the wanted value-field gradients: (host pointer array, [(list index, buffer)])."""
+    ptrs = (C.c_void_p * max(len(dirichlet), 1))()
+    outs = []
+    it = iter(want_values)
+    for i, (_, v) in enumerate(dirichlet):
+        if torch.is_tensor(v) and next(it):
+            vc = _canon(v, geom, f"dirichlet[{i}].value")
+            buf = _new_out((_grad_batch(vc, B),) + geom.spatial, dev)
+            ptrs[i] = buf.data_ptr()
+            outs.append((i, buf))
+    return ptrs, outs
+
+
+def energy_input_grads_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None,
+                           c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", mean_count=0.0, want_f=False,
+                           want_f_gp=False, want_values=()):
+    """dL/df, dL/df_gp and dL/d(value field) of the energy loss in ONE launch (dn_fem_energy_input_grads_*).
+    ``want_values``: one flag per tensor Dirichlet value, in list order.  Returns (grad_f | None,
+    grad_f_gp | None, [grad per tensor value | None]); a gradient of a field broadcast over the batch is (1, ...)."""
+    if reduction not in ("mean", "sum"):
+        raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
+    keep = []
+    uc = _canon(u, geom, "u")
+    nuc = _canon(nu, geom, "nu") if nu is not None else None
+    fc = _canon(f, geom, "f") if f is not None else None
+    nzm = _canon(nu_zero_mask, geom, "nu_zero_mask") if nu_zero_mask is not None else None
+    fg = _check_f_gp(geom, f_gp).contiguous() if f_gp is not None else None
+    masks_t = [m for m, _ in dirichlet] + list(_value_fields(dirichlet))
+    B = _batch_of(uc, nuc, fc, nzm, fg, *[_canon(m, geom, "mask") for m in masks_t])
+    if want_f:
+        fc = _per_sample(fc, B)
+    dirichlet = _grad_values_dirichlet(dirichlet, want_values, geom, B)
+    marr, nm = _masks_struct(dirichlet, geom, B, keep)
+    dev = uc.device
+    g = _geom_struct(geom, B, None, mean_count)
+    cs = L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1, 0)
+    gf = _new_out((_grad_batch(fc, B),) + geom.spatial, dev) if want_f else None
+    ngp = geom.ngp_1d ** geom.nsd
+    gfg = _new_out((_grad_batch(fg, B), ngp) + geom.elems, dev) if want_f_gp else None
+    ptrs, gvs = _grad_values_arg(dirichlet, want_values, geom, B, dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    with _on_device(dev):
+        fu, fnu, ff = _field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd)
+        ffg = L.dn_field(None, 0, 0, 0)
+        if fg is not None:
+            ffg = L.dn_field(fg.data_ptr(), fg.stride(0) if (fg.shape[0] == B and B > 1) else 0, 0, 0)
+        fnz = _field(nzm, B, geom.nsd)
+        lib = L.lib()
+        fn = lib.dn_fem_energy_input_grads_2d_f32 if geom.nsd == 2 else lib.dn_fem_energy_input_grads_3d_f32
+        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None, C.byref(ff) if fc is not None else None,
+                C.byref(ffg) if fg is not None else None, marr, nm, C.byref(fnz) if nzm is not None else None,
+                C.byref(g), C.byref(cs), _ptr(gf), _ptr(gfg), ptrs, C.c_void_p(stream))
+    L.check(rc, f"dn_fem_energy_input_grads_{geom.nsd}d_f32")
+    by_index = dict(gvs)
+    vals = [by_index.get(i) for i, (_, v) in enumerate(dirichlet) if torch.is_tensor(v)]
+    return gf, gfg, vals
+
+
+def residual_input_grads_raw(geom: Geometry, u, R, nu=None, f=None, dirichlet=(), jac=1.0, want_nu=False,
+                             want_f=False, want_values=()):
+    """dL/dnu, dL/df and dL/d(value field) of the residual loss sum(R^2) in ONE launch
+    (dn_fem_residual_input_grads_*); ``R`` is the residual the forward returned.  Returns (grad_nu | None,
+    grad_f | None, [grad per tensor value | None])."""
+    keep = []
+    uc = _canon(u, geom, "u")
+    nuc = _canon(nu, geom, "nu") if nu is not None else None
+    fc = _canon(f, geom, "f") if f is not None else None
+    B = R.shape[0]
+    if want_nu:
+        nuc = _per_sample(nuc, B)
+    if want_f:
+        fc = _per_sample(fc, B)
+    dirichlet = _grad_values_dirichlet(dirichlet, want_values, geom, B)
+    marr, nm = _masks_struct(dirichlet, geom, B, keep)
+    dev = uc.device
+    g = _geom_struct(geom, B)
+    gnu = _new_out((_grad_batch(nuc, B),) + geom.spatial, dev) if want_nu else None
+    gf = _new_out((_grad_batch(fc, B),) + geom.spatial, dev) if want_f else None
+    ptrs, gvs = _grad_values_arg(dirichlet, want_values, geom, B, dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    with _on_device(dev):
+        fu, fnu, ff, fr = (_field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd),
+                           _field(R, B, geom.nsd))
+        lib = L.lib()
+        fn = lib.dn_fem_residual_input_grads_2d_f32 if geom.nsd == 2 else lib.dn_fem_residual_input_grads_3d_f32
+        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None, C.byref(ff) if fc is not None else None,
+                C.byref(fr), marr, nm, C.byref(g), float(jac), _ptr(gnu), _ptr(gf), ptrs, C.c_void_p(stream))
+    L.check(rc, f"dn_fem_residual_input_grads_{geom.nsd}d_f32")
+    by_index = dict(gvs)
+    vals = [by_index.get(i) for i, (_, v) in enumerate(dirichlet) if torch.is_tensor(v)]
+    return gnu, gf, vals
+
+
 def scale_inplace_(x: torch.Tensor, factor: torch.Tensor) -> torch.Tensor:
     """x *= factor (0-dim device tensor), free when factor == 1 (checked on the device)."""
     _require_cuda(x, "x")
@@ -459,13 +582,25 @@ class FEMEnergyFunction(torch.autograd.Function):
     The gradient buffer is handed to autograd, not copied, and scaling it in place consumes it: a
     SECOND backward through the same node (``retain_graph=True``, or ``autograd.grad`` followed by
     ``backward``) raises instead of silently returning ``grad_output**2 * dL/du`` -- re-run the
-    forward (one launch) to differentiate again."""
+    forward (one launch) to differentiate again.
+
+    The tensor Dirichlet values follow the fixed arguments (``*values``, list order) so that autograd tracks them.
+    When ``f``, ``f_gp`` or a value requires grad, backward runs ONE more launch (dn_fem_energy_input_grads_*) for
+    those gradients; the inputs it reads are saved for backward, so an in-place change between forward and
+    backward raises torch's version-counter error."""
 
     @staticmethod
     def forward(ctx, u, nu, geom, f, f_gp, dirichlet, nu_zero_mask, c_k, c_f, scale, reduction,
-                z_own, mean_count):
+                z_own, mean_count, *values):
         need_u = ctx.needs_input_grad[0]
         need_nu = nu is not None and ctx.needs_input_grad[1]
+        need_f = f is not None and ctx.needs_input_grad[3]
+        need_fgp = f_gp is not None and ctx.needs_input_grad[4]
+        need_v = tuple(ctx.needs_input_grad[13:])
+        extra = need_f or need_fgp or any(need_v)
+        if extra and z_own is not None:
+            raise L.DiffNetFEMError("gradients w.r.t. f, f_gp or a Dirichlet value field are not available with "
+                                    "z_own: a z-slab only holds a partial gradient")
         loss, grad, grad_nu = energy_raw(
             geom, u.detach(), None if nu is None else nu.detach(), f, f_gp, dirichlet,
             nu_zero_mask, c_k, c_f, scale, reduction, want_grad=need_u or need_nu,
@@ -473,9 +608,15 @@ class FEMEnergyFunction(torch.autograd.Function):
         ctx.geom = geom
         ctx.u_ref = u if need_u else None
         ctx.nu_ref = nu if need_nu else None
-        ctx.save_for_backward(*[t for t in (grad if need_u else None, grad_nu) if t is not None])
+        head = [t for t in (grad if need_u else None, grad_nu) if t is not None]
         ctx.has = (need_u, need_nu)
         ctx.consumed = False
+        ctx.nvalues = len(values)
+        ctx.extra = None
+        if extra:
+            ctx.extra = (need_f, need_fgp, need_v, len(head), dirichlet, c_k, c_f, scale, reduction, mean_count)
+            head += [u, nu, f, f_gp, nu_zero_mask] + [m for m, _ in dirichlet] + list(values)
+        ctx.save_for_backward(*head)
         return loss
 
     @staticmethod
@@ -492,28 +633,69 @@ class FEMEnergyFunction(torch.autograd.Function):
             gu = _like_input(scale_inplace_(saved.pop(0), gout), ctx.u_ref, ctx.geom)
         if ctx.has[1]:
             gnu = _like_input(scale_inplace_(saved.pop(0), gout), ctx.nu_ref, ctx.geom)
-        return (gu, gnu) + (None,) * 11
+        if ctx.extra is None:
+            return (gu, gnu) + (None,) * (11 + ctx.nvalues)
+        need_f, need_fgp, need_v, _, dirichlet, c_k, c_f, scale, reduction, mean_count = ctx.extra
+        u, nu, f, f_gp, nzm = saved[:5]
+        values = saved[5 + len(dirichlet):]
+        gf, gfg, gv = energy_input_grads_raw(ctx.geom, u, nu, f, f_gp, dirichlet, nzm, c_k, c_f, scale, reduction,
+                                             mean_count, want_f=need_f, want_f_gp=need_fgp, want_values=need_v)
+        if gf is not None:
+            gf = _like_input(scale_inplace_(gf, gout), f, ctx.geom)
+        if gfg is not None:
+            gfg = scale_inplace_(gfg, gout).reshape(f_gp.shape)
+        gv = [None if g is None else _like_input(scale_inplace_(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
+        return (gu, gnu, None, gf, gfg) + (None,) * 8 + tuple(gv)
 
 
 class FEMResidualFunction(torch.autograd.Function):
     """loss = sum(R^2); dL/du = mask( K(nu) (2R) ) -- one more pass of the same operator
-    (K is symmetric; R is already zero on the Dirichlet nodes)."""
+    (K is symmetric; R is already zero on the Dirichlet nodes).
+
+    The tensor Dirichlet values follow the fixed arguments (``*values``).  When ``nu``, ``f`` or a value requires
+    grad, backward runs ONE more launch (dn_fem_residual_input_grads_*) for those gradients."""
 
     @staticmethod
-    def forward(ctx, u, geom, nu, f, dirichlet, jac):
+    def forward(ctx, u, geom, nu, f, dirichlet, jac, *values):
         loss, R = residual_raw(geom, u.detach(), nu, f, dirichlet, jac, True)
         ctx.geom, ctx.nu, ctx.dirichlet, ctx.jac, ctx.u_ref = geom, nu, dirichlet, jac, u
-        ctx.save_for_backward(R)
+        ctx.nvalues = len(values)
+        need_nu = nu is not None and ctx.needs_input_grad[2]
+        need_f = f is not None and ctx.needs_input_grad[3]
+        need_v = tuple(ctx.needs_input_grad[6:])
+        ctx.extra = None
+        if need_nu or need_f or any(need_v):
+            ctx.extra = (need_nu, need_f, need_v)
+            ctx.save_for_backward(R, u, nu, f, *[m for m, _ in dirichlet], *values)
+        else:
+            ctx.save_for_backward(R)
         return loss
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, gout):
-        (R,) = ctx.saved_tensors
-        _, KR = residual_raw(ctx.geom, R, ctx.nu, None, ctx.dirichlet, ctx.jac, False)
-        g = KR.mul_(2.0)
-        g = scale_inplace_(g, gout)
-        return (_like_input(g, ctx.u_ref, ctx.geom),) + (None,) * 5
+        saved = ctx.saved_tensors
+        R = saved[0]
+        if ctx.extra is None:
+            _, KR = residual_raw(ctx.geom, R, ctx.nu, None, ctx.dirichlet, ctx.jac, False)
+            g = KR.mul_(2.0)
+            g = scale_inplace_(g, gout)
+            return (_like_input(g, ctx.u_ref, ctx.geom),) + (None,) * (5 + ctx.nvalues)
+        need_nu, need_f, need_v = ctx.extra
+        u, nu, f = saved[1:4]
+        values = saved[4 + len(ctx.dirichlet):]
+        gu = None
+        if ctx.needs_input_grad[0]:
+            _, KR = residual_raw(ctx.geom, R, nu, None, ctx.dirichlet, ctx.jac, False)
+            gu = _like_input(scale_inplace_(KR.mul_(2.0), gout), ctx.u_ref, ctx.geom)
+        gnu, gf, gv = residual_input_grads_raw(ctx.geom, u, R, nu, f, ctx.dirichlet, ctx.jac, want_nu=need_nu,
+                                               want_f=need_f, want_values=need_v)
+        if gnu is not None:
+            gnu = _like_input(scale_inplace_(gnu, gout), nu, ctx.geom)
+        if gf is not None:
+            gf = _like_input(scale_inplace_(gf, gout), f, ctx.geom)
+        gv = [None if g is None else _like_input(scale_inplace_(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
+        return (gu, None, gnu, gf, None, None) + tuple(gv)
 
 
 _WHICH = {"N": 0, "dx": 1, "dy": 2, "dz": 3}
@@ -675,9 +857,11 @@ def gp_eval_general(t: torch.Tensor, nsd: int, nbf_1d: int, ngp_1d: int, factors
 def fem_energy(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet: Sequence = (),
                nu_zero_mask=None, c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", z_own=None,
                mean_count=0.0) -> torch.Tensor:
-    """Fused Poisson energy loss (SURVEY.md App. A.4), differentiable w.r.t. u and (2-D) nu."""
-    return FEMEnergyFunction.apply(u, nu, geom, f, f_gp, tuple(dirichlet), nu_zero_mask, c_k, c_f,
-                                   scale, reduction, z_own, mean_count)
+    """Fused Poisson energy loss (SURVEY.md App. A.4), differentiable w.r.t. u, nu, f, f_gp and the tensor
+    Dirichlet values (the last three not with ``z_own``)."""
+    dirichlet = tuple(dirichlet)
+    return FEMEnergyFunction.apply(u, nu, geom, f, f_gp, dirichlet, nu_zero_mask, c_k, c_f,
+                                   scale, reduction, z_own, mean_count, *_value_fields(dirichlet))
 
 
 def fem_energy_and_grad(geom: Geometry, u, **kw):
@@ -687,7 +871,9 @@ def fem_energy_and_grad(geom: Geometry, u, **kw):
 
 
 def fem_residual(geom: Geometry, u, nu=None, f=None, dirichlet: Sequence = (), jac=1.0) -> torch.Tensor:
-    return FEMResidualFunction.apply(u, geom, nu, f, tuple(dirichlet), jac)
+    """sum(R^2) of the assembled residual, differentiable w.r.t. u, nu, f and the tensor Dirichlet values."""
+    dirichlet = tuple(dirichlet)
+    return FEMResidualFunction.apply(u, geom, nu, f, dirichlet, jac, *_value_fields(dirichlet))
 
 
 def gp_eval(geom: Geometry, t: torch.Tensor, which: str = "N") -> torch.Tensor:

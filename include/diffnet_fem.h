@@ -19,6 +19,8 @@
  *   dn_fem_gp_eval_{2d,3d}_f32  gauss_pt_eval / gauss_pt_evaluation* themselves
  *   dn_fem_gp_eval_adj_*        (DiffNetFEM.py:7-18,143-156) and their autograd backward
  *                               (convolution_backward = scatter-transpose).
+ *   dn_fem_{energy,residual}_input_grads_*  the same bodies' autograd backward w.r.t. the source, the forcing at
+ *                               the Gauss points, the Dirichlet value fields and (residual) nu.
  *   dn_scale_inplace_f32        autograd's  grad_input = grad_output * dL/du.
  *   dn_peer_{put,wait}_f32      (no reference counterpart) one-plane halo exchange of the z-slab
  *                               decomposition through NVLink peer memory.
@@ -210,6 +212,47 @@ int dn_fem_residual_3d_f32(const dn_field* u, const dn_field* nu, const dn_field
                            const dn_geom* g, double jac, float* residual, void* workspace,
                            size_t workspace_bytes, double* loss_out, float* loss_out_f32,
                            void* stream);
+
+/*
+ * Gradients of the fused losses with respect to their OTHER inputs -- what autograd gives the reference's loss()
+ * bodies for a source, forcing, Dirichlet value field or diffusivity that requires grad (inverse problems, optimal
+ * control, coefficient identification).  ONE launch produces every requested output; each output pointer may be NULL
+ * (not wanted).  Notation of dn_fem_energy_*: S = scale / count, u' = u with the Dirichlet conditions applied,
+ * M / K(nu) = Q1 mass / stiffness matrices with the rule's reference-element weights (K includes (2/h)^2).
+ * "mask k is the last firing mask at n": mask k fires at n and no later mask of the list does.
+ *
+ * dn_fem_energy_input_grads_*   (the autograd backward of the loss() bodies listed at dn_fem_energy_*, w.r.t.
+ *                               forcing_tensor / f_gp / a value field, e8_2d_poisson_mms.py:154-175)
+ *   grad_f[b,n]       = -S c_f (M u')[b,n]                          (f required; NOT zeroed at Dirichlet nodes)
+ *   grad_fgp[b,G,e]   = -S c_f w_G u'_G(e)                          (fgp required; dense like fgp)
+ *   grad_values[k][b,n] = [k last firing at n] * S (2 c_k K(nu') u' - c_f (M f | sum_e sum_g w_g N_n f_gp))[b,n]
+ *                                                                   (masks[k].value_field required)
+ * dn_fem_residual_input_grads_* (the autograd backward of 12_klsum.py:80-132 w.r.t. nu, forcing, a value field)
+ *   residual: the R that dn_fem_residual_*_f32 returned for the same inputs (dense (B, nz, ny, nx))
+ *   grad_nu[b,n]      = 2 jac sum_{e around n} sum_g w_g N_n(g) grad u'_g . grad R_g     (nu required)
+ *   grad_f[b,n]       = -2 jac (M R)[b,n]                                                (f required)
+ *   grad_values[k][b,n] = [k last firing at n] * 2 jac (K(nu) R)[b,n]
+ * Output shapes: dense (B, nz, ny, nx) -- or (1, nz, ny, nx), summed over the batch in a fixed order, when the
+ * differentiated field has stride_b == 0 and batch > 1.  grad_values is a HOST array of nmasks pointers (or NULL).
+ * Gather form, no atomics: bit-reproducible.  No workspace.  z-slab ownership (z_own_lo/hi set) and
+ * DN_F_LOAD_VECTOR are rejected with DN_EINVAL (pass f_gp itself).
+ */
+int dn_fem_energy_input_grads_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                     const dn_field* fgp, const dn_mask* masks, int nmasks,
+                                     const dn_field* nu_zero_mask, const dn_geom* g, const dn_consts* c,
+                                     float* grad_f, float* grad_fgp, float* const* grad_values, void* stream);
+int dn_fem_energy_input_grads_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                     const dn_field* fgp, const dn_mask* masks, int nmasks,
+                                     const dn_field* nu_zero_mask, const dn_geom* g, const dn_consts* c,
+                                     float* grad_f, float* grad_fgp, float* const* grad_values, void* stream);
+int dn_fem_residual_input_grads_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                       const dn_field* residual, const dn_mask* masks, int nmasks,
+                                       const dn_geom* g, double jac, float* grad_nu, float* grad_f,
+                                       float* const* grad_values, void* stream);
+int dn_fem_residual_input_grads_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                       const dn_field* residual, const dn_mask* masks, int nmasks,
+                                       const dn_geom* g, double jac, float* grad_nu, float* grad_f,
+                                       float* const* grad_values, void* stream);
 
 /*
  * Gauss-point evaluation  out[b, G, elem] = sum_a T_which[G][a] * in[b, node(elem,a)]
