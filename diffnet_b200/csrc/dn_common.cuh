@@ -130,4 +130,6 @@ __device__ __forceinline__ float lds1(const float* __restrict__ p, bool pred) {
 namespace dn {
 int fail(int code, const char* fmt, ...);
 int check_cuda(cudaError_t e, const char* what);
+// Integer tuning knob from the environment, `dflt` when unset or empty.  Read on every call (DESIGN.md §10b).
+int env_int(const char* name, int dflt);
 }  // namespace dn

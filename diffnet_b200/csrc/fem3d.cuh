@@ -507,10 +507,4 @@ cudaError_t launch3d(const P3D& p, dim3 grid, dim3 block, size_t smem, cudaStrea
   return cudaGetLastError();
 }
 
-long long plan3d_max_ctas(const dn_geom* g);
-int run3d(const Field& u, const Field& nu, const Field& f, const Field& fgp, const Field& numask,
-          const Mask* mk, int MK, const Consts& k, const Rule& rule, bool vec4, const dn_geom* g,
-          float* grad, int mode, int mask_input, void* workspace, size_t wsb, double* loss_out,
-          float* loss_f32, void* stream, int sms, const dn_slab_link* link = nullptr);
-
 }  // namespace dn

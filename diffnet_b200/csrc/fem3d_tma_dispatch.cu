@@ -2,8 +2,8 @@
 // (instantiated in gen/fem3dt_mk*.cu).
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
 
+#include "dn_launch.h"
 #include "fem3d.cuh"
 #include "fem3d_tma.cuh"
 #include "fem3d_tma_combos.h"
@@ -31,11 +31,6 @@ occ3t_fn get_occ3t(int MK, int NU, int F, int NUMASK, int LK) {
   DN3T_ALL(DN_CASE)
 #undef DN_CASE
   return nullptr;
-}
-
-static int env_i3(const char* name, int dflt) {
-  const char* s = getenv(name);
-  return (s && *s) ? atoi(s) : dflt;
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no libcuda link dependency)
@@ -98,12 +93,12 @@ static Plan3T plan3t(const dn_geom* g, int nf, int sms, occ3t_fn occ, int maxt_v
   memset(&best, 0, sizeof(best));
   if (g->nx % 4 != 0 || g->nx < 8) return best;
   const int npairs = g->nx / 2;
-  int maxt = env_i3("DN_T3_THREADS", maxt_variant);
+  int maxt = env_int("DN_T3_THREADS", maxt_variant);
   if (maxt > maxt_variant) maxt = maxt_variant;
-  const int lx_forced = env_i3("DN_T3_LX", 0), ty_forced = env_i3("DN_T3_TY", 0), zc_forced = env_i3("DN_T3_ZC", 0);
-  int zmin = env_i3("DN_T3_ZCMIN", 4);
+  const int lx_forced = env_int("DN_T3_LX", 0), ty_forced = env_int("DN_T3_TY", 0), zc_forced = env_int("DN_T3_ZC", 0);
+  int zmin = env_int("DN_T3_ZCMIN", 4);
   if (zmin < 1) zmin = 1;
-  int S0 = env_i3("DN_T3_STAGES", 4);
+  int S0 = env_int("DN_T3_STAGES", 4);
   if (S0 < 2) S0 = 2;
   if (S0 > 8) S0 = 8;
   double best_cost = 0.0;
@@ -140,7 +135,7 @@ static Plan3T plan3t(const dn_geom* g, int nf, int sms, occ3t_fn occ, int maxt_v
       const size_t smem = smem_3t(S, nf, fstride);
       if (smem > (size_t)kMaxDynSmem) continue;
       int cps = occ ? occ(threads, smem) : (int)(65536 / (threads * (maxt_variant > 512 ? 96 : 128)));
-      if (env_i3("DN_DEBUG_PLAN", 0) >= 2)
+      if (env_int("DN_DEBUG_PLAN", 0) >= 2)
         fprintf(stderr, "[plan3t] candidate LXT=%d rows=%d TY=%d threads=%d smem=%zu -> %d CTA/SM\n", LXT, rows, TY,
                 threads, smem, cps);
       if (cps < 1) continue;
@@ -197,25 +192,21 @@ int debug_plan3t(const dn_geom* g, int nfields, int has_nu, int64_t* out) {
   return DN_OK;
 }
 
-int run3t(const Field& u, const Field& nu, const Field& f, const Field& fgp, const Field& numask,
-          const Mask* mk, int nmasks, int MK, const Consts& k, bool vec4, const dn_geom* g, float* grad,
-          int mode, int mask_input, void* workspace, size_t wsb, double* loss_out, float* loss_f32,
-          void* stream, int sms, bool* handled, const dn_slab_link* link) {
+int run3t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
   *handled = false;
   const char* path = getenv("DN_3D_PATH");
   if (path && !strcmp(path, "tile")) return DN_OK;
-  if (!vec4 || fgp.p || ((uintptr_t)grad % 16 != 0)) return DN_OK;
-  const bool iso = nu.p && k.kx == k.ky && k.kx == k.kz && k.kx != 0.f && env_i3("DN_T3_ISO", 1);
-  const bool iso1 = !nu.p && k.kx == k.ky && k.kx == k.kz && env_i3("DN_T3_ISO", 1);
-  const int NU = nu.p ? (iso ? 2 : 1) : (iso1 ? 3 : 0), F = f.p ? (k.lv ? 2 : 1) : 0, NMK = numask.p ? 1 : 0;
+  if (!c.vec4 || c.fgp.p || ((uintptr_t)o.grad % 16 != 0)) return DN_OK;
+  const Field& u = c.u;
+  const Consts& k = c.k;
+  const dn_slab_link* link = c.link;
+  const int sms = c.sms;
+  const bool iso = c.nu.p && k.kx == k.ky && k.kx == k.kz && k.kx != 0.f && env_int("DN_T3_ISO", 1);
+  const bool iso1 = !c.nu.p && k.kx == k.ky && k.kx == k.kz && env_int("DN_T3_ISO", 1);
+  const int NU = c.nu.p ? (iso ? 2 : 1) : (iso1 ? 3 : 0), F = c.f.p ? (k.lv ? 2 : 1) : 0, NMK = c.numask.p ? 1 : 0;
   // the load-vector term is nodal: with z-slab ownership a node plane has no single owner
   if (k.lv && (link || g->z_own_hi > g->z_own_lo)) return DN_OK;
-  int MKx = MK;
-  if (!mask_input) {                     // operator apply: only the plain-mask, no-source variants exist
-    if (MK == 0) MKx = 0;
-    else if (MK >= 1 && MK <= 3 && !F && !NMK) MKx = MK + 4;
-    else return DN_OK;
-  }
+  const int MKx = stream_variant(c, F, NMK);
   launch3t_fn fn = get_launch3t(MKx, NU, F, NMK, link ? 1 : 0);
   occ3t_fn occ = get_occ3t(MKx, NU, F, NMK, link ? 1 : 0);
   if (!fn || !occ || !get_encode()) return DN_OK;
@@ -224,25 +215,23 @@ int run3t(const Field& u, const Field& nu, const Field& f, const Field& fgp, con
   memset(&p, 0, sizeof(p));
   int nf = 0;
   fl[nf++] = u;
-  if (nu.p) fl[nf++] = nu;
-  if (F) fl[nf++] = f;
-  if (NMK) fl[nf++] = numask;
-  for (int i = 0; i < nmasks; ++i) { fl[nf++] = mk[i].m; p.mval[i] = mk[i].v; }
-  if (MK == 4) fl[nf++] = mk[0].vf;
-  const long long min_grid = (link && link->halo_plane[0] && env_i3("DN_SLAB_WAVES", 0)) ? (long long)(1.9 * sms) : 0;
-  Plan3T pl = plan3t(g, nf, sms, occ, DN_T3_MAXT_OF(nu.p != nullptr), min_grid);
+  if (c.nu.p) fl[nf++] = c.nu;
+  if (F) fl[nf++] = c.f;
+  if (NMK) fl[nf++] = c.numask;
+  for (int i = 0; i < c.nmasks; ++i) { fl[nf++] = c.mk[i].m; p.mval[i] = c.mk[i].v; }
+  if (c.MK == 4) fl[nf++] = c.mk[0].vf;
+  const long long min_grid = (link && link->halo_plane[0] && env_int("DN_SLAB_WAVES", 0)) ? (long long)(1.9 * sms) : 0;
+  Plan3T pl = plan3t(g, nf, sms, occ, DN_T3_MAXT_OF(c.nu.p != nullptr), min_grid);
   if (!pl.ok) { cudaGetLastError(); return DN_OK; }
   if (pl.grid > 0x7fffffffLL) return DN_OK;
   int nput = 0;
   if (link) {
-    nput = env_i3("DN_SLAB_NPUT", 2);
+    nput = env_int("DN_SLAB_NPUT", 2);
     if (nput < 1) nput = 1;
     if (nput > 16) nput = 16;
     pl.grid += 2 * nput;
   }
-  const size_t need = 64 + 8 * (size_t)pl.grid;
-  if (!workspace || wsb < need) return fail(DN_EWORKSPACE, "workspace too small: %zu < %zu", wsb, need);
-  if ((uintptr_t)workspace % 16) return fail(DN_EWORKSPACE, "workspace must be 16-byte aligned");
+  if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
   for (int i = 0; i < nf; ++i)
     if (!make_map(&p.tm[i], fl[i], g, pl.BX, pl.BY, &p.bmul[i])) return DN_OK;   // general kernel takes it
   p.nf = nf;
@@ -272,11 +261,8 @@ int run3t(const Field& u, const Field& nu, const Field& f, const Field& fgp, con
   }
   p.k3.nkb = -k.kb;
   p.k3.nkb_pre = pr(-k.kb / p.k3.kscale);
-  p.grad = grad;
-  p.red.counter = (unsigned int*)workspace;
-  p.red.partials = (double*)((char*)workspace + 64);
-  p.red.loss_out = loss_out; p.red.loss_f32 = loss_f32;
-  p.mode = mode;
+  p.grad = o.grad;
+  p.mode = c.mode;
   if (link) {
     if (g->batch != 1) return fail(DN_EINVAL, "linked z-slab launches are for one field (batch 1)");
     if (!link->step || !link->tickets || !link->status) return fail(DN_EINVAL, "dn_slab_link: step / tickets / status missing");
@@ -309,18 +295,18 @@ int run3t(const Field& u, const Field& nu, const Field& f, const Field& fgp, con
     p.lk.status = link->status;
     p.lk.max_spins = link->max_spins > 0 ? link->max_spins : (1LL << 26);
     p.red.step = link->step;
-    p.lk.dbg = env_i3("DN_SLAB_DBG", 0);
+    p.lk.dbg = env_int("DN_SLAB_DBG", 0);
     p.red.peer_slots = link->loss_slots;
     p.red.rank = link->rank; p.red.world = (p.lk.dbg & 4) ? 0 : link->world;
     if (link->loss_slots && (link->world < 1 || link->world > 32 || link->rank < 0 || link->rank >= link->world))
       return fail(DN_EINVAL, "dn_slab_link: rank %d / world %d (world <= 32)", link->rank, link->world);
   }
-  if (env_i3("DN_DEBUG_PLAN", 0))
+  if (env_int("DN_DEBUG_PLAN", 0))
     fprintf(stderr, "[plan3t] B=%d n=(%d,%d,%d) LXT=%d LXo=%d hl=%d ntx=%d rows=%d TY=%d nty=%d ZC=%d nzc=%d S=%d BX=%d BY=%d "
             "fstride=%d threads=%d grid=%lld smem=%zu\n", g->batch, g->nx, g->ny, g->nz, pl.LXT, pl.LXo, pl.hl, pl.ntx,
             pl.rows, pl.TY, pl.nty, pl.ZC, pl.nzc, pl.S, pl.BX, pl.BY, pl.fstride, pl.threads, pl.grid, pl.smem);
   *handled = true;
-  return check_cuda(fn(p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)stream),
+  return check_cuda(fn(p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)o.stream),
                     "fem3d_tma launch");
 }
 

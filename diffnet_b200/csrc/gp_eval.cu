@@ -383,16 +383,11 @@ cudaError_t launch_gp_eval(Field in, int B, int nx, int ny, int nz, int nsd, con
   return cudaSuccess;
 }
 
-static int env_gp(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}
-
 // z-marching 3-D adjoint; false: not applicable (the y-march takes the call)
 static bool launch_adj3(int B, int nx, int ny, int nz, const GpMultiAdj& m, float* gin, cudaStream_t s, cudaError_t* err) {
   const int NG = m.tb[0].n;
   const long long nel = (long long)(nx - 1) * (ny - 1) * (nz - 1);
-  if (env_gp("DN_GP_ADJ3", 1) == 0 || NG * NG * NG * nel >= (1LL << 31)) return false;
+  if (env_int("DN_GP_ADJ3", 1) == 0 || NG * NG * NG * nel >= (1LL << 31)) return false;
   const int LXW = nx <= 32 ? 32 : 64;
   const int ntx = nx <= LXW ? 1 : 1 + (nx - LXW + LXW - 2) / (LXW - 1);
   const int nty = ny <= kAdjR ? 1 : 1 + (ny - kAdjR + kAdjR - 2) / (kAdjR - 1);
@@ -423,7 +418,7 @@ static bool launch_adj3(int B, int nx, int ny, int nz, const GpMultiAdj& m, floa
     const long long cost = ((grid + slots - 1) / slots) * (zc + 4);
     if (best < 0 || cost < best) { best = cost; ZC = zc; }
   }
-  ZC = env_gp("DN_GP_ADJ3_ZC", ZC);
+  ZC = env_int("DN_GP_ADJ3_ZC", ZC);
   if (ZC < 1) ZC = 1;
   if (ZC > nz) ZC = nz;
   const long long grid = tiles * ((nz + ZC - 1) / ZC);

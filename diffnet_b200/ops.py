@@ -49,18 +49,10 @@ def _require_cuda(t: torch.Tensor, name: str):
             f"{name} is on {t.device}: the FEM ops are CUDA (sm_100a) only, there is no CPU fallback")
 
 
-def _canon(t: torch.Tensor, geom: Geometry, name: str) -> torch.Tensor:
-    """View `t` as (Bt, *spatial) with x contiguous, fp32.  Accepted layouts: bare spatial,
-    (B, *spatial) and (B, 1, *spatial) -- what the reference's where()/conv broadcasting accepts
-    (solve_in_object_3d.py:198-199 passes a bare (D,H,W) parameter)."""
-    _require_cuda(t, name)
-    sp = geom.spatial
-    nsd = geom.nsd
-    if t.dtype != torch.float32:
-        if t.dtype in (torch.bool, torch.uint8):
-            t = t.to(torch.float32)
-        else:
-            raise L.DiffNetFEMError(f"{name} must be float32 (got {t.dtype})")
+def _nodal(t: torch.Tensor, nsd: int, name: str) -> torch.Tensor:
+    """View `t` as (Bt, *nodes) with x contiguous.  Accepted layouts: bare nodes, (B, *nodes) and (B, 1, *nodes)
+    -- what the reference's where()/conv broadcasting accepts (solve_in_object_3d.py:198-199 passes a bare (D,H,W)
+    parameter)."""
     if t.dim() == nsd + 2:
         if t.shape[1] != 1:
             raise L.DiffNetFEMError(f"{name}: expected one channel, got shape {tuple(t.shape)}")
@@ -69,10 +61,22 @@ def _canon(t: torch.Tensor, geom: Geometry, name: str) -> torch.Tensor:
         t = t.unsqueeze(0)
     elif t.dim() != nsd + 1:
         raise L.DiffNetFEMError(f"{name}: bad shape {tuple(t.shape)} for a {nsd}-D nodal field")
-    if tuple(t.shape[1:]) != sp:
-        raise L.DiffNetFEMError(f"{name}: spatial shape {tuple(t.shape[1:])} != mesh nodes {sp}")
     if t.stride(-1) != 1:
         t = t.contiguous()
+    return t
+
+
+def _canon(t: torch.Tensor, geom: Geometry, name: str) -> torch.Tensor:
+    """`_nodal` view of a CUDA fp32 field on the mesh nodes (bool / uint8 masks are converted)."""
+    _require_cuda(t, name)
+    if t.dtype != torch.float32:
+        if t.dtype in (torch.bool, torch.uint8):
+            t = t.to(torch.float32)
+        else:
+            raise L.DiffNetFEMError(f"{name} must be float32 (got {t.dtype})")
+    t = _nodal(t, geom.nsd, name)
+    if tuple(t.shape[1:]) != geom.spatial:
+        raise L.DiffNetFEMError(f"{name}: spatial shape {tuple(t.shape[1:])} != mesh nodes {geom.spatial}")
     return t
 
 
@@ -142,32 +146,10 @@ def _workspace(device: torch.device, stream_ptr: int, nbytes: int) -> torch.Tens
     return ws
 
 
-def _masks_struct(dirichlet, geom: Geometry, B: int, keep):
-    n = len(dirichlet)
-    if n > L.DN_MAX_MASKS:
-        raise L.DiffNetFEMError(f"at most {L.DN_MAX_MASKS} Dirichlet conditions per call (got {n})")
-    arr = (L.dn_mask * max(n, 1))()
-    for i, (mask, value) in enumerate(dirichlet):
-        m = _canon(mask, geom, f"dirichlet[{i}].mask")
-        keep.append(m)
-        arr[i].mask = _field(m, B, geom.nsd)
-        if torch.is_tensor(value):
-            v = _canon(value, geom, f"dirichlet[{i}].value")
-            keep.append(v)
-            arr[i].value_field = _field(v, B, geom.nsd)
-            arr[i].value = 0.0
-        else:
-            arr[i].value_field = L.dn_field(None, 0, 0, 0)
-            arr[i].value = float(value)
-    return arr, n
-
-
-def _batch_of(*ts) -> int:
-    B = 1
-    for t in ts:
-        if t is not None:
-            B = max(B, t.shape[0])
-    return B
+def _consts(c_k, c_f, scale, reduction, flags=0) -> L.dn_consts:
+    if reduction not in ("mean", "sum"):
+        raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
+    return L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1, flags)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -184,22 +166,113 @@ def _check_f_gp(geom: Geometry, f_gp) -> torch.Tensor:
     return fg
 
 
+def _per_sample(t: Optional[torch.Tensor], B: int) -> Optional[torch.Tensor]:
+    """The canonical view of a field whose gradient is wanted.  The launch writes ONE (1, ...) gradient summed over
+    the batch for a field it reads with stride_b = 0.  A field that spans the batch with stride_b = 0 (``expand``)
+    needs a gradient per sample (autograd's expand backward sums it), so its values are materialised here."""
+    if t is not None and B > 1 and t.shape[0] == B and t.stride(0) == 0:
+        return t.contiguous()
+    return t
+
+
+class _Args:
+    """The inputs of one fused-loss launch, canonicalised once (``_canon``, ``_check_f_gp``).
+
+    ``B`` is the batch of the launch: the largest batch among all inputs (every other one is 1 or ``B``).  The ctypes
+    arguments are ``c_u``, ``c_nu``, ``c_f``, ``c_fgp``, ``c_nzm``, ``c_R`` (``C.byref(dn_field)``, or None for an
+    absent input) and ``marr``, ``nm`` (the ``dn_mask`` array and its length); this object holds the views they point
+    into.  ``want`` names the fields (``"nu"``, ``"f"``) and ``want_values`` flags the tensor Dirichlet values (list
+    order) whose gradient the launch writes: those take the ``_per_sample`` view.  ``bind=True`` (a prepared call,
+    which reads the same storage on every later call) refuses an input that would have to be copied."""
+
+    def __init__(self, geom: Geometry, u=None, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None, R=None,
+                 want=(), want_values=(), bind=False):
+        def canon(t, name):
+            if t is None:
+                return None
+            c = _canon(t, geom, name)
+            if bind and c.data_ptr() != t.data_ptr():
+                raise L.DiffNetFEMError(
+                    f"prepare_energy: {name} would have to be copied (dtype {t.dtype}, strides {tuple(t.stride())}); "
+                    "a prepared call binds storage -- pass float32 tensors whose x axis is contiguous")
+            return c
+
+        n = len(dirichlet)
+        if n > L.DN_MAX_MASKS:
+            raise L.DiffNetFEMError(f"at most {L.DN_MAX_MASKS} Dirichlet conditions per call (got {n})")
+        self.u, self.nu, self.f = canon(u, "u"), canon(nu, "nu"), canon(f, "f")
+        self.nzm, self.R = canon(nu_zero_mask, "nu_zero_mask"), canon(R, "R")
+        self.fg = None
+        if f_gp is not None:
+            self.fg = _check_f_gp(geom, f_gp)
+            if not self.fg.is_contiguous():
+                if bind:
+                    raise L.DiffNetFEMError("prepare_energy: f_gp must be contiguous (a prepared call binds storage)")
+                self.fg = self.fg.contiguous()
+        masks = [canon(m, f"dirichlet[{i}].mask") for i, (m, _) in enumerate(dirichlet)]
+        values = [canon(v, f"dirichlet[{i}].value") if torch.is_tensor(v) else None
+                  for i, (_, v) in enumerate(dirichlet)]
+        B = 1
+        for t in (self.u, self.nu, self.f, self.nzm, self.R, self.fg, *masks, *values):
+            if t is not None:
+                B = max(B, t.shape[0])
+        self.B = B
+        if "nu" in want:
+            self.nu = _per_sample(self.nu, B)
+        if "f" in want:
+            self.f = _per_sample(self.f, B)
+        flags = iter(want_values)
+        self.want_v = [i for i, v in enumerate(values) if v is not None and next(flags, False)]
+        for i in self.want_v:
+            values[i] = _per_sample(values[i], B)
+        self.masks, self.values = masks, values
+        self.dev = (self.u if self.u is not None else self.fg).device
+
+        nsd = geom.nsd
+        ref = lambda t: None if t is None else C.byref(_field(t, B, nsd))
+        self.c_u, self.c_nu, self.c_f, self.c_nzm, self.c_R = map(ref, (self.u, self.nu, self.f, self.nzm, self.R))
+        self.c_fgp = None
+        if self.fg is not None:
+            fg = self.fg
+            self.c_fgp = C.byref(L.dn_field(fg.data_ptr(), fg.stride(0) if (fg.shape[0] == B and B > 1) else 0, 0, 0))
+        self.marr, self.nm = (L.dn_mask * max(n, 1))(), n
+        for i, (m, (_, v)) in enumerate(zip(masks, dirichlet)):
+            self.marr[i].mask = _field(m, B, nsd)
+            if values[i] is not None:
+                self.marr[i].value_field = _field(values[i], B, nsd)
+                self.marr[i].value = 0.0
+            else:
+                self.marr[i].value_field = L.dn_field(None, 0, 0, 0)
+                self.marr[i].value = float(v)
+
+    def grad_out(self, t: torch.Tensor, tail) -> torch.Tensor:
+        """Gradient buffer for the canonical input ``t``: per sample, or one (1, ...) sum when ``t`` is broadcast."""
+        return _new_out((self.B if (self.B > 1 and t.shape[0] == self.B) else 1,) + tuple(tail), self.dev)
+
+    def value_grads(self, spatial):
+        """Buffers for the wanted value-field gradients: (pointer array for the C call, [buffer | None per tensor
+        value, list order])."""
+        ptrs = (C.c_void_p * max(self.nm, 1))()
+        bufs = {}
+        for i in self.want_v:
+            bufs[i] = self.grad_out(self.values[i], spatial)
+            ptrs[i] = bufs[i].data_ptr()
+        return ptrs, [bufs.get(i) for i, v in enumerate(self.values) if v is not None]
+
+
 def load_vector(geom: Geometry, f_gp: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Assembled load vector b (Bf, *nodes) of a forcing given at the Gauss points (Bf = f_gp's batch, 1 when it is
     shared by the batch): b_a = sum over elements and Gauss points of w_g N_a(g) f_gp.  The forcing term of the
     reference's f_gp form (e8_2d_poisson_mms.py:154-175) is linear in u, so sum_g w_g f_g u_g = sum_a b_a u_a:
     pass ``b`` as ``f`` with ``load_vector=True`` and the fused kernels stream 4 bytes per node instead of
     4 * ngp bytes per element."""
-    fg = _check_f_gp(geom, f_gp).contiguous()
-    Bf = fg.shape[0]
-    dev = fg.device
+    a = _Args(geom, f_gp=f_gp)
     if out is None:
-        out = _new_out((Bf,) + geom.spatial, dev)
-    g = _geom_struct(geom, Bf)
-    ffg = L.dn_field(fg.data_ptr(), fg.stride(0) if Bf > 1 else 0, 0, 0)
-    with _on_device(dev):
-        rc = L.lib().dn_fem_load_vector_f32(C.byref(ffg), C.byref(g), C.c_void_p(out.data_ptr()),
-                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+        out = _new_out((a.B,) + geom.spatial, a.dev)
+    g = _geom_struct(geom, a.B)
+    with _on_device(a.dev):
+        rc = L.lib().dn_fem_load_vector_f32(a.c_fgp, C.byref(g), C.c_void_p(out.data_ptr()),
+                                            C.c_void_p(torch.cuda.current_stream(a.dev).cuda_stream))
     L.check(rc, "dn_fem_load_vector_f32")
     return out
 
@@ -246,25 +319,12 @@ def energy_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_z
         except L.DiffNetFEMError as e:
             if e.code != L.DN_ENOSTREAM:
                 raise                      # anything else is a real error; DN_ENOSTREAM: the general kernels read f_gp
-    keep = []
-    uc = _canon(u, geom, "u")
-    nuc = _canon(nu, geom, "nu") if nu is not None else None
-    fc = _canon(f, geom, "f") if f is not None else None
-    nzm = _canon(nu_zero_mask, geom, "nu_zero_mask") if nu_zero_mask is not None else None
-    fg = None
-    if f_gp is not None:
-        fg = _check_f_gp(geom, f_gp).contiguous()
-    if load_vector and (fc is None or fg is not None):
+    a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask)
+    if load_vector and (a.f is None or a.fg is not None):
         raise L.DiffNetFEMError("load_vector=True: pass the assembled vector as f (and no f_gp)")
-    masks_t = [m for m, _ in dirichlet] + [v for _, v in dirichlet if torch.is_tensor(v)]
-    B = _batch_of(uc, nuc, fc, nzm, fg, *[_canon(m, geom, "mask") for m in masks_t])
-    marr, nm = _masks_struct(dirichlet, geom, B, keep)
-    dev = uc.device
+    cs = _consts(c_k, c_f, scale, reduction, L.DN_F_LOAD_VECTOR if load_vector else 0)
+    B, dev = a.B, a.dev
     g = _geom_struct(geom, B, z_own, mean_count)
-    cs = L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1,
-                     L.DN_F_LOAD_VECTOR if load_vector else 0)
-    if reduction not in ("mean", "sum"):
-        raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
     grad = _new_out((B,) + geom.spatial, dev) if want_grad else None
     grad_nu = _new_out((B,) + geom.spatial, dev) if want_grad_nu else None
     loss = _new_out((), dev)
@@ -273,17 +333,9 @@ def energy_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_z
     stream = torch.cuda.current_stream(dev).cuda_stream
     with _on_device(dev):
         ws = _workspace_for(lib, g, geom, B, dev, stream)
-        fu, fnu, ff = _field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd)
-        ffg = L.dn_field(None, 0, 0, 0)
-        if fg is not None:
-            ffg = L.dn_field(fg.data_ptr(), fg.stride(0) if (fg.shape[0] == B and B > 1) else 0, 0, 0)
-        fnz = _field(nzm, B, geom.nsd)
         fn = lib.dn_fem_energy_2d_f32 if geom.nsd == 2 else lib.dn_fem_energy_3d_f32
-        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None,
-                C.byref(ff) if fc is not None else None, C.byref(ffg) if fg is not None else None,
-                marr, nm, C.byref(fnz) if nzm is not None else None, C.byref(g), C.byref(cs),
-                _ptr(grad), _ptr(grad_nu), C.c_void_p(ws.data_ptr()), ws.numel(), _ptr(loss64),
-                _ptr(loss), C.c_void_p(stream))
+        rc = fn(a.c_u, a.c_nu, a.c_f, a.c_fgp, a.marr, a.nm, a.c_nzm, C.byref(g), C.byref(cs), _ptr(grad),
+                _ptr(grad_nu), C.c_void_p(ws.data_ptr()), ws.numel(), _ptr(loss64), _ptr(loss), C.c_void_p(stream))
     L.check(rc, f"dn_fem_energy_{geom.nsd}d_f32")
     out = (loss, grad, grad_nu)
     return out + (loss64,) if want_double else out
@@ -303,110 +355,67 @@ class PreparedEnergy:
                  c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", z_own=None, mean_count=0.0, link=None):
         """``link``: a ``_lib.dn_slab_link`` (3-D only, see include/diffnet_fem.h) -- the launch then also
         exchanges the z-halo planes of u with the neighbouring ranks and pushes the loss partial."""
-        if reduction not in ("mean", "sum"):
-            raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
+        cs = _consts(c_k, c_f, scale, reduction)
         if link is not None and (geom.nsd != 3 or f_gp is not None):
             raise L.DiffNetFEMError("a linked (z-slab) call is 3-D with a nodal source term")
-        self._link = link
+        if f is not None and f_gp is not None:
+            raise L.DiffNetFEMError("give f or f_gp, not both")
         self.geom = geom
-        keep = []
-        uc = _canon(u, geom, "u")
-        nuc = _canon(nu, geom, "nu") if nu is not None else None
-        fc = _canon(f, geom, "f") if f is not None else None
-        nzm = _canon(nu_zero_mask, geom, "nu_zero_mask") if nu_zero_mask is not None else None
-        # the call is bound to STORAGE: a tensor that had to be copied (dtype conversion, x not
-        # contiguous) would be read from a stale private copy on every later call
-        bound = [("u", u, uc), ("nu", nu, nuc), ("f", f, fc), ("nu_zero_mask", nu_zero_mask, nzm)]
-        bound += [(f"dirichlet[{i}].mask", m, _canon(m, geom, "mask")) for i, (m, _) in enumerate(dirichlet)]
-        bound += [(f"dirichlet[{i}].value", v, _canon(v, geom, "value")) for i, (_, v) in enumerate(dirichlet)
-                  if torch.is_tensor(v)]
-        for nm, orig, canon in bound:
-            if orig is not None and canon.data_ptr() != orig.data_ptr():
-                raise L.DiffNetFEMError(
-                    f"prepare_energy: {nm} would have to be copied (dtype {orig.dtype}, strides {tuple(orig.stride())}); "
-                    "a prepared call binds storage -- pass float32 tensors whose x axis is contiguous")
-        fg = None
-        if f_gp is not None:
-            fg = _check_f_gp(geom, f_gp)
-            if not fg.is_contiguous():
-                raise L.DiffNetFEMError("prepare_energy: f_gp must be contiguous (a prepared call binds storage)")
-            if f is not None:
-                raise L.DiffNetFEMError("give f or f_gp, not both")
-        masks_t = [m for m, _ in dirichlet] + [v for _, v in dirichlet if torch.is_tensor(v)]
-        B = _batch_of(uc, nuc, fc, nzm, fg, *[_canon(m, geom, "mask") for m in masks_t])
-        self._marr, self._nm = _masks_struct(dirichlet, geom, B, keep)
-        self.device = dev = uc.device
-        self._g = _geom_struct(geom, B, z_own, mean_count)
-        self._cs = L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1, 0)
-        self.grad = _new_out((B,) + geom.spatial, dev)
-        self.loss = _new_out((), dev)
-        self._fu, self._fnu, self._ff = _field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd)
-        self._ffg = L.dn_field(None, 0, 0, 0)
-        if fg is not None:
-            self._ffg = L.dn_field(fg.data_ptr(), fg.stride(0) if (fg.shape[0] == B and B > 1) else 0, 0, 0)
-        self._fnz = _field(nzm, B, geom.nsd)
-        self._has = (nuc is not None, fc is not None, fg is not None, nzm is not None)
+        self._a = a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask, bind=True)
+        self.device, self._B = a.dev, a.B
+        self._g = g = _geom_struct(geom, a.B, z_own, mean_count)
+        self.grad = _new_out((a.B,) + geom.spatial, a.dev)
+        self.loss = _new_out((), a.dev)
+        self._loss_ptr = C.c_void_p(self.loss.data_ptr())
+        grad = C.c_void_p(self.grad.data_ptr())
+        lib = L.lib()
+        fn, name = (lib.dn_fem_energy_2d_f32, "dn_fem_energy_2d_f32") if geom.nsd == 2 else \
+            (lib.dn_fem_energy_3d_f32, "dn_fem_energy_3d_f32")
+        # each call: (C function, arguments before the workspace, name); the workspace, loss and stream follow
+        self._plain = (fn, (a.c_u, a.c_nu, a.c_f, a.c_fgp, a.marr, a.nm, a.c_nzm, C.byref(g), C.byref(cs), grad,
+                            None), name)
+        self._call = self._plain
+        if link is not None:
+            self._call = (lib.dn_fem_energy_3d_linked_f32,
+                          (a.c_u, a.c_nu, a.c_f, a.marr, a.nm, a.c_nzm, C.byref(g), C.byref(cs), C.byref(link), grad),
+                          "dn_fem_energy_3d_linked_f32")
         # f_gp: the assembled load vector is what the streaming kernels read (re-assembled when f_gp's version
         # counter moves); the first call falls back to the general kernels for good if they refuse the launch
         self._lv = None
-        if fg is not None and link is None and z_own is None and USE_LOAD_VECTOR:
-            bvec = load_vector(geom, fg)
-            self._lv = (fg, fg._version, bvec, _field(bvec, B, geom.nsd),
-                        L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1,
-                                    L.DN_F_LOAD_VECTOR))
-        self._keep = (keep, uc, nuc, fc, nzm, fg)            # the views the pointers refer to
-        lib = L.lib()
-        self._fn = lib.dn_fem_energy_2d_f32 if geom.nsd == 2 else lib.dn_fem_energy_3d_f32
-        self._B = B
+        if a.fg is not None and link is None and z_own is None and USE_LOAD_VECTOR:
+            bvec = load_vector(geom, a.fg)
+            self._lv = (a.fg, a.fg._version, bvec)
+            cs_lv = _consts(c_k, c_f, scale, reduction, L.DN_F_LOAD_VECTOR)
+            self._call = (fn, (a.c_u, a.c_nu, C.byref(_field(bvec, a.B, geom.nsd)), None, a.marr, a.nm, a.c_nzm,
+                               C.byref(g), C.byref(cs_lv), grad, None), name)
         self._ws = {}
 
     def __call__(self):
         dev = self.device
         stream = torch.cuda.current_stream(dev).cuda_stream
-        ws = self._ws.get(stream)
         with _on_device(dev):
+            ws = self._ws.get(stream)
             if ws is None:
                 ws = self._ws[stream] = _workspace_for(L.lib(), self._g, self.geom, self._B, dev, stream)
-            hn, hf, hg, hz = self._has
-            if self._link is not None:
-                rc = L.lib().dn_fem_energy_3d_linked_f32(
-                    C.byref(self._fu), C.byref(self._fnu) if hn else None, C.byref(self._ff) if hf else None,
-                    self._marr, self._nm, C.byref(self._fnz) if hz else None, C.byref(self._g), C.byref(self._cs),
-                    C.byref(self._link), C.c_void_p(self.grad.data_ptr()), C.c_void_p(ws.data_ptr()), ws.numel(),
-                    None, C.c_void_p(self.loss.data_ptr()), C.c_void_p(stream))
-                L.check(rc, "dn_fem_energy_3d_linked_f32")
-                return self.loss, self.grad
-            if self._lv is not None:
-                fg, ver, bvec, fb, cs = self._lv
-                if fg._version != ver:
-                    load_vector(self.geom, fg, out=bvec)
-                    self._lv = (fg, fg._version, bvec, fb, cs)
-                rc = self._fn(C.byref(self._fu), C.byref(self._fnu) if hn else None, C.byref(fb), None, self._marr,
-                              self._nm, C.byref(self._fnz) if hz else None, C.byref(self._g), C.byref(cs),
-                              C.c_void_p(self.grad.data_ptr()), None, C.c_void_p(ws.data_ptr()), ws.numel(), None,
-                              C.c_void_p(self.loss.data_ptr()), C.c_void_p(stream))
-                if rc != L.DN_ENOSTREAM:
-                    L.check(rc, f"dn_fem_energy_{self.geom.nsd}d_f32")
-                    return self.loss, self.grad
+            tail = (C.c_void_p(ws.data_ptr()), ws.numel(), None, self._loss_ptr, C.c_void_p(stream))
+            if self._lv is not None and self._lv[0]._version != self._lv[1]:
+                fg, _, bvec = self._lv
+                load_vector(self.geom, fg, out=bvec)
+                self._lv = (fg, fg._version, bvec)
+            fn, head, name = self._call
+            rc = fn(*head, *tail)
+            if rc == L.DN_ENOSTREAM and self._lv is not None:     # the general kernels read f_gp from now on
                 self._lv = None
-            rc = self._fn(C.byref(self._fu), C.byref(self._fnu) if hn else None, C.byref(self._ff) if hf else None,
-                          C.byref(self._ffg) if hg else None, self._marr, self._nm,
-                          C.byref(self._fnz) if hz else None, C.byref(self._g), C.byref(self._cs),
-                          C.c_void_p(self.grad.data_ptr()), None, C.c_void_p(ws.data_ptr()), ws.numel(), None,
-                          C.c_void_p(self.loss.data_ptr()), C.c_void_p(stream))
-        L.check(rc, f"dn_fem_energy_{self.geom.nsd}d_f32")
+                fn, head, name = self._call = self._plain
+                rc = fn(*head, *tail)
+        L.check(rc, name)
         return self.loss, self.grad
 
 
 def residual_raw(geom: Geometry, u, nu=None, f=None, dirichlet=(), jac=1.0, apply_masks_to_input=True):
     """R = jac*(K(nu) u' - F(f)) masked, and sum(R^2).  Returns (loss 0-dim, R (B,*spatial))."""
-    keep = []
-    uc = _canon(u, geom, "u")
-    nuc = _canon(nu, geom, "nu") if nu is not None else None
-    fc = _canon(f, geom, "f") if f is not None else None
-    B = _batch_of(uc, nuc, fc, *[_canon(m, geom, "mask") for m, _ in dirichlet])
-    marr, nm = _masks_struct(dirichlet, geom, B, keep)
-    dev = uc.device
+    a = _Args(geom, u, nu, f, dirichlet=dirichlet)
+    B, dev = a.B, a.dev
     g = _geom_struct(geom, B)
     R = _new_out((B,) + geom.spatial, dev)
     loss = _new_out((), dev)
@@ -414,57 +423,11 @@ def residual_raw(geom: Geometry, u, nu=None, f=None, dirichlet=(), jac=1.0, appl
     stream = torch.cuda.current_stream(dev).cuda_stream
     with _on_device(dev):
         ws = _workspace_for(lib, g, geom, B, dev, stream)
-        fu, fnu, ff = _field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd)
         fn = lib.dn_fem_residual_2d_f32 if geom.nsd == 2 else lib.dn_fem_residual_3d_f32
-        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None,
-                C.byref(ff) if fc is not None else None, marr, nm, 1 if apply_masks_to_input else 0,
-                C.byref(g), float(jac), _ptr(R), C.c_void_p(ws.data_ptr()), ws.numel(), None,
-                _ptr(loss), C.c_void_p(stream))
+        rc = fn(a.c_u, a.c_nu, a.c_f, a.marr, a.nm, 1 if apply_masks_to_input else 0, C.byref(g), float(jac),
+                _ptr(R), C.c_void_p(ws.data_ptr()), ws.numel(), None, _ptr(loss), C.c_void_p(stream))
     L.check(rc, f"dn_fem_residual_{geom.nsd}d_f32")
     return loss, R
-
-
-def _value_fields(dirichlet):
-    """The tensor Dirichlet values, in list order (the ones autograd can differentiate)."""
-    return tuple(v for _, v in dirichlet if torch.is_tensor(v))
-
-
-def _per_sample(t: Optional[torch.Tensor], B: int) -> Optional[torch.Tensor]:
-    """The canonical view of a field whose gradient is wanted.  The launch writes ONE (1, ...) gradient summed over
-    the batch for a field it reads with stride_b = 0.  A field that spans the batch with stride_b = 0 (``expand``)
-    needs a gradient per sample (autograd's expand backward sums it), so its values are materialised here."""
-    if t is not None and B > 1 and t.shape[0] == B and t.stride(0) == 0:
-        return t.contiguous()
-    return t
-
-
-def _grad_batch(t: torch.Tensor, B: int) -> int:
-    """Batch of the gradient the launch writes for the canonical field ``t`` (after ``_per_sample``)."""
-    return B if (B > 1 and t.shape[0] == B) else 1
-
-
-def _grad_values_dirichlet(dirichlet, want_values, geom: Geometry, B: int):
-    """``dirichlet`` with every differentiated value field in the form ``_per_sample`` gives."""
-    out, it = [], iter(want_values)
-    for i, (m, v) in enumerate(dirichlet):
-        if torch.is_tensor(v) and next(it):
-            v = _per_sample(_canon(v, geom, f"dirichlet[{i}].value"), B)
-        out.append((m, v))
-    return out
-
-
-def _grad_values_arg(dirichlet, want_values, geom: Geometry, B: int, dev):
-    """Output buffers for the wanted value-field gradients: (host pointer array, [(list index, buffer)])."""
-    ptrs = (C.c_void_p * max(len(dirichlet), 1))()
-    outs = []
-    it = iter(want_values)
-    for i, (_, v) in enumerate(dirichlet):
-        if torch.is_tensor(v) and next(it):
-            vc = _canon(v, geom, f"dirichlet[{i}].value")
-            buf = _new_out((_grad_batch(vc, B),) + geom.spatial, dev)
-            ptrs[i] = buf.data_ptr()
-            outs.append((i, buf))
-    return ptrs, outs
 
 
 def energy_input_grads_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None,
@@ -473,43 +436,19 @@ def energy_input_grads_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirich
     """dL/df, dL/df_gp and dL/d(value field) of the energy loss in ONE launch (dn_fem_energy_input_grads_*).
     ``want_values``: one flag per tensor Dirichlet value, in list order.  Returns (grad_f | None,
     grad_f_gp | None, [grad per tensor value | None]); a gradient of a field broadcast over the batch is (1, ...)."""
-    if reduction not in ("mean", "sum"):
-        raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
-    keep = []
-    uc = _canon(u, geom, "u")
-    nuc = _canon(nu, geom, "nu") if nu is not None else None
-    fc = _canon(f, geom, "f") if f is not None else None
-    nzm = _canon(nu_zero_mask, geom, "nu_zero_mask") if nu_zero_mask is not None else None
-    fg = _check_f_gp(geom, f_gp).contiguous() if f_gp is not None else None
-    masks_t = [m for m, _ in dirichlet] + list(_value_fields(dirichlet))
-    B = _batch_of(uc, nuc, fc, nzm, fg, *[_canon(m, geom, "mask") for m in masks_t])
-    if want_f:
-        fc = _per_sample(fc, B)
-    dirichlet = _grad_values_dirichlet(dirichlet, want_values, geom, B)
-    marr, nm = _masks_struct(dirichlet, geom, B, keep)
-    dev = uc.device
-    g = _geom_struct(geom, B, None, mean_count)
-    cs = L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1, 0)
-    gf = _new_out((_grad_batch(fc, B),) + geom.spatial, dev) if want_f else None
-    ngp = geom.ngp_1d ** geom.nsd
-    gfg = _new_out((_grad_batch(fg, B), ngp) + geom.elems, dev) if want_f_gp else None
-    ptrs, gvs = _grad_values_arg(dirichlet, want_values, geom, B, dev)
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    with _on_device(dev):
-        fu, fnu, ff = _field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd)
-        ffg = L.dn_field(None, 0, 0, 0)
-        if fg is not None:
-            ffg = L.dn_field(fg.data_ptr(), fg.stride(0) if (fg.shape[0] == B and B > 1) else 0, 0, 0)
-        fnz = _field(nzm, B, geom.nsd)
+    cs = _consts(c_k, c_f, scale, reduction)
+    a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask, want=("f",) if want_f else (), want_values=want_values)
+    g = _geom_struct(geom, a.B, None, mean_count)
+    gf = a.grad_out(a.f, geom.spatial) if want_f else None
+    gfg = a.grad_out(a.fg, (geom.ngp_1d ** geom.nsd,) + geom.elems) if want_f_gp else None
+    ptrs, gv = a.value_grads(geom.spatial)
+    with _on_device(a.dev):
         lib = L.lib()
         fn = lib.dn_fem_energy_input_grads_2d_f32 if geom.nsd == 2 else lib.dn_fem_energy_input_grads_3d_f32
-        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None, C.byref(ff) if fc is not None else None,
-                C.byref(ffg) if fg is not None else None, marr, nm, C.byref(fnz) if nzm is not None else None,
-                C.byref(g), C.byref(cs), _ptr(gf), _ptr(gfg), ptrs, C.c_void_p(stream))
+        rc = fn(a.c_u, a.c_nu, a.c_f, a.c_fgp, a.marr, a.nm, a.c_nzm, C.byref(g), C.byref(cs), _ptr(gf), _ptr(gfg),
+                ptrs, C.c_void_p(torch.cuda.current_stream(a.dev).cuda_stream))
     L.check(rc, f"dn_fem_energy_input_grads_{geom.nsd}d_f32")
-    by_index = dict(gvs)
-    vals = [by_index.get(i) for i, (_, v) in enumerate(dirichlet) if torch.is_tensor(v)]
-    return gf, gfg, vals
+    return gf, gfg, gv
 
 
 def residual_input_grads_raw(geom: Geometry, u, R, nu=None, f=None, dirichlet=(), jac=1.0, want_nu=False,
@@ -517,34 +456,19 @@ def residual_input_grads_raw(geom: Geometry, u, R, nu=None, f=None, dirichlet=()
     """dL/dnu, dL/df and dL/d(value field) of the residual loss sum(R^2) in ONE launch
     (dn_fem_residual_input_grads_*); ``R`` is the residual the forward returned.  Returns (grad_nu | None,
     grad_f | None, [grad per tensor value | None])."""
-    keep = []
-    uc = _canon(u, geom, "u")
-    nuc = _canon(nu, geom, "nu") if nu is not None else None
-    fc = _canon(f, geom, "f") if f is not None else None
-    B = R.shape[0]
-    if want_nu:
-        nuc = _per_sample(nuc, B)
-    if want_f:
-        fc = _per_sample(fc, B)
-    dirichlet = _grad_values_dirichlet(dirichlet, want_values, geom, B)
-    marr, nm = _masks_struct(dirichlet, geom, B, keep)
-    dev = uc.device
-    g = _geom_struct(geom, B)
-    gnu = _new_out((_grad_batch(nuc, B),) + geom.spatial, dev) if want_nu else None
-    gf = _new_out((_grad_batch(fc, B),) + geom.spatial, dev) if want_f else None
-    ptrs, gvs = _grad_values_arg(dirichlet, want_values, geom, B, dev)
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    with _on_device(dev):
-        fu, fnu, ff, fr = (_field(uc, B, geom.nsd), _field(nuc, B, geom.nsd), _field(fc, B, geom.nsd),
-                           _field(R, B, geom.nsd))
+    want = ("nu",) * want_nu + ("f",) * want_f
+    a = _Args(geom, u, nu, f, dirichlet=dirichlet, R=R, want=want, want_values=want_values)
+    g = _geom_struct(geom, a.B)
+    gnu = a.grad_out(a.nu, geom.spatial) if want_nu else None
+    gf = a.grad_out(a.f, geom.spatial) if want_f else None
+    ptrs, gv = a.value_grads(geom.spatial)
+    with _on_device(a.dev):
         lib = L.lib()
         fn = lib.dn_fem_residual_input_grads_2d_f32 if geom.nsd == 2 else lib.dn_fem_residual_input_grads_3d_f32
-        rc = fn(C.byref(fu), C.byref(fnu) if nuc is not None else None, C.byref(ff) if fc is not None else None,
-                C.byref(fr), marr, nm, C.byref(g), float(jac), _ptr(gnu), _ptr(gf), ptrs, C.c_void_p(stream))
+        rc = fn(a.c_u, a.c_nu, a.c_f, a.c_R, a.marr, a.nm, C.byref(g), float(jac), _ptr(gnu), _ptr(gf), ptrs,
+                C.c_void_p(torch.cuda.current_stream(a.dev).cuda_stream))
     L.check(rc, f"dn_fem_residual_input_grads_{geom.nsd}d_f32")
-    by_index = dict(gvs)
-    vals = [by_index.get(i) for i, (_, v) in enumerate(dirichlet) if torch.is_tensor(v)]
-    return gnu, gf, vals
+    return gnu, gf, gv
 
 
 def scale_inplace_(x: torch.Tensor, factor: torch.Tensor) -> torch.Tensor:
@@ -803,17 +727,7 @@ class GaussPointEvalGeneralFunction(torch.autograd.Function):
         _require_cuda(t, "tensor")
         if t.dtype != torch.float32:
             raise L.DiffNetFEMError(f"tensor must be float32 (got {t.dtype})")
-        tc = t.detach()
-        if tc.dim() == nsd + 2:
-            if tc.shape[1] != 1:
-                raise L.DiffNetFEMError(f"expected one channel, got shape {tuple(tc.shape)}")
-            tc = tc[:, 0]
-        elif tc.dim() == nsd:
-            tc = tc.unsqueeze(0)
-        elif tc.dim() != nsd + 1:
-            raise L.DiffNetFEMError(f"bad shape {tuple(tc.shape)} for a {nsd}-D nodal field")
-        if tc.stride(-1) != 1:
-            tc = tc.contiguous()
+        tc = _nodal(t.detach(), nsd, "tensor")
         B = tc.shape[0]
         sp = tuple(tc.shape[1:])                                   # ([nz, ny,] nx)
         if any((n - 1) % (nb - 1) for n in sp):
@@ -860,8 +774,8 @@ def fem_energy(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet: Sequenc
     """Fused Poisson energy loss (SURVEY.md App. A.4), differentiable w.r.t. u, nu, f, f_gp and the tensor
     Dirichlet values (the last three not with ``z_own``)."""
     dirichlet = tuple(dirichlet)
-    return FEMEnergyFunction.apply(u, nu, geom, f, f_gp, dirichlet, nu_zero_mask, c_k, c_f,
-                                   scale, reduction, z_own, mean_count, *_value_fields(dirichlet))
+    return FEMEnergyFunction.apply(u, nu, geom, f, f_gp, dirichlet, nu_zero_mask, c_k, c_f, scale, reduction,
+                                   z_own, mean_count, *(v for _, v in dirichlet if torch.is_tensor(v)))
 
 
 def fem_energy_and_grad(geom: Geometry, u, **kw):
@@ -873,7 +787,7 @@ def fem_energy_and_grad(geom: Geometry, u, **kw):
 def fem_residual(geom: Geometry, u, nu=None, f=None, dirichlet: Sequence = (), jac=1.0) -> torch.Tensor:
     """sum(R^2) of the assembled residual, differentiable w.r.t. u, nu, f and the tensor Dirichlet values."""
     dirichlet = tuple(dirichlet)
-    return FEMResidualFunction.apply(u, geom, nu, f, dirichlet, jac, *_value_fields(dirichlet))
+    return FEMResidualFunction.apply(u, geom, nu, f, dirichlet, jac, *(v for _, v in dirichlet if torch.is_tensor(v)))
 
 
 def gp_eval(geom: Geometry, t: torch.Tensor, which: str = "N") -> torch.Tensor:

@@ -227,14 +227,18 @@ def test_residual_input_grads_parity(B, shape, ngp):
     fem = _fem(shape, ngp)
     x = _fields(B, shape, seed=sum(shape) * 7 + ngp)
     two = [(x["left"], 1.0), (x["right"], 0.0)]
+    u = x["u"]
     cases = [
-        ("nu_f", dict(nu=x["nu"], f=x["f"], dirichlet=two), ["nu", "f"], dict(jac=0.37)),
-        ("valuefield", dict(nu=x["nu"], f=x["f"], dirichlet=[(x["blob"], x["ubc"])]), ["nu", "v0"], {}),
-        ("nu_bcast_f_bare", dict(nu=x["nu"][:1], f=x["f"][0, 0].clone(), dirichlet=two), ["nu", "f"],
+        ("nu_f", u, dict(nu=x["nu"], f=x["f"], dirichlet=two), ["nu", "f"], dict(jac=0.37)),
+        ("valuefield", u, dict(nu=x["nu"], f=x["f"], dirichlet=[(x["blob"], x["ubc"])]), ["nu", "v0"], {}),
+        ("nu_bcast_f_bare", u, dict(nu=x["nu"][:1], f=x["f"][0, 0].clone(), dirichlet=two), ["nu", "f"],
          dict(jac=1.9)),
+        # only the value field carries the batch: the launch batch is taken from it, as in the energy form
+        ("valuefield_batched_only", u[:1], dict(nu=x["nu"][:1], f=x["f"][:1], dirichlet=[(x["blob"][:1], x["ubc"])]),
+         ["nu", "v0"], dict(jac=0.8)),
     ]
-    for name, kw, names, fixed in cases:
-        _check(fem, fem.residual_loss, OL.residual_loss, x["u"], kw, names,
+    for name, u0, kw, names, fixed in cases:
+        _check(fem, fem.residual_loss, OL.residual_loss, u0, kw, names,
                f"residual {name} {B}x{shape} ngp={ngp}", **fixed)
 
 
