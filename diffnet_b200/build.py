@@ -2,9 +2,11 @@
 
     python -m diffnet_b200.build [--force] [-j N]
 
-One object per translation unit, compiled in parallel; the kernel families are split into one
-TU per (lane width, Dirichlet set) under csrc/gen/ (written by this script, committed).
-The library has NO torch dependency: its boundary is the C ABI of include/diffnet_fem.h.
+One object per translation unit, compiled in parallel.  The variants of each fused-kernel family
+(csrc/fem*_combos.h) are split into slices: csrc/fem*_inst.cu is compiled once per (lane width V,
+Dirichlet variant MK) for the general families and once per MK for the streaming ones.  This file is
+the only list of the slices: one left out leaves the library with an undefined symbol, and it fails
+to load.  The library has NO torch dependency: its boundary is the C ABI of include/diffnet_fem.h.
 """
 from __future__ import annotations
 
@@ -19,7 +21,6 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
-GEN = os.path.join(CSRC, "gen")
 OBJ = os.environ.get("DN_BUILD_DIR", os.path.join(PKG, "build"))
 LIB = os.environ.get("DN_BUILD_LIB", os.path.join(PKG, "lib", "libdiffnet_fem.so"))
 
@@ -30,8 +31,9 @@ NVCC_FLAGS = [
     "-DDN_BUILD=1",
 ] + os.environ.get("DN_NVCC_EXTRA", "").split()
 
-VS = (4, 1)
-MKS = (0, 1, 2, 3, 4)
+VS = (4, 1)                     # lane widths of the general families (16-byte / scalar row loads)
+MKS = (0, 1, 2, 3, 4)           # Dirichlet variants of every family (dn_launch.h: mk_nmasks)
+MKS_OP = (5, 6, 7)              # streaming families only: operator apply (mask_input = 0)
 
 
 def nvcc_path() -> str:
@@ -41,48 +43,23 @@ def nvcc_path() -> str:
     raise RuntimeError("nvcc not found; libdiffnet_fem needs the CUDA 12.9 toolkit to build")
 
 
-def write_gen() -> list[str]:
-    os.makedirs(GEN, exist_ok=True)
-    out = []
+def units() -> list[tuple[str, str, list[str]]]:
+    """(source, object name, defines) of every translation unit."""
+    out = [(os.path.join(CSRC, n), n[:-3], []) for n in
+           ("dn_api.cu", "fem2d_dispatch.cu", "fem2d_tma_dispatch.cu", "fem3d_dispatch.cu", "fem3d_tma_dispatch.cu",
+            "gp_eval.cu", "input_grads.cu", "peer.cu", "producers.cu")]
     for dim in (2, 3):
-        for v in VS:
-            for mk in MKS:
-                path = os.path.join(GEN, f"fem{dim}d_v{v}_mk{mk}.cu")
-                text = (f"// generated by diffnet_b200/build.py -- one (V, MK) slice of the "
-                        f"{dim}-D kernel family\n#define DN_V {v}\n#define DN_MK {mk}\n"
-                        f'#include "../fem{dim}d_inst.inl"\n')
-                if not os.path.exists(path) or open(path).read() != text:
-                    with open(path, "w") as fh:
-                        fh.write(text)
-                out.append(path)
-    for mk in MKS + (5, 6, 7):                       # streaming 2-D family: one TU per Dirichlet set
-        path = os.path.join(GEN, f"fem2dt_mk{mk}.cu")
-        text = (f"// generated by diffnet_b200/build.py -- one MK slice of the streaming 2-D kernel "
-                f"family\n#define DN_MK {mk}\n#include \"../fem2d_tma_inst.inl\"\n")
-        if not os.path.exists(path) or open(path).read() != text:
-            with open(path, "w") as fh:
-                fh.write(text)
-        out.append(path)
-    for mk in MKS + (5, 6, 7):                       # streaming 3-D family
-        path = os.path.join(GEN, f"fem3dt_mk{mk}.cu")
-        text = (f"// generated by diffnet_b200/build.py -- one MK slice of the streaming 3-D kernel "
-                f"family\n#define DN_MK {mk}\n#include \"../fem3d_tma_inst.inl\"\n")
-        if not os.path.exists(path) or open(path).read() != text:
-            with open(path, "w") as fh:
-                fh.write(text)
-        out.append(path)
+        src = os.path.join(CSRC, f"fem{dim}d_inst.cu")
+        out += [(src, f"fem{dim}d_v{v}_mk{mk}", [f"-DDN_V={v}", f"-DDN_MK={mk}"]) for v in VS for mk in MKS]
+    for dim in (2, 3):
+        src = os.path.join(CSRC, f"fem{dim}d_tma_inst.cu")
+        out += [(src, f"fem{dim}dt_mk{mk}", [f"-DDN_MK={mk}"]) for mk in MKS + MKS_OP]
     return out
-
-
-def sources() -> list[str]:
-    fixed = [os.path.join(CSRC, n) for n in
-             ("dn_api.cu", "fem2d_dispatch.cu", "fem2d_tma_dispatch.cu", "fem3d_dispatch.cu", "fem3d_tma_dispatch.cu", "gp_eval.cu", "input_grads.cu", "peer.cu", "producers.cu")]
-    return fixed + write_gen()
 
 
 def _deps_digest() -> str:
     h = hashlib.sha1()
-    hdrs = [os.path.join(CSRC, n) for n in sorted(os.listdir(CSRC)) if n.endswith((".cuh", ".h", ".inl"))]
+    hdrs = [os.path.join(CSRC, n) for n in sorted(os.listdir(CSRC)) if n.endswith((".cuh", ".h"))]
     hdrs.append(os.path.join(ROOT, "include", "diffnet_fem.h"))
     for p in hdrs:
         h.update(open(p, "rb").read())
@@ -91,16 +68,16 @@ def _deps_digest() -> str:
 
 
 def _compile_one(args):
-    nvcc, src, obj, stamp, digest = args
-    key = hashlib.sha1(open(src, "rb").read() + digest.encode()).hexdigest()
+    nvcc, src, defines, obj, stamp, digest = args
+    key = hashlib.sha1(open(src, "rb").read() + " ".join(defines).encode() + digest.encode()).hexdigest()
     if os.path.exists(obj) and os.path.exists(stamp) and open(stamp).read() == key:
-        return src, 0, "cached"
-    cmd = [nvcc, *NVCC_FLAGS, "-I", os.path.join(ROOT, "include"), "-c", src, "-o", obj]
+        return obj, 0, "cached"
+    cmd = [nvcc, *NVCC_FLAGS, *defines, "-I", os.path.join(ROOT, "include"), "-c", src, "-o", obj]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode == 0:
         with open(stamp, "w") as fh:
             fh.write(key)
-    return src, r.returncode, (r.stdout + r.stderr).strip()
+    return obj, r.returncode, (r.stdout + r.stderr).strip()
 
 
 def build(force: bool = False, jobs: int | None = None, verbose: bool = True) -> str:
@@ -108,25 +85,23 @@ def build(force: bool = False, jobs: int | None = None, verbose: bool = True) ->
     os.makedirs(OBJ, exist_ok=True)
     os.makedirs(os.path.dirname(LIB), exist_ok=True)
     digest = _deps_digest()
-    srcs = sources()
     work = []
-    for s in srcs:
-        base = os.path.splitext(os.path.basename(s))[0]
+    for src, base, defines in units():
         obj, stamp = os.path.join(OBJ, base + ".o"), os.path.join(OBJ, base + ".stamp")
         if force and os.path.exists(stamp):
             os.remove(stamp)
-        work.append((nvcc, s, obj, stamp, digest))
+        work.append((nvcc, src, defines, obj, stamp, digest))
     jobs = jobs or min(len(work), max(1, os.cpu_count() or 1))
     rebuilt = 0
     with cf.ThreadPoolExecutor(max_workers=jobs) as ex:
-        for src, rc, msg in ex.map(_compile_one, work):
+        for obj, rc, msg in ex.map(_compile_one, work):
             if rc != 0:
-                raise RuntimeError(f"nvcc failed on {src}:\n{msg}")
+                raise RuntimeError(f"nvcc failed on {os.path.basename(obj)}:\n{msg}")
             if msg != "cached":
                 rebuilt += 1
                 if verbose:
-                    print(f"[diffnet_b200.build] compiled {os.path.relpath(src, ROOT)}", flush=True)
-    objs = [w[2] for w in work]
+                    print(f"[diffnet_b200.build] compiled {os.path.basename(obj)}", flush=True)
+    objs = [w[3] for w in work]
     if rebuilt or not os.path.exists(LIB):
         # cudart is linked statically (nvcc default): the library then does not care which
         # libcudart the host process (e.g. torch 2.11+cu128) has loaded; streams are shared

@@ -8,7 +8,6 @@
 
 #include "dn_common.cuh"
 #include "dn_launch.h"
-#include "fem2d_tma.cuh"     // DN_T2_MAXF
 #include "gp_eval.cuh"
 #include "input_grads.cuh"
 

@@ -9,6 +9,8 @@ namespace dn {
 
 constexpr int kWarpsPerCta2D = 4;
 
+#define DN_T2_MAXF 8        // field slots of a streaming launch: u, nu, f, numask, masks[3] | mask+value_field
+
 struct Field {
   const float* p;
   long long sb, sz, sy;

@@ -345,18 +345,8 @@ __global__ void __launch_bounds__(128) k_fem2d(const P2D p) {
   finish_loss(p.red, cta, s_red);
 }
 
-// ---- dispatch -----------------------------------------------------------------------------
-// MK encodes the Dirichlet set: 0,1,2,3 = that many scalar-valued masks; 4 = one mask with a
-// nodal value field.
-typedef cudaError_t (*launch2d_fn)(const P2D&, dim3, dim3, cudaStream_t);
-launch2d_fn get_launch2d(int V, int MK, int NU, int FM, int NUMASK, int GN);
-
+// The kernel of one fem2d_combos.h variant (MK as in dn_launch.h), instantiated by fem2d_inst.cu.
 template <int V, int MK, bool HAS_NU, int FM, bool NUMASK, bool GN>
-cudaError_t launch2d(const P2D& p, dim3 grid, dim3 block, cudaStream_t s) {
-  constexpr int NM = (MK == 4) ? 1 : MK;
-  constexpr bool VF = (MK == 4);
-  k_fem2d<V, NM, VF, HAS_NU, FM, NUMASK, GN><<<grid, block, 0, s>>>(p);
-  return cudaGetLastError();
-}
+const void* kernel2d();
 
 }  // namespace dn

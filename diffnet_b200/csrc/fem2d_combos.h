@@ -3,6 +3,7 @@
 //   MK  Dirichlet set (0..3 scalar-valued masks, 4 = one mask with a nodal value field)
 //   FM  source term (0 none, 1 nodal f, 2 f at Gauss points)
 //   NUMASK  nu zeroed under a mask (Neumann IBN);  GN  also emit d(loss)/d(nu)
+// DN2D_COMBOS(X, V, MK) is one slice (one object file, see build.py), DN2D_ALL(X) all of them.
 #pragma once
 #define DN2D_COMBOS(X, V, MK)                                                          \
   X(V, MK, false, 0, false, false) X(V, MK, false, 1, false, false)                    \

@@ -1,21 +1,18 @@
-// Launch planning and runtime -> compile-time dispatch of the 2-D kernel family (instantiated in gen/fem2d_*.cu).
+// Launch planning and runtime -> compile-time dispatch of the 2-D kernel family (instantiated by fem2d_inst.cu).
 #include "dn_launch.h"
 #include "fem2d.cuh"
 #include "fem2d_combos.h"
-#include "fem2d_tma.cuh"
 namespace dn {
-#define DN_EXT(V, MK, NU, FM, NMK, GN) \
-  extern template cudaError_t launch2d<V, MK, NU, FM, NMK, GN>(const P2D&, dim3, dim3, cudaStream_t);
-DN2D_ALL(DN_EXT)
-#undef DN_EXT
 
-launch2d_fn get_launch2d(int V, int MK, int NU, int FM, int NUMASK, int GN) {
-#define DN_CASE(V_, MK_, NU_, FM_, NMK_, GN_)                                          \
-  if (V == V_ && MK == MK_ && NU == (int)NU_ && FM == FM_ && NUMASK == (int)NMK_ &&   \
-      GN == (int)GN_)                                                                  \
-    return &launch2d<V_, MK_, NU_, FM_, NMK_, GN_>;
-  DN2D_ALL(DN_CASE)
-#undef DN_CASE
+// The kernel of a variant of fem2d_combos.h, or null when it is not instantiated.
+static Kernel* find2d(int V, int MK, int NU, int FM, int NUMASK, int GN) {
+  static struct { int V, MK, NU, FM, NUMASK, GN; Kernel k; } tab[] = {
+#define DN_ROW(V_, MK_, NU_, FM_, NMK_, GN_) {V_, MK_, NU_, FM_, NMK_, GN_, {kernel2d<V_, MK_, NU_, FM_, NMK_, GN_>()}},
+      DN2D_ALL(DN_ROW)
+#undef DN_ROW
+  };
+  for (auto& r : tab)
+    if (r.V == V && r.MK == MK && r.NU == NU && r.FM == FM && r.NUMASK == NUMASK && r.GN == GN) return &r.k;
   return nullptr;
 }
 
@@ -76,11 +73,12 @@ int run2d(const Common& c, const dn_geom* g, const Out& o) {
   p.grad = o.grad; p.grad_nu = o.grad_nu;
   p.mode = c.mode; p.mask_input = c.mask_input;
   const int FM = c.f.p ? 1 : (c.fgp.p ? 2 : 0);
-  launch2d_fn fn = get_launch2d(pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0, o.grad_nu ? 1 : 0);
-  if (!fn)
+  Kernel* k = find2d(pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0, o.grad_nu ? 1 : 0);
+  if (!k)
     return fail(DN_EINVAL, "unsupported option combination (V=%d MK=%d nu=%d fmode=%d numask=%d grad_nu=%d)",
                 pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0, o.grad_nu ? 1 : 0);
-  return check_cuda(fn(p, dim3(pl.grid), dim3(32 * pl.wpc), (cudaStream_t)o.stream), "fem2d launch");
+  return check_cuda(launch(*k, &p, dim3(pl.grid), dim3(32 * pl.wpc), 0, (cudaStream_t)o.stream, false),
+                    "fem2d launch");
 }
 
 }  // namespace dn

@@ -21,16 +21,11 @@
 //   * Chunk seams: one halo row above and below is re-read (from L2) and the element row above
 //     the chunk recomputed; (R+2)/R reads, (R+1)/R arithmetic.
 #pragma once
-#include <cstdlib>
-#include <cstring>
 #include <type_traits>
 
 #include "dn_common.cuh"
 
 namespace dn {
-
-#define DN_T2_MAXF 8        // u, nu, f, numask, masks[3] | mask+value_field
-#define DN_T2_MAXT 512      // threads per CTA -> nx <= 2048
 
 // Packed constants of one launch (see prepare(): kx, ky carry S c_k W (2/h)^2 / 64, kf = S c_f W / 16)
 struct K2 {
@@ -589,70 +584,8 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
   finish_loss_w0(p.red, cta, s_ticket);
 }
 
-// ---- dispatch (fem2d_tma_dispatch.cu) --------------------------------------------------------
-// MK encodes the Dirichlet set: 0..3 scalar-valued masks; 4 = one mask with a nodal value field.
-typedef cudaError_t (*launch2t_fn)(const P2T&, dim3, dim3, size_t, cudaStream_t);
-typedef int (*occ2t_fn)(int, size_t);
-launch2t_fn get_launch2t(int MK, int NU, int F, int NUMASK);
-occ2t_fn get_occ2t(int MK, int NU, int F, int NUMASK);
-
-// DN_PDL=0 disables programmatic dependent launch (default on)
-inline bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DN_PDL"); v = (e && *e == '0') ? 0 : 1; }
-  return v == 1;
-}
-
-constexpr int kMaxDynSmem = 226 * 1024;   // 227 KB per CTA minus the kernels' static shared memory
-
-// One register budget (<= 128 registers, CTAs of up to 512 threads).  A tighter variant
-// (<= 96 registers, 10 instead of 8 resident 64-thread CTAs per SM) measured 10% SLOWER on
-// 256^2 x 64: more CTAs per wave means shorter row chunks and more seam work (profiles/).
+// The kernel of one fem2d_tma_combos.h variant (MK as in dn_launch.h), instantiated by fem2d_tma_inst.cu.
 template <int MK, bool HAS_NU, int FK, bool NUMASK>
-struct Kern2T {
-  // MK 0..3: that many scalar-valued masks; 4: one mask with a value field; 5..7: 1..3 masks whose
-  // values are NOT substituted into u (mask_input = 0: the operator v -> mask(K v) of the resmin backward)
-  static constexpr int NM = (MK == 4) ? 1 : (MK >= 5 ? MK - 4 : MK);
-  static auto get() { return k_fem2d_tma<NM, (MK == 4), HAS_NU, FK, NUMASK, (MK < 5), DN_T2_MAXT, 1>; }
-};
-
-template <int MK, bool HAS_NU, int FK, bool NUMASK>
-cudaError_t prep2t() {
-  // opt in to the full dynamic shared memory once per device
-  static bool done[64] = {};
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev >= 0 && dev < 64 && done[dev]) return cudaSuccess;
-  e = cudaFuncSetAttribute(Kern2T<MK, HAS_NU, FK, NUMASK>::get(),
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxDynSmem);
-  if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
-  return e;
-}
-
-template <int MK, bool HAS_NU, int FK, bool NUMASK>
-cudaError_t launch2t(const P2T& p, dim3 grid, dim3 block, size_t smem, cudaStream_t s) {
-  cudaError_t e = prep2t<MK, HAS_NU, FK, NUMASK>();
-  if (e != cudaSuccess) return e;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  if (pdl_enabled()) { cfg.attrs = at; cfg.numAttrs = 1; }
-  return cudaLaunchKernelEx(&cfg, Kern2T<MK, HAS_NU, FK, NUMASK>::get(), p);
-}
-
-// resident CTAs per SM for a block of `threads` threads and `smem` bytes of dynamic shared memory
-template <int MK, bool HAS_NU, int FK, bool NUMASK>
-int occ2t(int threads, size_t smem) {
-  if (prep2t<MK, HAS_NU, FK, NUMASK>() != cudaSuccess) return 0;
-  int n = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, Kern2T<MK, HAS_NU, FK, NUMASK>::get(),
-                                                    threads, smem) != cudaSuccess)
-    return 0;
-  return n;
-}
+const void* kernel2t();
 
 }  // namespace dn

@@ -1,29 +1,19 @@
-// Launch planning and runtime -> compile-time dispatch of the streaming 2-D kernel family (gen/fem2dt_mk*.cu).
+// Launch planning and runtime -> compile-time dispatch of the streaming 2-D kernel family (instantiated by
+// fem2d_tma_inst.cu).
 #include "dn_launch.h"
 #include "fem2d_tma.cuh"
 #include "fem2d_tma_combos.h"
 namespace dn {
-#define DN_EXT(MK, NU, F, NMK)                                                                        \
-  extern template cudaError_t launch2t<MK, NU, F, NMK>(const P2T&, dim3, dim3, size_t, cudaStream_t); \
-  extern template int occ2t<MK, NU, F, NMK>(int, size_t);
-DN2T_ALL(DN_EXT)
-#undef DN_EXT
 
-launch2t_fn get_launch2t(int MK, int NU, int F, int NUMASK) {
-#define DN_CASE(MK_, NU_, F_, NMK_)                                                          \
-  if (MK == MK_ && NU == (int)NU_ && F == (int)F_ && NUMASK == (int)NMK_)     \
-    return &launch2t<MK_, NU_, F_, NMK_>;
-  DN2T_ALL(DN_CASE)
-#undef DN_CASE
-  return nullptr;
-}
-
-occ2t_fn get_occ2t(int MK, int NU, int F, int NUMASK) {
-#define DN_CASE(MK_, NU_, F_, NMK_)                                                          \
-  if (MK == MK_ && NU == (int)NU_ && F == (int)F_ && NUMASK == (int)NMK_)     \
-    return &occ2t<MK_, NU_, F_, NMK_>;
-  DN2T_ALL(DN_CASE)
-#undef DN_CASE
+// The kernel of a variant of fem2d_tma_combos.h, or null when it is not instantiated.
+static Kernel* find2t(int MK, int NU, int F, int NUMASK) {
+  static struct { int MK, NU, F, NUMASK; Kernel k; } tab[] = {
+#define DN_ROW(MK_, NU_, F_, NMK_) {MK_, NU_, F_, NMK_, {kernel2t<MK_, NU_, F_, NMK_>()}},
+      DN2T_ALL(DN_ROW)
+#undef DN_ROW
+  };
+  for (auto& r : tab)
+    if (r.MK == MK && r.NU == NU && r.F == F && r.NUMASK == NUMASK) return &r.k;
   return nullptr;
 }
 
@@ -33,9 +23,9 @@ static size_t smem_2t(int S, int nf, int nx, int threads) {
   return (size_t)S * nf * 2 * nx * 4 + 16 + (size_t)S * 8 + 4 * (size_t)(threads / 32) * 4;
 }
 
-// Eligibility + launch shape.  `occ` (resident CTAs per SM) may be null: then only the upper
+// Eligibility + launch shape.  `k` (whose occupancy bounds the grid) may be null: then only the upper
 // bound of the grid matters (workspace sizing).
-static Plan2T plan2t(const dn_geom* g, int nf, int sms, occ2t_fn occ) {
+static Plan2T plan2t(const dn_geom* g, int nf, int sms, Kernel* k) {
   Plan2T pl;
   memset(&pl, 0, sizeof(pl));
   if (g->nx % 4 != 0 || g->nx < 8) return pl;
@@ -50,7 +40,7 @@ static Plan2T plan2t(const dn_geom* g, int nf, int sms, occ2t_fn occ) {
   pl.S = S;
   pl.smem = smem_2t(S, nf, g->nx, pl.threads);
   if (pl.smem > (size_t)kMaxDynSmem) return pl;
-  int cps = occ ? occ(pl.threads, pl.smem) : 8;
+  int cps = k ? occupancy(*k, pl.threads, pl.smem) : 8;
   if (cps < 1) return pl;
   const int cap = env_int("DN_T2_CPS", 0);
   if (cap > 0 && cps > cap) cps = cap;
@@ -119,22 +109,14 @@ int run2t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
   if (!c.vec4 || c.fgp.p || ((uintptr_t)o.grad % 16 != 0)) return DN_OK;
   const int NU = c.nu.p ? 1 : 0, F = c.f.p ? (c.k.lv ? 2 : 1) : 0, NMK = c.numask.p ? 1 : 0;
   if (g->nx % 4 != 0 || g->nx / 4 > DN_T2_MAXT) return DN_OK;
-  const int MKx = stream_variant(c, F, NMK);
-  launch2t_fn fn = get_launch2t(MKx, NU, F, NMK);
-  occ2t_fn occ = get_occ2t(MKx, NU, F, NMK);
-  if (!fn || !occ) return DN_OK;
+  Kernel* k = find2t(stream_variant(c, F, NMK), NU, F, NMK);
+  if (!k) return DN_OK;
   P2T p;
   memset(&p, 0, sizeof(p));
-  int nf = 0;
-  p.fld[nf++] = c.u;
-  if (NU) p.fld[nf++] = c.nu;
-  if (F) p.fld[nf++] = c.f;
-  if (NMK) p.fld[nf++] = c.numask;
-  for (int i = 0; i < c.nmasks; ++i) { p.fld[nf++] = c.mk[i].m; p.mval[i] = c.mk[i].v; }
-  if (c.MK == 4) p.fld[nf++] = c.mk[0].vf;
+  const int nf = stream_fields(c, p.fld, p.mval);
   for (int i = 0; i < nf; ++i)
     if (p.fld[i].sy != g->nx) return DN_OK;      // bulk copies take whole runs of rows
-  Plan2T pl = plan2t(g, nf, c.sms, occ);
+  Plan2T pl = plan2t(g, nf, c.sms, k);
   if (!pl.ok) { cudaGetLastError(); return DN_OK; }
   if (pl.grid > 0x7fffffffLL) return DN_OK;
   if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
@@ -155,7 +137,7 @@ int run2t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
   p.grad = o.grad;
   p.mode = c.mode;
   *handled = true;
-  return check_cuda(fn(p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)o.stream),
+  return check_cuda(launch(*k, &p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)o.stream, true),
                     "fem2d_tma launch");
 }
 

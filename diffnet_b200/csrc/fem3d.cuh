@@ -490,21 +490,8 @@ __global__ void __launch_bounds__(DN_MAXT_3D) k_fem3d(const P3D p) {
   }
 }
 
-// ---- dispatch / planning (fem3d_dispatch.cu) -----------------------------------------------
-typedef cudaError_t (*launch3d_fn)(const P3D&, dim3, dim3, size_t, cudaStream_t);
-launch3d_fn get_launch3d(int V, int MK, int NU, int FM, int NUMASK);
-
+// The kernel of one fem3d_combos.h variant (MK as in dn_launch.h), instantiated by fem3d_inst.cu.
 template <int V, int MK, bool HAS_NU, int FM, bool NUMASK>
-cudaError_t launch3d(const P3D& p, dim3 grid, dim3 block, size_t smem, cudaStream_t s) {
-  constexpr int NM = (MK == 4) ? 1 : MK;
-  constexpr bool VF = (MK == 4);
-  auto kern = k_fem3d<V, NM, VF, HAS_NU, FM, NUMASK>;
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-  }
-  kern<<<grid, block, smem, s>>>(p);
-  return cudaGetLastError();
-}
+const void* kernel3d();
 
 }  // namespace dn

@@ -1,4 +1,5 @@
 // Instantiation list of k_fem3d: X(V, MK, HAS_NU, FM, NUMASK) -- see fem2d_combos.h for the codes.
+// DN3D_COMBOS(X, V, MK) is one slice (one object file, see build.py), DN3D_ALL(X) all of them.
 #pragma once
 #define DN3D_COMBOS(X, V, MK)                                                         \
   X(V, MK, false, 0, false) X(V, MK, false, 1, false) X(V, MK, false, 2, false)       \

@@ -1,20 +1,19 @@
-// Launch planning and runtime -> compile-time dispatch of the 3-D kernel family.
+// Launch planning and runtime -> compile-time dispatch of the 3-D kernel family (instantiated by fem3d_inst.cu).
 #include "dn_launch.h"
 #include "fem3d.cuh"
 #include "fem3d_combos.h"
 
 namespace dn {
-#define DN_EXT(V, MK, NU, FM, NMK) \
-  extern template cudaError_t launch3d<V, MK, NU, FM, NMK>(const P3D&, dim3, dim3, size_t, cudaStream_t);
-DN3D_ALL(DN_EXT)
-#undef DN_EXT
 
-launch3d_fn get_launch3d(int V, int MK, int NU, int FM, int NUMASK) {
-#define DN_CASE(V_, MK_, NU_, FM_, NMK_)                                                    \
-  if (V == V_ && MK == MK_ && NU == (int)NU_ && FM == FM_ && NUMASK == (int)NMK_)           \
-    return &launch3d<V_, MK_, NU_, FM_, NMK_>;
-  DN3D_ALL(DN_CASE)
-#undef DN_CASE
+// The kernel of a variant of fem3d_combos.h, or null when it is not instantiated.
+static Kernel* find3d(int V, int MK, int NU, int FM, int NUMASK) {
+  static struct { int V, MK, NU, FM, NUMASK; Kernel k; } tab[] = {
+#define DN_ROW(V_, MK_, NU_, FM_, NMK_) {V_, MK_, NU_, FM_, NMK_, {kernel3d<V_, MK_, NU_, FM_, NMK_>()}},
+      DN3D_ALL(DN_ROW)
+#undef DN_ROW
+  };
+  for (auto& r : tab)
+    if (r.V == V && r.MK == MK && r.NU == NU && r.FM == FM && r.NUMASK == NUMASK) return &r.k;
   return nullptr;
 }
 
@@ -100,12 +99,12 @@ int run3d(const Common& c, const dn_geom* g, const Out& o) {
   p.grad = o.grad;
   p.mode = c.mode; p.mask_input = c.mask_input;
   const int FM = c.f.p ? 1 : (c.fgp.p ? 2 : 0);
-  launch3d_fn fn = get_launch3d(pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0);
-  if (!fn)
+  Kernel* k = find3d(pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0);
+  if (!k)
     return fail(DN_EINVAL, "unsupported option combination (V=%d MK=%d nu=%d fmode=%d numask=%d)",
                 pl.V, c.MK, c.nu.p ? 1 : 0, FM, c.numask.p ? 1 : 0);
-  return check_cuda(fn(p, dim3((unsigned)pl.grid), dim3(pl.LX, pl.TY + 1), pl.smem,
-                       (cudaStream_t)o.stream), "fem3d launch");
+  return check_cuda(launch(*k, &p, dim3((unsigned)pl.grid), dim3(pl.LX, pl.TY + 1), pl.smem,
+                           (cudaStream_t)o.stream, false), "fem3d launch");
 }
 
 }  // namespace dn

@@ -678,54 +678,8 @@ __global__ void __maxnreg__(DN_T3_REGS_OF(HAS_NU)) k_fem3d_tma(const __grid_cons
   finish_loss_w0<8>(p.red, cta, s_ticket);   // 3-D grids are a few hundred CTAs
 }
 
-// ---- dispatch (fem3d_tma_dispatch.cu) --------------------------------------------------------
-typedef cudaError_t (*launch3t_fn)(const P3T&, dim3, dim3, size_t, cudaStream_t);
-typedef int (*occ3t_fn)(int, size_t);
-launch3t_fn get_launch3t(int MK, int NU, int F, int NUMASK, int LK);
-occ3t_fn get_occ3t(int MK, int NU, int F, int NUMASK, int LK);
-
+// The kernel of one fem3d_tma_combos.h variant (MK as in dn_launch.h), instantiated by fem3d_tma_inst.cu.
 template <int MK, int NUK, int FK, bool NUMASK, bool LK>
-struct Kern3T {
-  // MK 0..3 / 4 / 5..7 as in fem2d_tma.cuh (5..7: mask_input = 0)
-  static constexpr int NM = (MK == 4) ? 1 : (MK >= 5 ? MK - 4 : MK);
-  static auto get() { return k_fem3d_tma<NM, (MK == 4), (NUK == 1 || NUK == 2), FK, NUMASK, (MK < 5), (NUK >= 2), LK>; }
-};
-
-template <int MK, int NUK, int FK, bool NUMASK, bool LK>
-cudaError_t prep3t() {
-  static bool done[64] = {};
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  if (dev >= 0 && dev < 64 && done[dev]) return cudaSuccess;
-  e = cudaFuncSetAttribute(Kern3T<MK, NUK, FK, NUMASK, LK>::get(),
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxDynSmem);
-  if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
-  return e;
-}
-
-template <int MK, int NUK, int FK, bool NUMASK, bool LK>
-cudaError_t launch3t(const P3T& p, dim3 grid, dim3 block, size_t smem, cudaStream_t s) {
-  cudaError_t e = prep3t<MK, NUK, FK, NUMASK, LK>();
-  if (e != cudaSuccess) return e;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  if (pdl_enabled()) { cfg.attrs = at; cfg.numAttrs = 1; }
-  return cudaLaunchKernelEx(&cfg, Kern3T<MK, NUK, FK, NUMASK, LK>::get(), p);
-}
-
-template <int MK, int NUK, int FK, bool NUMASK, bool LK>
-int occ3t(int threads, size_t smem) {
-  if (prep3t<MK, NUK, FK, NUMASK, LK>() != cudaSuccess) return 0;
-  int n = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, Kern3T<MK, NUK, FK, NUMASK, LK>::get(), threads,
-                                                    smem) != cudaSuccess)
-    return 0;
-  return n;
-}
+const void* kernel3t();
 
 }  // namespace dn

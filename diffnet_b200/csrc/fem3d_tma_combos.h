@@ -21,11 +21,15 @@
 #define DN3T_COMBOS_2(X) DN3T_COMBOS_PLAIN(X, 2) DN3T_COMBOS_LINKED(X, 2)
 #define DN3T_COMBOS_3(X) DN3T_COMBOS_PLAIN(X, 3) DN3T_COMBOS_LINKED(X, 3)
 #define DN3T_COMBOS_4(X) DN3T_COMBOS_PLAIN(X, 4)
-#define DN3T_CAT_(a, b) a##b
-#define DN3T_COMBOS(X, MK) DN3T_CAT_(DN3T_COMBOS_, MK)(X)
 // MK 5..7 (mask_input = 0, the resmin backward operator): no source term, no nu mask
 #define DN3T_COMBOS_OP(X, MK) \
   X(MK, 0, false, false, false) X(MK, 1, false, false, false) X(MK, 2, false, false, false) X(MK, 3, false, false, false)
+#define DN3T_COMBOS_5(X) DN3T_COMBOS_OP(X, 5)
+#define DN3T_COMBOS_6(X) DN3T_COMBOS_OP(X, 6)
+#define DN3T_COMBOS_7(X) DN3T_COMBOS_OP(X, 7)
+// DN3T_COMBOS(X, MK) is one slice (one object file, see build.py), DN3T_ALL(X) all of them.
+#define DN3T_CAT_(a, b) a##b
+#define DN3T_COMBOS(X, MK) DN3T_CAT_(DN3T_COMBOS_, MK)(X)
 #define DN3T_ALL(X)                                                                              \
   DN3T_COMBOS(X, 0) DN3T_COMBOS(X, 1) DN3T_COMBOS(X, 2) DN3T_COMBOS(X, 3) DN3T_COMBOS(X, 4)             \
-  DN3T_COMBOS_OP(X, 5) DN3T_COMBOS_OP(X, 6) DN3T_COMBOS_OP(X, 7)
+  DN3T_COMBOS(X, 5) DN3T_COMBOS(X, 6) DN3T_COMBOS(X, 7)

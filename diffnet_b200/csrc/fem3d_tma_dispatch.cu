@@ -1,5 +1,5 @@
-// Launch planning and runtime -> compile-time dispatch of the streaming 3-D kernel family
-// (instantiated in gen/fem3dt_mk*.cu).
+// Launch planning and runtime -> compile-time dispatch of the streaming 3-D kernel family (instantiated by
+// fem3d_tma_inst.cu).
 #include <cstdio>
 #include <cstdlib>
 
@@ -9,27 +9,16 @@
 #include "fem3d_tma_combos.h"
 
 namespace dn {
-#define DN_EXT(MK, NU, F, NMK, LK)                                                                        \
-  extern template cudaError_t launch3t<MK, NU, F, NMK, LK>(const P3T&, dim3, dim3, size_t, cudaStream_t); \
-  extern template int occ3t<MK, NU, F, NMK, LK>(int, size_t);
-DN3T_ALL(DN_EXT)
-#undef DN_EXT
 
-launch3t_fn get_launch3t(int MK, int NU, int F, int NUMASK, int LK) {
-#define DN_CASE(MK_, NU_, F_, NMK_, LK_)                                                          \
-  if (MK == MK_ && NU == (int)NU_ && F == (int)F_ && NUMASK == (int)NMK_ && LK == (int)LK_)       \
-    return &launch3t<MK_, NU_, F_, NMK_, LK_>;
-  DN3T_ALL(DN_CASE)
-#undef DN_CASE
-  return nullptr;
-}
-
-occ3t_fn get_occ3t(int MK, int NU, int F, int NUMASK, int LK) {
-#define DN_CASE(MK_, NU_, F_, NMK_, LK_)                                                          \
-  if (MK == MK_ && NU == (int)NU_ && F == (int)F_ && NUMASK == (int)NMK_ && LK == (int)LK_)       \
-    return &occ3t<MK_, NU_, F_, NMK_, LK_>;
-  DN3T_ALL(DN_CASE)
-#undef DN_CASE
+// The kernel of a variant of fem3d_tma_combos.h, or null when it is not instantiated.
+static Kernel* find3t(int MK, int NU, int F, int NUMASK, int LK) {
+  static struct { int MK, NU, F, NUMASK, LK; Kernel k; } tab[] = {
+#define DN_ROW(MK_, NU_, F_, NMK_, LK_) {MK_, NU_, F_, NMK_, LK_, {kernel3t<MK_, NU_, F_, NMK_, LK_>()}},
+      DN3T_ALL(DN_ROW)
+#undef DN_ROW
+  };
+  for (auto& r : tab)
+    if (r.MK == MK && r.NU == NU && r.F == F && r.NUMASK == NUMASK && r.LK == LK) return &r.k;
   return nullptr;
 }
 
@@ -87,8 +76,8 @@ static size_t smem_3t(int S, int nf, int fstride) {
 // bound; CTAs on one SM share the pipe):
 //   SM time ~ ceil(grid / SMs) * threads * (ZC + 1)   [thread-layers executed by the busiest SM]
 // with a penalty when fewer than 12 warps per SM are resident and a mild preference for one wave.
-// `occ` may be null (workspace sizing): then the register bound is assumed.
-static Plan3T plan3t(const dn_geom* g, int nf, int sms, occ3t_fn occ, int maxt_variant, long long min_grid = 0) {
+// `k` may be null (workspace sizing): then the register bound is assumed instead of its occupancy.
+static Plan3T plan3t(const dn_geom* g, int nf, int sms, Kernel* k, int maxt_variant, long long min_grid = 0) {
   Plan3T best;
   memset(&best, 0, sizeof(best));
   if (g->nx % 4 != 0 || g->nx < 8) return best;
@@ -134,7 +123,7 @@ static Plan3T plan3t(const dn_geom* g, int nf, int sms, occ3t_fn occ, int maxt_v
       while (S > 2 && smem_3t(S, nf, fstride) > (size_t)kMaxDynSmem) --S;
       const size_t smem = smem_3t(S, nf, fstride);
       if (smem > (size_t)kMaxDynSmem) continue;
-      int cps = occ ? occ(threads, smem) : (int)(65536 / (threads * (maxt_variant > 512 ? 96 : 128)));
+      int cps = k ? occupancy(*k, threads, smem) : (int)(65536 / (threads * (maxt_variant > 512 ? 96 : 128)));
       if (env_int("DN_DEBUG_PLAN", 0) >= 2)
         fprintf(stderr, "[plan3t] candidate LXT=%d rows=%d TY=%d threads=%d smem=%zu -> %d CTA/SM\n", LXT, rows, TY,
                 threads, smem, cps);
@@ -206,22 +195,14 @@ int run3t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
   const int NU = c.nu.p ? (iso ? 2 : 1) : (iso1 ? 3 : 0), F = c.f.p ? (k.lv ? 2 : 1) : 0, NMK = c.numask.p ? 1 : 0;
   // the load-vector term is nodal: with z-slab ownership a node plane has no single owner
   if (k.lv && (link || g->z_own_hi > g->z_own_lo)) return DN_OK;
-  const int MKx = stream_variant(c, F, NMK);
-  launch3t_fn fn = get_launch3t(MKx, NU, F, NMK, link ? 1 : 0);
-  occ3t_fn occ = get_occ3t(MKx, NU, F, NMK, link ? 1 : 0);
-  if (!fn || !occ || !get_encode()) return DN_OK;
+  Kernel* kern = find3t(stream_variant(c, F, NMK), NU, F, NMK, link ? 1 : 0);
+  if (!kern || !get_encode()) return DN_OK;
   Field fl[DN_T2_MAXF];
   P3T p;
   memset(&p, 0, sizeof(p));
-  int nf = 0;
-  fl[nf++] = u;
-  if (c.nu.p) fl[nf++] = c.nu;
-  if (F) fl[nf++] = c.f;
-  if (NMK) fl[nf++] = c.numask;
-  for (int i = 0; i < c.nmasks; ++i) { fl[nf++] = c.mk[i].m; p.mval[i] = c.mk[i].v; }
-  if (c.MK == 4) fl[nf++] = c.mk[0].vf;
+  const int nf = stream_fields(c, fl, p.mval);
   const long long min_grid = (link && link->halo_plane[0] && env_int("DN_SLAB_WAVES", 0)) ? (long long)(1.9 * sms) : 0;
-  Plan3T pl = plan3t(g, nf, sms, occ, DN_T3_MAXT_OF(c.nu.p != nullptr), min_grid);
+  Plan3T pl = plan3t(g, nf, sms, kern, DN_T3_MAXT_OF(c.nu.p != nullptr), min_grid);
   if (!pl.ok) { cudaGetLastError(); return DN_OK; }
   if (pl.grid > 0x7fffffffLL) return DN_OK;
   int nput = 0;
@@ -306,7 +287,7 @@ int run3t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
             "fstride=%d threads=%d grid=%lld smem=%zu\n", g->batch, g->nx, g->ny, g->nz, pl.LXT, pl.LXo, pl.hl, pl.ntx,
             pl.rows, pl.TY, pl.nty, pl.ZC, pl.nzc, pl.S, pl.BX, pl.BY, pl.fstride, pl.threads, pl.grid, pl.smem);
   *handled = true;
-  return check_cuda(fn(p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)o.stream),
+  return check_cuda(launch(*kern, &p, dim3((unsigned)pl.grid), dim3(pl.threads), pl.smem, (cudaStream_t)o.stream, true),
                     "fem3d_tma launch");
 }
 
