@@ -15,6 +15,7 @@ LIB_PATH = os.environ.get("DIFFNET_FEM_LIB", os.path.join(PKG, "lib", "libdiffne
 DN_MAX_MASKS = 3
 DN_OK, DN_EINVAL, DN_EARCH, DN_ECUDA, DN_EWORKSPACE, DN_ENOSTREAM = 0, -1, -2, -3, -4, -5
 DN_F_LOAD_VECTOR = 1
+DN_REDUCE_NONE = 2          # dn_consts.reduction: one loss per sample
 
 
 class dn_field(C.Structure):
@@ -78,6 +79,8 @@ PROTOTYPES = {
                                        C.c_void_p]),
     "dn_fem_residual_2d_f32": (C.c_int, _RESID_ARGS),
     "dn_fem_residual_3d_f32": (C.c_int, _RESID_ARGS),
+    "dn_fem_residual_reduce_2d_f32": (C.c_int, _RESID_ARGS + [C.c_int]),
+    "dn_fem_residual_reduce_3d_f32": (C.c_int, _RESID_ARGS + [C.c_int]),
     "dn_fem_energy_input_grads_2d_f32": (C.c_int, _EIG_ARGS),
     "dn_fem_energy_input_grads_3d_f32": (C.c_int, _EIG_ARGS),
     "dn_fem_residual_input_grads_2d_f32": (C.c_int, _RIG_ARGS),
@@ -104,6 +107,7 @@ PROTOTYPES = {
     "dn_gen_star_inputs_f32": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dn_gen_box_masks_3d_f32": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dn_scale_inplace_f32": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "dn_scale_per_sample_f32": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p]),
     "dn_peer_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
     "dn_peer_free": (C.c_int, [C.c_void_p]),
     "dn_peer_export": (C.c_int, [C.c_void_p, C.c_char_p]),

@@ -105,16 +105,30 @@ static int check_geom(const dn_geom* g, int nsd, bool spacing = true) {
   return DN_OK;
 }
 
-// Divisor of the loss: 1 for reduction = sum; for mean g->mean_count, else B times the elements the call owns.
+// Divisor of the loss: 1 for reduction = sum; for mean g->mean_count, else B times the elements the call owns; for
+// none (DN_REDUCE_NONE, which check_per_sample admits only without mean_count and z-slab ownership) the elements of
+// one sample.
 static double loss_count(const dn_geom* g, int nsd, int reduction) {
-  if (reduction != 0) return 1.0;
-  if (g->mean_count > 0) return g->mean_count;
+  const bool none = (reduction == DN_REDUCE_NONE);
+  if (reduction != 0 && !none) return 1.0;
+  if (!none && g->mean_count > 0) return g->mean_count;
   double nelz = 1.0;
   if (nsd == 3) {
     const int hi = g->z_own_hi < g->nz - 1 ? g->z_own_hi : g->nz - 1;
     nelz = (g->z_own_hi > g->z_own_lo) ? (double)(hi - g->z_own_lo) : (double)(g->nz - 1);
   }
-  return (double)g->batch * (g->nx - 1) * (double)(g->ny - 1) * nelz;
+  return (none ? 1.0 : (double)g->batch) * (g->nx - 1) * (double)(g->ny - 1) * nelz;
+}
+
+// reduction = none: every sample's loss has to come out of this launch whole, so it refuses what splits a sample
+// (a z-slab holds part of one) or redefines the divisor.
+static int check_per_sample(const dn_geom* g, const dn_slab_link* link) {
+  if (link) return fail(DN_EINVAL, "reduction = none is not available for a linked z-slab launch");
+  if (g->z_own_lo != 0 || g->z_own_hi != 0)
+    return fail(DN_EINVAL, "reduction = none is not available under z-slab ownership (z_own_lo/hi set): a slab holds "
+                           "part of a sample");
+  if (g->mean_count != 0) return fail(DN_EINVAL, "reduction = none takes no mean_count");
+  return DN_OK;
 }
 
 static Field to_field(const dn_field* f) {
@@ -216,6 +230,9 @@ static int energy(int nsd, const dn_field* u, const dn_field* nu, const dn_field
   Common cm;
   if (int rc = prepare(nsd, u, nu, f, fgp, masks, nmasks, nu_zero_mask, g, cs, &cm)) return rc;
   if (o.grad_nu && !cm.nu.p) return fail(DN_EINVAL, "grad_nu requested without nu");
+  cm.per_sample = (cs.reduction == DN_REDUCE_NONE);
+  if (cm.per_sample)
+    if (int rc = check_per_sample(g, link)) return rc;
   cm.mask_input = 1; cm.sms = sms; cm.link = link;
   if (nsd == 2) return run2d(cm, g, o);
   if (int rc = run3d(cm, g, o)) return rc;
@@ -237,16 +254,21 @@ static int energy(int nsd, const dn_field* u, const dn_field* nu, const dn_field
   return check_cuda(launch_grad_nu_3d(q, o.grad_nu, (cudaStream_t)o.stream), "grad_nu launch");
 }
 
-// dn_fem_residual_{2d,3d}_f32
+// dn_fem_residual_reduce_{2d,3d}_f32; reduction 1 (sum) or DN_REDUCE_NONE
 static int residual(int nsd, const dn_field* u, const dn_field* nu, const dn_field* f, const dn_mask* masks,
-                    int nmasks, int apply_masks_to_input, const dn_geom* g, double jac, const Out& o) {
+                    int nmasks, int apply_masks_to_input, const dn_geom* g, double jac, int reduction, const Out& o) {
   int sms = 0;
   if (int rc = device_ok(&sms)) return rc;
   if (!o.grad) return fail(DN_EINVAL, "residual output is NULL");
+  if (reduction != 1 && reduction != DN_REDUCE_NONE)
+    return fail(DN_EINVAL, "residual reduction=%d (1 = sum, %d = none)", reduction, DN_REDUCE_NONE);
   // R = d/du [ sum_e sum_g jac w_g ( 1/2 nu |grad u|^2 - u f ) ]
   const dn_consts cs = {0.5 * jac, jac, 1.0, 1, 0};
   Common cm;
   if (int rc = prepare(nsd, u, nu, f, nullptr, masks, nmasks, nullptr, g, cs, &cm)) return rc;
+  cm.per_sample = (reduction == DN_REDUCE_NONE);
+  if (cm.per_sample)
+    if (int rc = check_per_sample(g, nullptr)) return rc;
   cm.mode = 1; cm.mask_input = apply_masks_to_input ? 1 : 0; cm.sms = sms;
   return nsd == 2 ? run2d(cm, g, o) : run3d(cm, g, o);
 }
@@ -274,7 +296,8 @@ size_t dn_fem_workspace_bytes(const dn_geom* g) {
     cudaGetLastError();
   }
   const long long worst = (g->nsd == 2) ? plan2d_max_ctas(g, sms) : plan3d_max_ctas(g);
-  return ws_bytes_for_grid(worst + 1024);
+  // + one ticket counter per sample for reduction = none (reduce_into)
+  return ws_bytes_for_grid(worst + 1024) + 4 * (size_t)(g->batch > 0 ? g->batch : 0);
 }
 
 int dn_debug_plan(const dn_geom* g, int nfields, int has_nu, int64_t out[16]) {
@@ -315,12 +338,30 @@ int dn_fem_energy_3d_linked_f32(const dn_field* u, const dn_field* nu, const dn_
                 Out{grad_u, nullptr, loss_out, loss_out_f32, workspace, workspace_bytes, stream});
 }
 
+int dn_fem_residual_reduce_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                  const dn_mask* masks, int nmasks, int apply_masks_to_input,
+                                  const dn_geom* g, double jac, float* residual_out, void* workspace,
+                                  size_t workspace_bytes, double* loss_out, float* loss_out_f32,
+                                  void* stream, int reduction) {
+  return residual(2, u, nu, f, masks, nmasks, apply_masks_to_input, g, jac, reduction,
+                  Out{residual_out, nullptr, loss_out, loss_out_f32, workspace, workspace_bytes, stream});
+}
+
 int dn_fem_residual_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
                            const dn_mask* masks, int nmasks, int apply_masks_to_input,
                            const dn_geom* g, double jac, float* residual_out, void* workspace,
                            size_t workspace_bytes, double* loss_out, float* loss_out_f32,
                            void* stream) {
-  return residual(2, u, nu, f, masks, nmasks, apply_masks_to_input, g, jac,
+  return dn_fem_residual_reduce_2d_f32(u, nu, f, masks, nmasks, apply_masks_to_input, g, jac, residual_out,
+                                       workspace, workspace_bytes, loss_out, loss_out_f32, stream, 1);
+}
+
+int dn_fem_residual_reduce_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                  const dn_mask* masks, int nmasks, int apply_masks_to_input,
+                                  const dn_geom* g, double jac, float* residual_out, void* workspace,
+                                  size_t workspace_bytes, double* loss_out, float* loss_out_f32,
+                                  void* stream, int reduction) {
+  return residual(3, u, nu, f, masks, nmasks, apply_masks_to_input, g, jac, reduction,
                   Out{residual_out, nullptr, loss_out, loss_out_f32, workspace, workspace_bytes, stream});
 }
 
@@ -329,8 +370,8 @@ int dn_fem_residual_3d_f32(const dn_field* u, const dn_field* nu, const dn_field
                            const dn_geom* g, double jac, float* residual_out, void* workspace,
                            size_t workspace_bytes, double* loss_out, float* loss_out_f32,
                            void* stream) {
-  return residual(3, u, nu, f, masks, nmasks, apply_masks_to_input, g, jac,
-                  Out{residual_out, nullptr, loss_out, loss_out_f32, workspace, workspace_bytes, stream});
+  return dn_fem_residual_reduce_3d_f32(u, nu, f, masks, nmasks, apply_masks_to_input, g, jac, residual_out,
+                                       workspace, workspace_bytes, loss_out, loss_out_f32, stream, 1);
 }
 
 int dn_peer_loss_sum_f32(const double* slots, int world, const int32_t* step, int64_t max_spins,
@@ -393,6 +434,8 @@ static int energy_input_grads(int nsd, const dn_field* u, const dn_field* nu, co
   if (f && f->ptr && fgp && fgp->ptr) return fail(DN_EINVAL, "give f or fgp, not both");
   InGrad q;
   if (int rc = ingrad_common(nsd, u, nu, f, fgp, masks, nmasks, g, grad_values, &q)) return rc;
+  if (c->reduction == DN_REDUCE_NONE)
+    if (int rc = check_per_sample(g, nullptr)) return rc;
   q.numask = to_field(nu_zero_mask);
   if (q.numask.p && !q.nu.p) return fail(DN_EINVAL, "nu_zero_mask needs nu");
   if (grad_f && !q.f.p) return fail(DN_EINVAL, "grad_f requested without f");
@@ -634,6 +677,15 @@ int dn_scale_inplace_f32(float* x, size_t n, const float* factor_dev, void* stre
   if (!x || !factor_dev) return fail(DN_EINVAL, "NULL pointer");
   if (n == 0) return DN_OK;
   return check_cuda(launch_scale(x, n, factor_dev, (cudaStream_t)stream), "scale launch");
+}
+
+int dn_scale_per_sample_f32(float* x, int batch, size_t n_per_sample, const float* factors_dev, void* stream) {
+  if (int rc = device_ok(nullptr)) return rc;
+  if (!x || !factors_dev) return fail(DN_EINVAL, "NULL pointer");
+  if (batch < 1) return fail(DN_EINVAL, "batch=%d", batch);
+  if (n_per_sample == 0) return DN_OK;
+  return check_cuda(launch_scale_per_sample(x, batch, n_per_sample, factors_dev, (cudaStream_t)stream),
+                    "scale_per_sample launch");
 }
 
 }  // extern "C"

@@ -36,7 +36,20 @@ struct Reduce {
   double* const* peer_slots;
   int* step;             // this rank's launch counter of the current parity (device word)
   int rank, world;
+  // reduction = none (DN_REDUCE_NONE): one loss per sample, loss_out[b].  Sample b owns the partial slots
+  // [seg_lo(b), seg_lo(b) + seg_len(b)) and the ticket counter seg_counter[b] (zero on entry, zero on exit); the
+  // kernel that writes the slot knows its sample.  seg_q == 0: one loss for the whole launch.
+  unsigned int* seg_counter;
+  int seg_q, seg_rem;    // every sample owns seg_q slots, samples [0, seg_rem) one more
 };
+
+__device__ __forceinline__ int seg_lo(const Reduce& r, int b) { return b * r.seg_q + min(b, r.seg_rem); }
+__device__ __forceinline__ int seg_len(const Reduce& r, int b) { return r.seg_q + (b < r.seg_rem ? 1 : 0); }
+// the sample that owns slot i (the inverse of seg_lo): the finishers recompute it rather than keep it live
+__device__ __forceinline__ int seg_of(const Reduce& r, int i) {
+  const int hi = r.seg_rem * (r.seg_q + 1);
+  return i < hi ? i / (r.seg_q + 1) : r.seg_rem + (i - hi) / r.seg_q;
+}
 
 // Folded constants of the closed-form Q1 energy (DESIGN.md "element math"):
 //   kd[d] = S * c_k * W1^nsd * (2/h_d)^2 / 4^nsd(=norm of C) / ... (see host code), kf likewise,
@@ -90,6 +103,39 @@ __device__ __forceinline__ void finish_loss(const Reduce& r, double cta_value, d
     if (r.loss_out) *r.loss_out = tot;
     if (r.loss_f32) *r.loss_f32 = (float)tot;
     *r.counter = 0u;   // self-reset: the workspace is ready for the next call
+  }
+}
+
+// reduction = none in the general kernels: one warp publishes the partial `v` (valid in lane 0) into slot `slot`.
+// The warp that draws the last ticket of the slot's sample b sums the sample's slots in a fixed order (strided over
+// the warp's lanes, then a shuffle tree: bit-reproducible for a given launch shape) and writes loss[b].  Called by
+// the `nlanes` (1..32) threads lanes 0..nlanes-1 of the warp: a 3-D tile block can have fewer than 32 threads.
+__device__ __forceinline__ void finish_sample_warp(const Reduce& r, int slot, double v, int lane, int nlanes) {
+  const unsigned live = nlanes >= 32 ? 0xffffffffu : (1u << nlanes) - 1u;
+  const int b = seg_of(r, slot);
+  unsigned last = 0u;
+  if (lane == 0) {
+    r.partials[slot] = v;
+    __threadfence();
+    last = (atomicAdd(r.seg_counter + b, 1u) == (unsigned)seg_len(r, b) - 1u) ? 1u : 0u;
+  }
+  if (!__shfl_sync(live, last, 0)) return;
+  __threadfence();
+  const int lo = seg_lo(r, b), n = seg_len(r, b);
+  double s = 0.0;
+  for (int i = lane; i < n; i += nlanes) {     // every slot of the sample is read and zeroed
+    s += __ldcg(r.partials + lo + i);
+    __stcg(r.partials + lo + i, 0.0);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double t = __shfl_down_sync(live, s, o);   // from a lane beyond nlanes: undefined, and not used
+    if (lane + o < nlanes) s += t;
+  }
+  if (lane == 0) {
+    if (r.loss_out) r.loss_out[b] = s;
+    if (r.loss_f32) r.loss_f32[b] = (float)s;
+    r.seg_counter[b] = 0u;
   }
 }
 

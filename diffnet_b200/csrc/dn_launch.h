@@ -24,6 +24,7 @@ struct Common {
   int mask_input;            // 0: the mask values are not substituted into the input (operator apply)
   int sms;
   const dn_slab_link* link;  // linked z-slab launch (3-D streaming kernel only), else null
+  bool per_sample;           // reduction = none: one loss per sample (never linked)
 };
 
 // Where a launch writes.
@@ -41,14 +42,22 @@ struct Out {
 inline size_t ws_bytes_for_grid(long long grid) { return 64 + 8 * (size_t)grid; }
 
 // Checks the workspace for a `grid`-CTA launch and points the reduction epilogue at it and at the loss outputs.
-inline int reduce_into(const Out& o, long long grid, Reduce* r) {
-  const size_t need = ws_bytes_for_grid(grid);
+// c.per_sample (reduction = none): the kernel writes `q` partial slots per sample, one more for samples [0, rem), and
+// the workspace also holds one ticket counter per sample behind the slots.
+inline int reduce_into(const Common& c, const Out& o, const dn_geom* g, long long grid, int q, int rem, Reduce* r) {
+  const long long slots = c.per_sample ? (long long)g->batch * q + rem : grid;
+  const size_t need = ws_bytes_for_grid(slots) + (c.per_sample ? 4 * (size_t)g->batch : 0);
   if (!o.workspace || o.wsb < need) return fail(DN_EWORKSPACE, "workspace too small: %zu < %zu", o.wsb, need);
   if ((uintptr_t)o.workspace % 16) return fail(DN_EWORKSPACE, "workspace must be 16-byte aligned");
   r->counter = (unsigned int*)o.workspace;
   r->partials = (double*)((char*)o.workspace + 64);
   r->loss_out = o.loss_out;
   r->loss_f32 = o.loss_f32;
+  if (c.per_sample) {
+    r->seg_counter = (unsigned int*)(r->partials + slots);
+    r->seg_q = q;
+    r->seg_rem = rem;
+  }
   return DN_OK;
 }
 

@@ -336,6 +336,10 @@ __global__ void __launch_bounds__(128) k_fem2d(const P2D p) {
   }
 
   acc = warp_sum(acc);
+  if (p.red.seg_q) {     // reduction = none: one slot per item (warp); the warps of one CTA can hold different samples
+    if (item < p.nitems) finish_sample_warp(p.red, item, acc, lane, 32);
+    return;
+  }
   if (lane == 0) s_red[warp] = acc;
   __syncthreads();
   double cta = 0.0;

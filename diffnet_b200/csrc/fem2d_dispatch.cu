@@ -64,7 +64,8 @@ int run2d(const Common& c, const dn_geom* g, const Out& o) {
   Plan2D pl = plan2d(g, vec4, c.sms);
   P2D p;
   memset(&p, 0, sizeof(p));
-  if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
+  // reduction = none: one slot per item (warp), not per CTA -- the wpc items of a CTA can span two samples
+  if (int rc = reduce_into(c, o, g, pl.grid, pl.ntx * pl.nchunks, 0, &p.red)) return rc;
   p.u = c.u; p.nu = c.nu; p.f = c.f; p.fgp = c.fgp; p.numask = c.numask;
   for (int i = 0; i < DN_MAX_MASKS; ++i) p.mk[i] = c.mk[i];
   p.B = g->batch; p.nx = g->nx; p.ny = g->ny;

@@ -300,7 +300,12 @@ struct Fem2T {
 //   * the finisher polls the slots until none is zero (one batched L2 round trip per sweep), sums them in
 //     a fixed order (lane-strided, then an xor butterfly: bit-reproducible), and zeroes slots and counter
 //     again: the workspace contract (zero on entry, zero on exit) is unchanged.
-__device__ __forceinline__ unsigned int draw_start_ticket(const Reduce& r) { return atomicAdd(r.counter, 1u); }
+//   * reduction = none (r.seg_q > 0): the same scheme per sample.  A CTA draws its ticket from its sample's counter,
+//     the CTA with the sample's last ticket is that sample's finisher and sums only the sample's slots, so the
+//     samples finish in parallel and each finisher's wait is no longer than the whole-launch one.
+__device__ __forceinline__ unsigned int draw_start_ticket(const Reduce& r, int b) {
+  return atomicAdd(r.seg_q ? r.seg_counter + b : r.counter, 1u);
+}
 
 __device__ __forceinline__ long long ld_relaxed_b64(const void* p) {
   long long v;
@@ -308,21 +313,11 @@ __device__ __forceinline__ long long ld_relaxed_b64(const void* p) {
   return v;
 }
 
-// NB = slots per lane fetched per sweep (all of them are live registers while the sweep is checked)
-template <int NB = 40>
-__device__ __forceinline__ void finish_loss_w0(const Reduce& r, double cta_value, unsigned int start_ticket) {
-  if (threadIdx.x >= 32) return;
-  const int lane = threadIdx.x;
-  unsigned fin = 0u;
-  if (lane == 0) {
-    long long bits = __double_as_longlong(cta_value);
-    if ((bits << 1) == 0) bits = (long long)0x8000000000000000ull;      // +-0.0 -> -0.0: never the "empty" pattern
-    __stcg(reinterpret_cast<long long*>(r.partials + blockIdx.x), bits);
-    fin = (start_ticket == gridDim.x - 1) ? 1u : 0u;
-  }
-  fin = __shfl_sync(0xffffffffu, fin, 0);
-  if (!fin) return;
-  const unsigned n = gridDim.x;
+// Waits until the n slots at `slots` are all written, sums them in a fixed order (lane-strided, then the xor
+// butterfly: bit-reproducible) and zeroes them again.  NB = slots per lane fetched per sweep (all of them are live
+// registers while the sweep is checked).  Called by the 32 lanes of warp 0.
+template <int NB>
+__device__ __forceinline__ double sum_slots_w0(double* slots, unsigned n, int lane) {
   double s = 0.0;
   for (unsigned base = 0; base < n; base += 32 * NB) {   // up to NB independent L2 loads per lane in flight
     long long v[NB];
@@ -332,7 +327,7 @@ __device__ __forceinline__ void finish_loss_w0(const Reduce& r, double cta_value
 #pragma unroll
       for (int q = 0; q < NB; ++q) {
         const unsigned i = base + q * 32 + lane;
-        v[q] = (i < n) ? ld_relaxed_b64(r.partials + i) : (long long)0x8000000000000000ull;
+        v[q] = (i < n) ? ld_relaxed_b64(slots + i) : (long long)0x8000000000000000ull;
         all = all && (v[q] != 0);
       }
       all = __all_sync(0xffffffffu, all);
@@ -341,10 +336,56 @@ __device__ __forceinline__ void finish_loss_w0(const Reduce& r, double cta_value
     for (int q = 0; q < NB; ++q) {
       const unsigned i = base + q * 32 + lane;
       s += __longlong_as_double(v[q]);                    // out-of-range slots hold -0.0
-      if (i < n) __stcg(reinterpret_cast<long long*>(r.partials + i), 0ll);   // self-reset
+      if (i < n) __stcg(reinterpret_cast<long long*>(slots + i), 0ll);   // self-reset
     }
   }
-  s = warp_sum(s) + 0.0;                                  // -0.0 (all partials zero) -> +0.0
+  return warp_sum(s) + 0.0;                               // -0.0 (all partials zero) -> +0.0
+}
+
+// reduction = none: sample b's loss `s` (valid in every lane) and the reset of its ticket counter
+__device__ __forceinline__ void finish_sample_w0(const Reduce& r, int b, double s, int lane) {
+  if (lane == 0) {
+    if (r.loss_out) r.loss_out[b] = s;
+    if (r.loss_f32) r.loss_f32[b] = (float)s;
+    r.seg_counter[b] = 0u;
+  }
+}
+
+template <int NB = 40>
+__device__ __forceinline__ void finish_loss_w0(const Reduce& r, double cta_value, unsigned int start_ticket) {
+  if (threadIdx.x >= 32) return;
+  const int lane = threadIdx.x;
+  unsigned fin = 0u;
+  if (lane == 0) {
+    long long bits = __double_as_longlong(cta_value);
+    if ((bits << 1) == 0) bits = (long long)0x8000000000000000ull;      // +-0.0 -> -0.0: never the "empty" pattern
+    __stcg(reinterpret_cast<long long*>(r.partials + blockIdx.x), bits);
+  }
+  unsigned n = gridDim.x;                                // the slots this finisher sums
+  double* slots = r.partials;
+  int b = 0;
+  if (r.seg_q) {           // reduction = none (never linked): this CTA's slot is blockIdx.x, its sample b
+    b = seg_of(r, blockIdx.x);
+    n = (unsigned)seg_len(r, b);
+    if (lane == 0) fin = (start_ticket == n - 1u) ? 1u : 0u;
+    if (!__shfl_sync(0xffffffffu, fin, 0)) return;
+    slots += seg_lo(r, b);
+    if constexpr (NB > 8) {
+      // a sample owns few slots: 8 per lane and sweep suffice, and a second NB-deep sweep would push the largest
+      // 2-D instantiations' march into local memory
+      finish_sample_w0(r, b, sum_slots_w0<8>(slots, n, lane), lane);
+      return;
+    }
+  } else {
+    if (lane == 0) fin = (start_ticket == n - 1u) ? 1u : 0u;
+    fin = __shfl_sync(0xffffffffu, fin, 0);
+    if (!fin) return;
+  }
+  const double s = sum_slots_w0<NB>(slots, n, lane);   // NB == 8 (3-D): one sweep serves both reductions
+  if (r.seg_q) {
+    finish_sample_w0(r, b, s, lane);
+    return;
+  }
   if (r.peer_slots) {      // linked z-slab launch: push the rank total to every rank (NVLink stores), then the flags
     const int want = *r.step + 1;
     if (lane < r.world) {
@@ -434,7 +475,7 @@ __global__ void __launch_bounds__(TB, MINB) k_fem2d_tma(const __grid_constant__ 
     const int n0 = min(S, nst);
     for (int q = 0; q < n0; ++q) issue_stage();     // thread 0 only; the others just count
   }
-  if (tid == 0) s_ticket = draw_start_ticket(p.red);  // its round trip hides behind the first tile loads
+  if (tid == 0) s_ticket = draw_start_ticket(p.red, b);  // its round trip hides behind the first tile loads
   __syncthreads();                                   // barriers initialised before anyone waits
 
   const bool act = tid * 4 < nx;

@@ -119,7 +119,9 @@ int run2t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
   Plan2T pl = plan2t(g, nf, c.sms, k);
   if (!pl.ok) { cudaGetLastError(); return DN_OK; }
   if (pl.grid > 0x7fffffffLL) return DN_OK;
-  if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
+  // a CTA is one chunk of one image; the chunks of an image are consecutive CTAs
+  const bool bal = pl.bal_q > 0;
+  if (int rc = reduce_into(c, o, g, pl.grid, bal ? pl.bal_q : pl.nchunks, bal ? pl.bal_rem : 0, &p.red)) return rc;
   p.nf = nf;
   p.B = g->batch; p.nx = g->nx; p.ny = g->ny;
   p.R = pl.R; p.nchunks = pl.nchunks; p.S = pl.S;

@@ -458,6 +458,10 @@ __global__ void __launch_bounds__(DN_MAXT_3D) k_fem3d(const P3D p) {
   double cta = 0.0;
   if (tid == 0)
     for (int w2 = 0; w2 < (nthreads + 31) / 32; ++w2) cta += s_red[w2];
+  if (p.red.seg_q) {     // reduction = none: a CTA is one work item of one sample, one slot per CTA
+    if (warp == 0) finish_sample_warp(p.red, blockIdx.x, cta, lane, nthreads < 32 ? nthreads : 32);
+    return;
+  }
   __syncthreads();
   // finish_loss indexes threads by threadIdx.x: re-linearise through a 1-D view
   {

@@ -87,7 +87,8 @@ int run3d(const Common& c, const dn_geom* g, const Out& o) {
   if (pl.smem > 200 * 1024) return fail(DN_EINVAL, "3-D tile needs %zu B of shared memory", pl.smem);
   P3D p;
   memset(&p, 0, sizeof(p));
-  if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
+  // a CTA is one (x-tile, y-tile, z-chunk) work item of one sample; the items of a sample are consecutive CTAs
+  if (int rc = reduce_into(c, o, g, pl.grid, pl.ntx * pl.nty * pl.nzc, 0, &p.red)) return rc;
   if (pl.grid > 0x7fffffffLL) return fail(DN_EINVAL, "grid too large");
   p.u = c.u; p.nu = c.nu; p.f = c.f; p.fgp = c.fgp; p.numask = c.numask;
   for (int i = 0; i < DN_MAX_MASKS; ++i) p.mk[i] = c.mk[i];

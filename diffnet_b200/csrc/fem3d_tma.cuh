@@ -433,7 +433,7 @@ __global__ void __maxnreg__(DN_T3_REGS_OF(HAS_NU)) k_fem3d_tma(const __grid_cons
     pdl_wait();
     if ((int)blockIdx.x < nputc) {
       const int want = *p.red.step + 1;
-      if (tid == 0) s_ticket = draw_start_ticket(p.red);
+      if (tid == 0) s_ticket = draw_start_ticket(p.red, 0);
       const int side = (int)blockIdx.x / p.lk.nput, part = (int)blockIdx.x - side * p.lk.nput;
       if (p.lk.pdst[side]) {
         float4* dst = p.lk.pdst[side];
@@ -514,7 +514,7 @@ __global__ void __maxnreg__(DN_T3_REGS_OF(HAS_NU)) k_fem3d_tma(const __grid_cons
     const int n0 = min(S, npl);
     for (int q = 0; q < n0; ++q) issue_plane();
   }
-  if (tid == 0) s_ticket = draw_start_ticket(p.red);   // its round trip hides behind the first plane loads
+  if (tid == 0) s_ticket = draw_start_ticket(p.red, b);   // its round trip hides behind the first plane loads
 
   // ---- thread geometry
   const int r_raw = tid / LXT, lx = tid - r_raw * LXT;

@@ -212,7 +212,8 @@ int run3t(const Common& c, const dn_geom* g, const Out& o, bool* handled) {
     if (nput > 16) nput = 16;
     pl.grid += 2 * nput;
   }
-  if (int rc = reduce_into(o, pl.grid, &p.red)) return rc;
+  // a CTA is one (x-tile, y-tile, z-chunk) work item of one sample; the items of a sample are consecutive CTAs
+  if (int rc = reduce_into(c, o, g, pl.grid, pl.ntx * pl.nty * pl.nzc, 0, &p.red)) return rc;
   for (int i = 0; i < nf; ++i)
     if (!make_map(&p.tm[i], fl[i], g, pl.BX, pl.BY, &p.bmul[i])) return DN_OK;   // general kernel takes it
   p.nf = nf;

@@ -480,6 +480,38 @@ cudaError_t launch_scale(float* x, size_t n, const float* factor_dev, cudaStream
   return cudaGetLastError();
 }
 
+// x[b, :] *= factors[b]: blockIdx.y walks the samples (b = blockIdx.y, + gridDim.y, ...), and a CTA reads the factor
+// of each sample it scales once; 16-byte accesses when the sample's row is aligned (n % 4 == 0 and x aligned), else
+// scalar ones.
+__global__ void __launch_bounds__(256) k_scale_per_sample(float* __restrict__ x, int batch, size_t n,
+                                                          const float* __restrict__ factors) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (int b = blockIdx.y; b < batch; b += gridDim.y) {
+    const float f = __ldg(factors + b);
+    float* xb = x + (size_t)b * n;
+    const size_t n4 = (((uintptr_t)xb % 16) == 0) ? n / 4 : 0;
+    float4* x4 = reinterpret_cast<float4*>(xb);
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n4; i += stride) {
+      float4 v = x4[i];
+      v.x *= f; v.y *= f; v.z *= f; v.w *= f;
+      x4[i] = v;
+    }
+    for (size_t i = n4 * 4 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += stride)
+      xb[i] *= f;
+  }
+}
+
+cudaError_t launch_scale_per_sample(float* x, int batch, size_t n, const float* factors_dev, cudaStream_t s) {
+  long long g = ((long long)(n + 3) / 4 + 255) / 256;
+  long long cap = 16LL * sm_count() / batch;          // ~16 CTAs per SM over the whole launch
+  if (cap < 1) cap = 1;
+  if (g > cap) g = cap;
+  if (g < 1) g = 1;
+  const int gy = batch < 65535 ? batch : 65535;       // the grid's y limit: larger batches loop in the kernel
+  k_scale_per_sample<<<dim3((unsigned)g, (unsigned)gy), 256, 0, s>>>(x, batch, n, factors_dev);
+  return cudaGetLastError();
+}
+
 }  // namespace dn
 
 // ---- general basis / rule / dimension ---------------------------------------------------------------------------

@@ -48,5 +48,6 @@ struct GradNu3 {
 cudaError_t launch_grad_nu_3d(const GradNu3& q, float* out, cudaStream_t s);
 
 cudaError_t launch_scale(float* x, size_t n, const float* factor_dev, cudaStream_t s);
+cudaError_t launch_scale_per_sample(float* x, int batch, size_t n, const float* factors_dev, cudaStream_t s);
 
 }  // namespace dn

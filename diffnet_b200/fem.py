@@ -339,14 +339,16 @@ class DiffNetFEM(PDE):
     def energy_loss(self, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None,
                     c_k=1.0, c_f=1.0, scale=1.0, reduction="mean"):
         """scale * sum_g gpw_g (c_k nu_g |grad u|_g^2 - c_f u_g f_g), mean/sum over batch x elements,
-        with u = where(mask > 0.5, value, u) applied for each (mask, value) of `dirichlet` in order."""
+        with u = where(mask > 0.5, value, u) applied for each (mask, value) of `dirichlet` in order.
+        ``reduction="none"``: one loss per sample, a (B,) tensor whose mean is the "mean" loss."""
         self._q1_only("energy_loss")
         return ops.fem_energy(self.geometry, u, nu=nu, f=f, f_gp=f_gp, dirichlet=dirichlet,
                               nu_zero_mask=nu_zero_mask, c_k=c_k, c_f=c_f, scale=scale,
                               reduction=reduction)
 
     def energy_loss_and_grad(self, u, **kw):
-        """(loss, dloss/du) in one launch, outside autograd."""
+        """(loss, dloss/du) in one launch, outside autograd.  With ``reduction="none"`` loss is (B,) and dloss/du the
+        gradient of loss.sum(): each sample's own gradient."""
         self._q1_only("energy_loss_and_grad")
         return ops.fem_energy_and_grad(self.geometry, u, **kw)
 
@@ -356,10 +358,11 @@ class DiffNetFEM(PDE):
         self._q1_only("prepare_energy")
         return ops.PreparedEnergy(self.geometry, u, **kw)
 
-    def residual_loss(self, u, nu=None, f=None, dirichlet=(), jac=1.0):
-        """sum(R^2) of the assembled, Dirichlet-zeroed Galerkin residual (12_klsum.py:80-132)."""
+    def residual_loss(self, u, nu=None, f=None, dirichlet=(), jac=1.0, reduction="sum"):
+        """sum(R^2) of the assembled, Dirichlet-zeroed Galerkin residual (12_klsum.py:80-132); ``reduction="none"``:
+        one sum per sample, a (B,) tensor."""
         self._q1_only("residual_loss")
-        return ops.fem_residual(self.geometry, u, nu=nu, f=f, dirichlet=dirichlet, jac=jac)
+        return ops.fem_residual(self.geometry, u, nu=nu, f=f, dirichlet=dirichlet, jac=jac, reduction=reduction)
 
     def _q1_only(self, what):
         if self.fem_basis_deg != 1:

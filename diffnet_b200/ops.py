@@ -146,10 +146,31 @@ def _workspace(device: torch.device, stream_ptr: int, nbytes: int) -> torch.Tens
     return ws
 
 
-def _consts(c_k, c_f, scale, reduction, flags=0) -> L.dn_consts:
-    if reduction not in ("mean", "sum"):
-        raise L.DiffNetFEMError("reduction must be 'mean' or 'sum'")
-    return L.dn_consts(float(c_k), float(c_f), float(scale), 0 if reduction == "mean" else 1, flags)
+_REDUCTION = {"mean": 0, "sum": 1, "none": L.DN_REDUCE_NONE}
+
+
+def _check_none(reduction, z_own=None, mean_count=0.0, link=None):
+    """``reduction="none"`` gives one loss per sample, so a launch must hold whole samples: refuse what splits one."""
+    if reduction != "none":
+        return
+    if z_own is not None:
+        raise L.DiffNetFEMError("reduction='none' is not available with z_own: a z-slab holds part of a sample")
+    if mean_count:
+        raise L.DiffNetFEMError("reduction='none' takes no mean_count (each sample is divided by its element count)")
+    if link is not None:
+        raise L.DiffNetFEMError("reduction='none' is not available for a linked (z-slab) launch")
+
+
+def _consts(c_k, c_f, scale, reduction, flags=0, z_own=None, mean_count=0.0, link=None) -> L.dn_consts:
+    """``reduction``: "mean", "sum" or "none" (a (B,) loss, one value per sample)."""
+    if reduction not in _REDUCTION:
+        raise L.DiffNetFEMError("reduction must be 'mean', 'sum' or 'none'")
+    _check_none(reduction, z_own, mean_count, link)
+    return L.dn_consts(float(c_k), float(c_f), float(scale), _REDUCTION[reduction], flags)
+
+
+def _loss_shape(reduction, B):
+    return (B,) if reduction == "none" else ()
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -166,12 +187,16 @@ def _check_f_gp(geom: Geometry, f_gp) -> torch.Tensor:
     return fg
 
 
-def _per_sample(t: Optional[torch.Tensor], B: int) -> Optional[torch.Tensor]:
+def _per_sample(t: Optional[torch.Tensor], B: int, expand: bool = False) -> Optional[torch.Tensor]:
     """The canonical view of a field whose gradient is wanted.  The launch writes ONE (1, ...) gradient summed over
     the batch for a field it reads with stride_b = 0.  A field that spans the batch with stride_b = 0 (``expand``)
-    needs a gradient per sample (autograd's expand backward sums it), so its values are materialised here."""
+    needs a gradient per sample (autograd's expand backward sums it), so its values are materialised here.
+    ``expand=True`` (reduction="none": every sample's gradient gets its own weight) materialises a batch-1 field
+    over the batch as well, at B times its memory."""
     if t is not None and B > 1 and t.shape[0] == B and t.stride(0) == 0:
         return t.contiguous()
+    if expand and t is not None and B > 1 and t.shape[0] == 1:
+        return t.expand((B,) + tuple(t.shape[1:])).contiguous()
     return t
 
 
@@ -181,12 +206,13 @@ class _Args:
     ``B`` is the batch of the launch: the largest batch among all inputs (every other one is 1 or ``B``).  The ctypes
     arguments are ``c_u``, ``c_nu``, ``c_f``, ``c_fgp``, ``c_nzm``, ``c_R`` (``C.byref(dn_field)``, or None for an
     absent input) and ``marr``, ``nm`` (the ``dn_mask`` array and its length); this object holds the views they point
-    into.  ``want`` names the fields (``"nu"``, ``"f"``) and ``want_values`` flags the tensor Dirichlet values (list
-    order) whose gradient the launch writes: those take the ``_per_sample`` view.  ``bind=True`` (a prepared call,
-    which reads the same storage on every later call) refuses an input that would have to be copied."""
+    into.  ``want`` names the fields (``"nu"``, ``"f"``, ``"f_gp"``) and ``want_values`` flags the tensor Dirichlet
+    values (list order) whose gradient the launch writes: those take the ``_per_sample`` view (``per_sample=True``:
+    a gradient per sample even for a field shared by the batch).  ``bind=True`` (a prepared call, which reads the
+    same storage on every later call) refuses an input that would have to be copied."""
 
     def __init__(self, geom: Geometry, u=None, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None, R=None,
-                 want=(), want_values=(), bind=False):
+                 want=(), want_values=(), bind=False, per_sample=False):
         def canon(t, name):
             if t is None:
                 return None
@@ -218,13 +244,15 @@ class _Args:
                 B = max(B, t.shape[0])
         self.B = B
         if "nu" in want:
-            self.nu = _per_sample(self.nu, B)
+            self.nu = _per_sample(self.nu, B, per_sample)
         if "f" in want:
-            self.f = _per_sample(self.f, B)
+            self.f = _per_sample(self.f, B, per_sample)
+        if "f_gp" in want:
+            self.fg = _per_sample(self.fg, B, per_sample)
         flags = iter(want_values)
         self.want_v = [i for i, v in enumerate(values) if v is not None and next(flags, False)]
         for i in self.want_v:
-            values[i] = _per_sample(values[i], B)
+            values[i] = _per_sample(values[i], B, per_sample)
         self.masks, self.values = masks, values
         self.dev = (self.u if self.u is not None else self.fg).device
 
@@ -303,11 +331,13 @@ def energy_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_z
                c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", want_grad=True, want_grad_nu=False,
                z_own=None, mean_count=0.0, want_double=False, load_vector=False):
     """One fused launch.  Returns (loss 0-dim fp32, grad_u (B,*spatial) or None,
-    grad_nu or None[, loss fp64 0-dim]).
+    grad_nu or None[, loss fp64 0-dim]).  With ``reduction="none"`` both losses are (B,), one per sample, and the
+    gradients are each sample's own.
 
     ``load_vector=True``: ``f`` is an assembled load vector (``load_vector()``), not a nodal source.  A call with
     ``f_gp`` takes that route by itself (assembling b once per f_gp tensor and version) whenever the streaming
     kernels can run the launch, and reads f_gp in the general kernels otherwise."""
+    cs = _consts(c_k, c_f, scale, reduction, L.DN_F_LOAD_VECTOR if load_vector else 0, z_own, mean_count)
     if (f_gp is not None and f is None and USE_LOAD_VECTOR and not load_vector and z_own is None
             and not want_grad_nu):
         _check_f_gp(geom, f_gp)
@@ -322,13 +352,12 @@ def energy_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_z
     a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask)
     if load_vector and (a.f is None or a.fg is not None):
         raise L.DiffNetFEMError("load_vector=True: pass the assembled vector as f (and no f_gp)")
-    cs = _consts(c_k, c_f, scale, reduction, L.DN_F_LOAD_VECTOR if load_vector else 0)
     B, dev = a.B, a.dev
     g = _geom_struct(geom, B, z_own, mean_count)
     grad = _new_out((B,) + geom.spatial, dev) if want_grad else None
     grad_nu = _new_out((B,) + geom.spatial, dev) if want_grad_nu else None
-    loss = _new_out((), dev)
-    loss64 = torch.empty((), dtype=torch.float64, device=dev) if want_double else None
+    loss = _new_out(_loss_shape(reduction, B), dev)
+    loss64 = torch.empty(_loss_shape(reduction, B), dtype=torch.float64, device=dev) if want_double else None
     lib = L.lib()
     stream = torch.cuda.current_stream(dev).cuda_stream
     with _on_device(dev):
@@ -348,14 +377,14 @@ class PreparedEnergy:
     u-as-parameter solves (solve_in_object_3d.py, LBFGS closures), the z-slab steps, benchmarks.
 
     The returned ``(loss, grad)`` are the SAME tensors on every call (overwritten in place):
-    consume or copy them before calling again.  In-place updates of the bound tensors are seen
+    consume or copy them before calling again.  ``reduction="none"``: ``loss`` is a (B,) buffer.  In-place updates of the bound tensors are seen
     (pointers, not values, are captured); re-prepare if a tensor is reallocated."""
 
     def __init__(self, geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet=(), nu_zero_mask=None,
                  c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", z_own=None, mean_count=0.0, link=None):
         """``link``: a ``_lib.dn_slab_link`` (3-D only, see include/diffnet_fem.h) -- the launch then also
         exchanges the z-halo planes of u with the neighbouring ranks and pushes the loss partial."""
-        cs = _consts(c_k, c_f, scale, reduction)
+        cs = _consts(c_k, c_f, scale, reduction, 0, z_own, mean_count, link)
         if link is not None and (geom.nsd != 3 or f_gp is not None):
             raise L.DiffNetFEMError("a linked (z-slab) call is 3-D with a nodal source term")
         if f is not None and f_gp is not None:
@@ -365,7 +394,7 @@ class PreparedEnergy:
         self.device, self._B = a.dev, a.B
         self._g = g = _geom_struct(geom, a.B, z_own, mean_count)
         self.grad = _new_out((a.B,) + geom.spatial, a.dev)
-        self.loss = _new_out((), a.dev)
+        self.loss = _new_out(_loss_shape(reduction, a.B), a.dev)
         self._loss_ptr = C.c_void_p(self.loss.data_ptr())
         grad = C.c_void_p(self.grad.data_ptr())
         lib = L.lib()
@@ -412,21 +441,26 @@ class PreparedEnergy:
         return self.loss, self.grad
 
 
-def residual_raw(geom: Geometry, u, nu=None, f=None, dirichlet=(), jac=1.0, apply_masks_to_input=True):
-    """R = jac*(K(nu) u' - F(f)) masked, and sum(R^2).  Returns (loss 0-dim, R (B,*spatial))."""
+def residual_raw(geom: Geometry, u, nu=None, f=None, dirichlet=(), jac=1.0, apply_masks_to_input=True,
+                 reduction="sum"):
+    """R = jac*(K(nu) u' - F(f)) masked, and sum(R^2).  Returns (loss 0-dim, R (B,*spatial));
+    ``reduction="none"``: loss (B,), the sum of R^2 over each sample."""
+    if reduction not in ("sum", "none"):
+        raise L.DiffNetFEMError("residual reduction must be 'sum' or 'none'")
     a = _Args(geom, u, nu, f, dirichlet=dirichlet)
     B, dev = a.B, a.dev
     g = _geom_struct(geom, B)
     R = _new_out((B,) + geom.spatial, dev)
-    loss = _new_out((), dev)
+    loss = _new_out(_loss_shape(reduction, B), dev)
     lib = L.lib()
     stream = torch.cuda.current_stream(dev).cuda_stream
     with _on_device(dev):
         ws = _workspace_for(lib, g, geom, B, dev, stream)
-        fn = lib.dn_fem_residual_2d_f32 if geom.nsd == 2 else lib.dn_fem_residual_3d_f32
+        fn = lib.dn_fem_residual_reduce_2d_f32 if geom.nsd == 2 else lib.dn_fem_residual_reduce_3d_f32
         rc = fn(a.c_u, a.c_nu, a.c_f, a.marr, a.nm, 1 if apply_masks_to_input else 0, C.byref(g), float(jac),
-                _ptr(R), C.c_void_p(ws.data_ptr()), ws.numel(), None, _ptr(loss), C.c_void_p(stream))
-    L.check(rc, f"dn_fem_residual_{geom.nsd}d_f32")
+                _ptr(R), C.c_void_p(ws.data_ptr()), ws.numel(), None, _ptr(loss), C.c_void_p(stream),
+                _REDUCTION[reduction])
+    L.check(rc, f"dn_fem_residual_reduce_{geom.nsd}d_f32")
     return loss, R
 
 
@@ -435,9 +469,12 @@ def energy_input_grads_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirich
                            want_f_gp=False, want_values=()):
     """dL/df, dL/df_gp and dL/d(value field) of the energy loss in ONE launch (dn_fem_energy_input_grads_*).
     ``want_values``: one flag per tensor Dirichlet value, in list order.  Returns (grad_f | None,
-    grad_f_gp | None, [grad per tensor value | None]); a gradient of a field broadcast over the batch is (1, ...)."""
-    cs = _consts(c_k, c_f, scale, reduction)
-    a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask, want=("f",) if want_f else (), want_values=want_values)
+    grad_f_gp | None, [grad per tensor value | None]); a gradient of a field broadcast over the batch is (1, ...).
+    ``reduction="none"``: every gradient is per sample, (B, ...), the gradient of that sample's loss."""
+    cs = _consts(c_k, c_f, scale, reduction, 0, None, mean_count)
+    want = ("f",) * want_f + ("f_gp",) * want_f_gp
+    a = _Args(geom, u, nu, f, f_gp, dirichlet, nu_zero_mask, want=want, want_values=want_values,
+              per_sample=reduction == "none")
     g = _geom_struct(geom, a.B, None, mean_count)
     gf = a.grad_out(a.f, geom.spatial) if want_f else None
     gfg = a.grad_out(a.fg, (geom.ngp_1d ** geom.nsd,) + geom.elems) if want_f_gp else None
@@ -452,12 +489,13 @@ def energy_input_grads_raw(geom: Geometry, u, nu=None, f=None, f_gp=None, dirich
 
 
 def residual_input_grads_raw(geom: Geometry, u, R, nu=None, f=None, dirichlet=(), jac=1.0, want_nu=False,
-                             want_f=False, want_values=()):
+                             want_f=False, want_values=(), per_sample=False):
     """dL/dnu, dL/df and dL/d(value field) of the residual loss sum(R^2) in ONE launch
     (dn_fem_residual_input_grads_*); ``R`` is the residual the forward returned.  Returns (grad_nu | None,
-    grad_f | None, [grad per tensor value | None])."""
+    grad_f | None, [grad per tensor value | None]).  ``per_sample=True``: every gradient is (B, ...), the gradient
+    of its sample's sum(R^2), also for a field shared by the batch."""
     want = ("nu",) * want_nu + ("f",) * want_f
-    a = _Args(geom, u, nu, f, dirichlet=dirichlet, R=R, want=want, want_values=want_values)
+    a = _Args(geom, u, nu, f, dirichlet=dirichlet, R=R, want=want, want_values=want_values, per_sample=per_sample)
     g = _geom_struct(geom, a.B)
     gnu = a.grad_out(a.nu, geom.spatial) if want_nu else None
     gf = a.grad_out(a.f, geom.spatial) if want_f else None
@@ -484,6 +522,25 @@ def scale_inplace_(x: torch.Tensor, factor: torch.Tensor) -> torch.Tensor:
     return x
 
 
+def scale_per_sample_(x: torch.Tensor, factors: torch.Tensor) -> torch.Tensor:
+    """x[b] *= factors[b] for a (B, ...) tensor and a (B,) device tensor of factors, no host sync."""
+    _require_cuda(x, "x")
+    assert x.is_contiguous() and x.dtype == torch.float32
+    B = x.shape[0]
+    fac = factors.detach().to(device=x.device, dtype=torch.float32).reshape(B).contiguous()
+    stream = torch.cuda.current_stream(x.device).cuda_stream
+    with _on_device(x.device):
+        rc = L.lib().dn_scale_per_sample_f32(C.c_void_p(x.data_ptr()), B, x.numel() // max(B, 1),
+                                             C.c_void_p(fac.data_ptr()), C.c_void_p(stream))
+    L.check(rc, "dn_scale_per_sample_f32")
+    return x
+
+
+def _scale(x: torch.Tensor, gout: torch.Tensor) -> torch.Tensor:
+    """x *= grad_output: one factor (reduction "mean" / "sum"), or one per sample (reduction "none", gout (B,))."""
+    return scale_inplace_(x, gout) if gout.dim() == 0 else scale_per_sample_(x, gout)
+
+
 def _like_input(grad_b: torch.Tensor, ref: torch.Tensor, geom: Geometry) -> torch.Tensor:
     """Reduce/reshape a dense (B,*spatial) gradient to the shape of the tensor the user passed."""
     if ref.dim() == geom.nsd:                       # bare field broadcast over the batch
@@ -497,7 +554,8 @@ def _like_input(grad_b: torch.Tensor, ref: torch.Tensor, geom: Geometry) -> torc
 
 # ------------------------------------------------------------------------------ autograd
 class FEMEnergyFunction(torch.autograd.Function):
-    """loss = energy(u, nu, ...); backward returns grad_output * dloss/du (and dloss/dnu).
+    """loss = energy(u, nu, ...); backward returns grad_output * dloss/du (and dloss/dnu).  With reduction="none"
+    the loss is (B,) and grad_output weighs each sample's gradient (dn_scale_per_sample_f32).
 
     Forward AND gradient come from the single fused launch in forward(); backward only scales
     (in place, skipped on the device when grad_output == 1).  First-order only
@@ -554,9 +612,9 @@ class FEMEnergyFunction(torch.autograd.Function):
         saved = list(ctx.saved_tensors)
         gu = gnu = None
         if ctx.has[0]:
-            gu = _like_input(scale_inplace_(saved.pop(0), gout), ctx.u_ref, ctx.geom)
+            gu = _like_input(_scale(saved.pop(0), gout), ctx.u_ref, ctx.geom)
         if ctx.has[1]:
-            gnu = _like_input(scale_inplace_(saved.pop(0), gout), ctx.nu_ref, ctx.geom)
+            gnu = _like_input(_scale(saved.pop(0), gout), ctx.nu_ref, ctx.geom)
         if ctx.extra is None:
             return (gu, gnu) + (None,) * (11 + ctx.nvalues)
         need_f, need_fgp, need_v, _, dirichlet, c_k, c_f, scale, reduction, mean_count = ctx.extra
@@ -565,28 +623,33 @@ class FEMEnergyFunction(torch.autograd.Function):
         gf, gfg, gv = energy_input_grads_raw(ctx.geom, u, nu, f, f_gp, dirichlet, nzm, c_k, c_f, scale, reduction,
                                              mean_count, want_f=need_f, want_f_gp=need_fgp, want_values=need_v)
         if gf is not None:
-            gf = _like_input(scale_inplace_(gf, gout), f, ctx.geom)
+            gf = _like_input(_scale(gf, gout), f, ctx.geom)
         if gfg is not None:
-            gfg = scale_inplace_(gfg, gout).reshape(f_gp.shape)
-        gv = [None if g is None else _like_input(scale_inplace_(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
+            gfg = _scale(gfg, gout)
+            if gfg.shape[0] > 1 and (f_gp.dim() == ctx.geom.nsd + 1 or f_gp.shape[0] == 1):
+                gfg = gfg.sum(0, keepdim=True)    # reduction="none": per-sample gradients of a shared f_gp
+            gfg = gfg.reshape(f_gp.shape)
+        gv = [None if g is None else _like_input(_scale(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
         return (gu, gnu, None, gf, gfg) + (None,) * 8 + tuple(gv)
 
 
 class FEMResidualFunction(torch.autograd.Function):
     """loss = sum(R^2); dL/du = mask( K(nu) (2R) ) -- one more pass of the same operator
-    (K is symmetric; R is already zero on the Dirichlet nodes).
+    (K is symmetric; R is already zero on the Dirichlet nodes).  reduction="none": loss[b] = sum of R^2 over sample
+    b, and a (B,) grad_output weighs each sample's gradient.
 
     The tensor Dirichlet values follow the fixed arguments (``*values``).  When ``nu``, ``f`` or a value requires
     grad, backward runs ONE more launch (dn_fem_residual_input_grads_*) for those gradients."""
 
     @staticmethod
-    def forward(ctx, u, geom, nu, f, dirichlet, jac, *values):
-        loss, R = residual_raw(geom, u.detach(), nu, f, dirichlet, jac, True)
+    def forward(ctx, u, geom, nu, f, dirichlet, jac, reduction, *values):
+        loss, R = residual_raw(geom, u.detach(), nu, f, dirichlet, jac, True, reduction)
         ctx.geom, ctx.nu, ctx.dirichlet, ctx.jac, ctx.u_ref = geom, nu, dirichlet, jac, u
+        ctx.per_sample = reduction == "none"
         ctx.nvalues = len(values)
         need_nu = nu is not None and ctx.needs_input_grad[2]
         need_f = f is not None and ctx.needs_input_grad[3]
-        need_v = tuple(ctx.needs_input_grad[6:])
+        need_v = tuple(ctx.needs_input_grad[7:])
         ctx.extra = None
         if need_nu or need_f or any(need_v):
             ctx.extra = (need_nu, need_f, need_v)
@@ -603,23 +666,23 @@ class FEMResidualFunction(torch.autograd.Function):
         if ctx.extra is None:
             _, KR = residual_raw(ctx.geom, R, ctx.nu, None, ctx.dirichlet, ctx.jac, False)
             g = KR.mul_(2.0)
-            g = scale_inplace_(g, gout)
-            return (_like_input(g, ctx.u_ref, ctx.geom),) + (None,) * (5 + ctx.nvalues)
+            g = _scale(g, gout)
+            return (_like_input(g, ctx.u_ref, ctx.geom),) + (None,) * (6 + ctx.nvalues)
         need_nu, need_f, need_v = ctx.extra
         u, nu, f = saved[1:4]
         values = saved[4 + len(ctx.dirichlet):]
         gu = None
         if ctx.needs_input_grad[0]:
             _, KR = residual_raw(ctx.geom, R, nu, None, ctx.dirichlet, ctx.jac, False)
-            gu = _like_input(scale_inplace_(KR.mul_(2.0), gout), ctx.u_ref, ctx.geom)
+            gu = _like_input(_scale(KR.mul_(2.0), gout), ctx.u_ref, ctx.geom)
         gnu, gf, gv = residual_input_grads_raw(ctx.geom, u, R, nu, f, ctx.dirichlet, ctx.jac, want_nu=need_nu,
-                                               want_f=need_f, want_values=need_v)
+                                               want_f=need_f, want_values=need_v, per_sample=ctx.per_sample)
         if gnu is not None:
-            gnu = _like_input(scale_inplace_(gnu, gout), nu, ctx.geom)
+            gnu = _like_input(_scale(gnu, gout), nu, ctx.geom)
         if gf is not None:
-            gf = _like_input(scale_inplace_(gf, gout), f, ctx.geom)
-        gv = [None if g is None else _like_input(scale_inplace_(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
-        return (gu, None, gnu, gf, None, None) + tuple(gv)
+            gf = _like_input(_scale(gf, gout), f, ctx.geom)
+        gv = [None if g is None else _like_input(_scale(g, gout), v, ctx.geom) for g, v in zip(gv, values)]
+        return (gu, None, gnu, gf, None, None, None) + tuple(gv)
 
 
 _WHICH = {"N": 0, "dx": 1, "dy": 2, "dz": 3}
@@ -772,7 +835,9 @@ def fem_energy(geom: Geometry, u, nu=None, f=None, f_gp=None, dirichlet: Sequenc
                nu_zero_mask=None, c_k=1.0, c_f=1.0, scale=1.0, reduction="mean", z_own=None,
                mean_count=0.0) -> torch.Tensor:
     """Fused Poisson energy loss (SURVEY.md App. A.4), differentiable w.r.t. u, nu, f, f_gp and the tensor
-    Dirichlet values (the last three not with ``z_own``)."""
+    Dirichlet values (the last three not with ``z_own``).  ``reduction``: "mean", "sum" or "none" (a (B,) loss,
+    loss[b] = scale / elements * the sum over sample b, so that its mean is the "mean" loss)."""
+    _consts(c_k, c_f, scale, reduction, 0, z_own, mean_count)     # refuses a bad reduction before any launch
     dirichlet = tuple(dirichlet)
     return FEMEnergyFunction.apply(u, nu, geom, f, f_gp, dirichlet, nu_zero_mask, c_k, c_f, scale, reduction,
                                    z_own, mean_count, *(v for _, v in dirichlet if torch.is_tensor(v)))
@@ -784,10 +849,15 @@ def fem_energy_and_grad(geom: Geometry, u, **kw):
     return loss, grad
 
 
-def fem_residual(geom: Geometry, u, nu=None, f=None, dirichlet: Sequence = (), jac=1.0) -> torch.Tensor:
-    """sum(R^2) of the assembled residual, differentiable w.r.t. u, nu, f and the tensor Dirichlet values."""
+def fem_residual(geom: Geometry, u, nu=None, f=None, dirichlet: Sequence = (), jac=1.0,
+                 reduction="sum") -> torch.Tensor:
+    """sum(R^2) of the assembled residual, differentiable w.r.t. u, nu, f and the tensor Dirichlet values.
+    ``reduction="none"``: a (B,) loss, the sum of R^2 over each sample."""
+    if reduction not in ("sum", "none"):
+        raise L.DiffNetFEMError("residual reduction must be 'sum' or 'none'")
     dirichlet = tuple(dirichlet)
-    return FEMResidualFunction.apply(u, geom, nu, f, dirichlet, jac, *(v for _, v in dirichlet if torch.is_tensor(v)))
+    return FEMResidualFunction.apply(u, geom, nu, f, dirichlet, jac, reduction,
+                                     *(v for _, v in dirichlet if torch.is_tensor(v)))
 
 
 def gp_eval(geom: Geometry, t: torch.Tensor, which: str = "N") -> torch.Tensor:

@@ -22,6 +22,7 @@
  *   dn_fem_{energy,residual}_input_grads_*  the same bodies' autograd backward w.r.t. the source, the forcing at
  *                               the Gauss points, the Dirichlet value fields and (residual) nu.
  *   dn_scale_inplace_f32        autograd's  grad_input = grad_output * dL/du.
+ *   dn_scale_per_sample_f32     the same with one grad_output per sample (reduction = none).
  *   dn_peer_{put,wait}_f32      (no reference counterpart) one-plane halo exchange of the z-slab
  *                               decomposition through NVLink peer memory.
  *
@@ -99,9 +100,19 @@ typedef struct dn_consts {
   double c_k;            /* multiplies nu * |grad u|^2      (SURVEY.md App. A.4) */
   double c_f;            /* multiplies u * f */
   double scale;          /* overall factor s (e.g. 0.5*(h/2)^2 in 0_base.py:51-52) */
-  int32_t reduction;     /* 0 = mean over batch x elements, 1 = sum */
+  int32_t reduction;     /* 0 = mean over batch x elements, 1 = sum, DN_REDUCE_NONE = one loss per sample */
   int32_t flags;         /* DN_F_* bits; 0 = the reference's forms */
 } dn_consts;
+
+/* dn_consts.reduction (and the `reduction` of dn_fem_residual_reduce_*): one loss per sample instead of one for the
+ * launch.  loss_out / loss_out_f32 then point to g->batch values each, and
+ *   energy:    loss[b] = scale / (elements of one sample) * sum_{e in sample b} sum_g w_g (...),
+ *              so the mean of loss[] is the reduction = 0 loss and its sum times the element count the reduction = 1 one;
+ *   residual:  loss[b] = sum_{nodes of sample b} R^2, whose sum is the reduction = 1 loss.
+ * The gradients written are those of loss[b] with respect to the inputs of sample b.  The per-sample values are
+ * summed in a fixed order that depends only on the launch shape (bit-reproducible run to run).  Not available with
+ * mean_count != 0, z-slab ownership (z_own_lo/hi) or a linked launch: DN_EINVAL. */
+#define DN_REDUCE_NONE 2
 
 /* dn_consts.flags: `f` is not a nodal source but an ASSEMBLED load vector b_a = sum_e sum_g w_g N_a(g) f_g
  * (dn_fem_load_vector_f32; reference-element weights, |J| stays in `scale`): the source term becomes
@@ -136,7 +147,8 @@ int dn_debug_plan(const dn_geom* g, int nfields, int has_nu, int64_t out[16]);
  * nu == NULL means nu == 1 (IBN_3D.py:132); f and fgp NULL means no source term; at most one of
  * f (nodal, (B|1,nz,ny,nx)) and fgp (at Gauss points, dense (B|1, ngp, elems), stride_b given,
  * other strides ignored; e8_2d_poisson_mms.py:47,154) may be set.
- * loss_out: device double[1] (nullable); loss_out_f32: device float[1] (nullable).
+ * loss_out: device double[1] (nullable); loss_out_f32: device float[1] (nullable); double[B] / float[B] with
+ * c->reduction == DN_REDUCE_NONE.
  * grad_u NULL -> forward only.
  */
 int dn_fem_energy_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
@@ -212,6 +224,18 @@ int dn_fem_residual_3d_f32(const dn_field* u, const dn_field* nu, const dn_field
                            const dn_geom* g, double jac, float* residual, void* workspace,
                            size_t workspace_bytes, double* loss_out, float* loss_out_f32,
                            void* stream);
+/* The same with reduction = 1 (sum, what dn_fem_residual_* do) or DN_REDUCE_NONE (loss_out / loss_out_f32 then hold
+ * g->batch values: the sum of R^2 over each sample's nodes). */
+int dn_fem_residual_reduce_2d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                  const dn_mask* masks, int nmasks, int apply_masks_to_input,
+                                  const dn_geom* g, double jac, float* residual, void* workspace,
+                                  size_t workspace_bytes, double* loss_out, float* loss_out_f32,
+                                  void* stream, int reduction);
+int dn_fem_residual_reduce_3d_f32(const dn_field* u, const dn_field* nu, const dn_field* f,
+                                  const dn_mask* masks, int nmasks, int apply_masks_to_input,
+                                  const dn_geom* g, double jac, float* residual, void* workspace,
+                                  size_t workspace_bytes, double* loss_out, float* loss_out_f32,
+                                  void* stream, int reduction);
 
 /*
  * Gradients of the fused losses with respect to their OTHER inputs -- what autograd gives the reference's loss()
@@ -227,6 +251,7 @@ int dn_fem_residual_3d_f32(const dn_field* u, const dn_field* nu, const dn_field
  *   grad_fgp[b,G,e]   = -S c_f w_G u'_G(e)                          (fgp required; dense like fgp)
  *   grad_values[k][b,n] = [k last firing at n] * S (2 c_k K(nu') u' - c_f (M f | sum_e sum_g w_g N_n f_gp))[b,n]
  *                                                                   (masks[k].value_field required)
+ *   With c->reduction == DN_REDUCE_NONE, S = scale / (elements of one sample): the gradients of loss[b].
  * dn_fem_residual_input_grads_* (the autograd backward of 12_klsum.py:80-132 w.r.t. nu, forcing, a value field)
  *   residual: the R that dn_fem_residual_*_f32 returned for the same inputs (dense (B, nz, ny, nx))
  *   grad_nu[b,n]      = 2 jac sum_{e around n} sum_g w_g N_n(g) grad u'_g . grad R_g     (nu required)
@@ -347,6 +372,9 @@ int dn_gen_box_masks_3d_f32(const int* params, int batch, int size, float* sourc
 /* x[i] *= *factor_dev for i < n, skipping all memory traffic when *factor_dev == 1.0f
  * (the usual loss.backward() case).  factor_dev is a device pointer: no host sync. */
 int dn_scale_inplace_f32(float* x, size_t n, const float* factor_dev, void* stream);
+/* x[b, i] *= factors_dev[b] for b < batch, i < n_per_sample (x dense (batch, n_per_sample)): the backward of a
+ * reduction = none loss with a (B,) grad_output.  factors_dev is a device pointer: no host sync. */
+int dn_scale_per_sample_f32(float* x, int batch, size_t n_per_sample, const float* factors_dev, void* stream);
 
 /*
  * Halo planes over NVLink peer memory (z-slab decomposition of one 3-D field over several GPUs,
