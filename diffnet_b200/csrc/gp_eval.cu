@@ -97,9 +97,10 @@ __global__ void __launch_bounds__(kGpThreads) k_gp_eval(Field in, int nx, int ny
 // gin[b, node] = sum_w sum over the elements e around the node and all Gauss points G of
 //                T_w[G][a(node in e)] * gout_w[b, G, e]          (gather form: no atomics, deterministic).
 // Lane l of a warp works on element column e = xw - 1 + l and (for l >= 1) stores node column x = e.
+// 3-D: grid z = (sample, node plane z0 + 0 .. nzl - 1) of this launch's slice.
 template <int NSD, int NG>
 __global__ void __launch_bounds__(kGpThreads) k_gp_eval_adj(GpMultiAdj m, int nx, int ny, int nz, int RY,
-                                                            float* __restrict__ gin) {
+                                                            float* __restrict__ gin, int z0, int nzl) {
   constexpr int NZ = (NSD == 3) ? 2 : 1;
   constexpr int NGP = (NSD == 3) ? NG * NG * NG : NG * NG;
   const int nelx = nx - 1, nely = ny - 1, nelz = (NSD == 3) ? nz - 1 : 1;
@@ -112,8 +113,8 @@ __global__ void __launch_bounds__(kGpThreads) k_gp_eval_adj(GpMultiAdj m, int nx
   const int x = e;                                                       // node column stored by lanes >= 1
   const bool sv = (lane >= 1) && (x < nx);
   const int y0 = blockIdx.y * RY, y1 = min(ny, y0 + RY);                 // node rows [y0, y1)
-  const int z = (NSD == 3) ? (int)(blockIdx.z % nzz) : 0;
-  const int b = (NSD == 3) ? (int)(blockIdx.z / nzz) : (int)blockIdx.z;
+  const int z = (NSD == 3) ? z0 + (int)(blockIdx.z % nzl) : 0;
+  const int b = (NSD == 3) ? (int)(blockIdx.z / nzl) : (int)blockIdx.z;
   const long long nel = (long long)nelx * nely * nelz;
   const long long gb = (long long)b * NGP * nel + (ev ? e : 0);
   float* orow = gin + (((long long)b * nzz + z) * ny + y0) * nx + (sv ? x : 0);
@@ -371,6 +372,22 @@ cudaError_t launch_gp_eval(Field in, int B, int nx, int ny, int nz, int nsd, con
   // 4 ngp B written per node and table), so sharing the read buys little, and a pass that writes 12-32 output streams
   // per thread runs at a lower fraction of the peak: measured 256^2 x 64, 3 tables: 70.4 / 65.6 / 61.7 us with
   // 4 / 2 / 1 tables per pass; 64^3 x 16, 4 tables: 204.7 / 164.8 / 136.1 us.
+  if (nsd == 3 && nz - 1 > 65535) {
+    // more element layers than grid z holds (launch_fwd puts samples x layers there): the general-basis kernel, a
+    // flat grid-stride loop, evaluates the Q1 tables one at a time
+    for (int w = 0; w < m.nw; ++w) {
+      const int ng = m.tb[w].n;
+      float fac[3 * 4 * 2];
+      for (int d = 0; d < 3; ++d)
+        for (int g = 0; g < ng; ++g)
+          for (int a = 0; a < 2; ++a) fac[(d * ng + g) * 2 + a] = m.tb[w].c[d][g][a];
+      int bad = 0;
+      const cudaError_t e = launch_gp_eval_general(in, B, 3, nx, ny, nz, 2, ng, fac, m.out[w], s, &bad);
+      if (e != cudaSuccess) return e;
+      if (bad) return cudaErrorInvalidValue;
+    }
+    return cudaSuccess;
+  }
   const char* ev = getenv("DN_GP_TABLES_PER_PASS");
   int per = (ev && atoi(ev) > 0) ? atoi(ev) : 1;
   for (int w0 = 0; w0 < m.nw; w0 += per) {
@@ -447,18 +464,23 @@ static cudaError_t launch_adj(int B, int nx, int ny, int nz, GpMultiAdj m, float
   const int warps_needed = (nx + 30) / 31;
   const int wpc = warps_needed >= kGpThreads / 32 ? kGpThreads / 32 : warps_needed;
   const int gx = (warps_needed + wpc - 1) / wpc;
-  const int bmax = 65535 / nzz;
-  if (bmax < 1) return cudaErrorInvalidConfiguration;
+  // gridDim.z = batch slice * node planes (<= 65535): a mesh of more planes runs one sample and a slice of its planes
+  // per launch
+  const int zs = nzz < 65535 ? nzz : 65535;
+  const int bmax = 65535 / zs;
   for (int b0 = 0; b0 < B; b0 += bmax) {
     const int nb = (B - b0 < bmax) ? B - b0 : bmax;
-    const long long gz = (long long)nb * nzz;
-    const int RY = rows_per_chunk((long long)gx * gz, ny);
-    dim3 grid(gx, (ny + RY - 1) / RY, (unsigned)gz);
-    switch (NG) {
-      case 2: k_gp_eval_adj<NSD, 2><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin); break;
-      case 3: k_gp_eval_adj<NSD, 3><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin); break;
-      case 4: k_gp_eval_adj<NSD, 4><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin); break;
-      default: return cudaErrorInvalidValue;
+    for (int z0 = 0; z0 < nzz; z0 += zs) {
+      const int nzl = (nzz - z0 < zs) ? nzz - z0 : zs;
+      const long long gz = (long long)nb * nzl;
+      const int RY = rows_per_chunk((long long)gx * gz, ny);
+      dim3 grid(gx, (ny + RY - 1) / RY, (unsigned)gz);
+      switch (NG) {
+        case 2: k_gp_eval_adj<NSD, 2><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin, z0, nzl); break;
+        case 3: k_gp_eval_adj<NSD, 3><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin, z0, nzl); break;
+        case 4: k_gp_eval_adj<NSD, 4><<<grid, wpc * 32, 0, s>>>(m, nx, ny, nz, RY, gin, z0, nzl); break;
+        default: return cudaErrorInvalidValue;
+      }
     }
     gin += (long long)nb * nzz * ny * nx;
     for (int w = 0; w < m.nw; ++w) m.gout[w] += (long long)nb * per_b;

@@ -296,8 +296,9 @@ __device__ __forceinline__ void store_node(const InGrad& q, const Flags& fl, int
 // ---- 2-D ------------------------------------------------------------------------------------------------------------
 constexpr int kIgWarps = 4;
 
+// b0: the first sample of this launch's batch slice (gridDim.z is capped at 65535)
 template <int NG, int MODE>
-__global__ void __launch_bounds__(32 * kIgWarps, 4) k_input_grads_2d(InGrad q, Flags fl, int RY, int ball) {
+__global__ void __launch_bounds__(32 * kIgWarps, 4) k_input_grads_2d(InGrad q, Flags fl, int RY, int ball, int b0) {
   constexpr int NS = MODE ? 3 : 2;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int nx = q.nx, ny = q.ny, nelx = nx - 1, nely = ny - 1;
@@ -310,7 +311,7 @@ __global__ void __launch_bounds__(32 * kIgWarps, 4) k_input_grads_2d(InGrad q, F
   if (y0 >= ny) return;                                       // warp-uniform; the kernel has no CTA barrier
   const int y1 = min(ny, y0 + RY);
   const long long nodes = (long long)nx * ny, nel = (long long)nelx * nely, ngpe = (long long)NG * NG * nel;
-  const int bb = ball ? 0 : (int)blockIdx.z, be = ball ? q.B : (int)blockIdx.z + 1;
+  const int bb = ball ? 0 : b0 + (int)blockIdx.z, be = ball ? q.B : bb + 1;
   const unsigned full = 0xffffffffu;
 
   for (int b = bb; b < be; ++b) {
@@ -481,9 +482,15 @@ cudaError_t launch(const InGrad& q, const Flags& fl, int nsd, int sms, cudaStrea
     long long ry = (q.ny * ntx * bgrid + sms * 48LL - 1) / (sms * 48LL);
     ry = std::min(64LL, std::max(8LL, ry));
     const long long nch = (q.ny + ry - 1) / ry;
-    const dim3 grid((unsigned)ntx, (unsigned)((nch + kIgWarps - 1) / kIgWarps), (unsigned)bgrid);
-    k_input_grads_2d<NG, MODE><<<grid, 32 * kIgWarps, 0, s>>>(q, fl, (int)ry, ball);
-    return cudaGetLastError();
+    // one sample per grid z: batches beyond the 65535 limit of that axis run in slices
+    for (long long b0 = 0; b0 < bgrid; b0 += 65535) {
+      const dim3 grid((unsigned)ntx, (unsigned)((nch + kIgWarps - 1) / kIgWarps),
+                      (unsigned)std::min(65535LL, bgrid - b0));
+      k_input_grads_2d<NG, MODE><<<grid, 32 * kIgWarps, 0, s>>>(q, fl, (int)ry, ball, (int)b0);
+      const cudaError_t e = cudaGetLastError();
+      if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
   }
   constexpr int NS = MODE ? 3 : 2;
   constexpr int ML = kIg3MaxLanes<NG>;
